@@ -66,6 +66,11 @@ def load():
         lib.rzo_go_random_games.restype = C.c_int
         lib.rzo_go_random_games.argtypes = [C.c_int, C.c_int, C.c_double, C.c_int, i32p, C.c_int, C.c_uint64, i32p, i32p,
                                             i8p, i32p, i32p, i32p, f64p, i8p]
+        lib.rzo_philox4.restype = None
+        lib.rzo_philox4.argtypes = [C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint32, C.c_uint64, C.POINTER(C.c_uint32)]
+        lib.rzo_go_rollout_dm.restype = C.c_int
+        lib.rzo_go_rollout_dm.argtypes = [C.c_int, C.c_double, C.c_int, i8p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                          C.c_int, C.c_int, C.c_uint32, C.c_uint32, C.c_uint64, f64p, i8p]
         _lib = lib
     return _lib
 

@@ -351,3 +351,61 @@ int rzo_go_random_games(int G, int N, double komi, int move_cap, const int32_t* 
   }
   return 0;
 }
+
+/* ---- the device's random playouts (rz_eval_rollout_dm_kernel<rz_go_game>, rlzero_b200/csrc/rz_game.cu:342-389) ------
+ * Philox-4x32-10 as rz_philox4 (rz_common.cuh:178-195); oracle/philox.py restates it in Python and the CPU tests pin
+ * both to the Random123 known-answer vectors. */
+static void rzo_philox4_(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint64_t seed, uint32_t out[4]) {
+  uint32_t c[4] = {c0, c1, c2, c3};
+  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+  for (int r = 0; r < 10; ++r) {
+    const uint64_t p0 = (uint64_t)0xD2511F53u * c[0], p1 = (uint64_t)0xCD9E8D57u * c[2];
+    const uint32_t n0 = (uint32_t)(p1 >> 32) ^ c[1] ^ k0, n1 = (uint32_t)p1, n2 = (uint32_t)(p0 >> 32) ^ c[3] ^ k1,
+                   n3 = (uint32_t)p0;
+    c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+    k0 += 0x9E3779B9u; k1 += 0xBB67AE85u;
+  }
+  out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
+}
+
+void rzo_philox4(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint64_t seed, uint32_t* out) {
+  rzo_philox4_(c0, c1, c2, c3, seed, out);
+}
+
+/* mean returns of n_rollouts random playouts from one position (cell[N*N] +1 / -1 / 0, to_play +1 black / -1 white,
+ * n moves played, pass1 / pass2 = the last / the one before last move was a pass).  Playout r, ply i: counter
+ * (g, visit, r << 16 | i, 0xd311); the candidates are the legal points ascending, then the pass; the status is tested
+ * before every move and once more after n_limit moves, a playout cut there returns [0, 0].  out[2] = sum / n_rollouts
+ * for (black, white); legal_out[N*N + 1] = the legal mask of the position (the evaluator's priors). */
+int rzo_go_rollout_dm(int N, double komi, int max_moves, const int8_t* cell, int ko, int to_play, int n, int pass1,
+                      int pass2, int n_rollouts, int n_limit, uint32_t g, uint32_t visit, uint64_t seed, double* out,
+                      int8_t* legal_out) {
+  if (N < 1 || N * N > GMAX || n_rollouts < 1 || n_limit < 0) return -3;
+  const int NN = N * N;
+  gob_t b0;
+  gob_reset(&b0, N, komi, max_moves);
+  for (int c = 0; c < NN; ++c) b0.cell[c] = cell[c];
+  b0.ko = ko; b0.to_play = to_play; b0.n = n; b0.pass1 = pass1; b0.pass2 = pass2;
+  for (int a = 0; a <= NN; ++a) legal_out[a] = (int8_t)go_legal(&b0, a);
+  int sum0 = 0, sum1 = 0;
+  for (int r = 0; r < n_rollouts; ++r) {
+    gob_t b = b0;
+    for (int i = 0; i <= n_limit; ++i) {
+      if (go_over(&b) || i == n_limit) break;
+      int cand[GMAX + 1], n_act = 0;
+      for (int a = 0; a < NN; ++a) if (go_legal(&b, a)) cand[n_act++] = a;
+      cand[n_act++] = NN;                                  /* the pass is the last candidate */
+      uint32_t w[4];
+      rzo_philox4_(g, visit, ((uint32_t)r << 16) | (uint32_t)i, 0xd311u, seed, w);
+      const int pick = (int)(((uint64_t)w[0] * (uint64_t)n_act) >> 32);
+      if (go_play(&b, cand[pick]) != 0) return -4;
+    }
+    if (go_over(&b)) {                                     /* rz_game_returns: Go always ends decided */
+      const int r0 = go_winner(&b) == 0 ? 1 : -1;
+      sum0 += r0; sum1 -= r0;
+    }
+  }
+  out[0] = (double)sum0 / (double)n_rollouts;
+  out[1] = (double)sum1 / (double)n_rollouts;
+  return 0;
+}

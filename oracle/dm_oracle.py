@@ -26,9 +26,10 @@ import numpy as np
 
 
 class Node(object):
-    __slots__ = ('action', 'player', 'prior', 'n', 'w', 'outcome', 'children')
+    __slots__ = ('action', 'player', 'prior', 'n', 'w', 'outcome', 'children', 'index')
 
     def __init__(self, action, player, prior):
+        self.index = -1                  # the device's allocation index (set at the node's evaluation)
         self.action = action
         self.player = player
         self.prior = prior
@@ -76,6 +77,12 @@ class DMSearch(object):
         self.max_utility = max_utility
         self.noise_fn = noise_fn or (lambda k: np.random.dirichlet([self.alpha] * k))
         self.shuffle_fn = shuffle_fn          # in-place list shuffle (deepmind_mcts.py:508); None = keep the order
+        # what an evaluator / shuffle_fn restating the device's random draws reads: the root of the running search
+        # and the node whose children are being created (Node.index numbers nodes in the order the device
+        # allocates them: at their first evaluation, where the reference creates children at the second visit)
+        self.root = None
+        self.expanding = None
+        self.n_nodes = 0
 
     def _score(self, ch, parent_n):
         return ch.puct(parent_n, self.uct_c) if self.rule == 'puct' else ch.uct(parent_n, self.uct_c)
@@ -91,6 +98,7 @@ class DMSearch(object):
                     noise = self.noise_fn(len(pri))
                     pri = [(a, self.eps * z + (1 - self.eps) * p) for (a, p), z in zip(pri, noise)]
                 if self.shuffle_fn is not None:
+                    self.expanding = node
                     self.shuffle_fn(pri)                  # "Reduce bias from move generation order" (:508)
                 mover = work.current_player()
                 node.children = [Node(a, mover, p) for a, p in pri]
@@ -106,6 +114,7 @@ class DMSearch(object):
 
     def search(self, env):               # deepmind_mcts.py:554-646
         root = Node(None, env.current_player(), 1)
+        self.root, self.n_nodes = root, 0
         for _ in range(self.max_simulations):
             path, work = self._descend(root, env)
             if work.is_terminal():
@@ -115,6 +124,8 @@ class DMSearch(object):
             else:
                 returns = self.evaluator.evaluate(work)
                 solved = False
+                path[-1].index = self.n_nodes
+                self.n_nodes += 1
             while path:
                 node = path.pop()
                 node.w += returns[node.player]

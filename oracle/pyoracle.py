@@ -380,7 +380,9 @@ class RolloutSearch(object):
     """RolloutMCTS restated (rollout_mcts.py:10-108): uniform priors, leaf value from a random
     playout.  ``rollout`` selects the rollout policy: 'random' draws ``np.random.rand(len(legal))``
     per ply and plays the argmax exactly like the reference (:96-100, :63-65); 'first' / 'last' play
-    the lowest / highest legal move (deterministic stand-ins for device parity tests).
+    the lowest / highest legal move (deterministic stand-ins for device parity tests); a callable
+    ``rollout(board, root_n)`` returns the leaf value itself (``rollout_oracle.AZRollout``: the device's
+    counter-based playouts, draw for draw).
 
     Quirk kept on purpose: the winner is compared with ``current_player()`` AFTER the playout
     (:69-72), and the env flips the player after every move (gomoku_env.py:67-68), so every
@@ -409,6 +411,10 @@ class RolloutSearch(object):
         return zip(legal, probs)
 
     def evaluate(self, board):  # :49-74
+        if callable(self.rollout):
+            # a restatement of the device's playout (oracle/rollout_oracle.AZRollout), keyed by the root's
+            # visit count at this evaluation
+            return self.rollout(board, self.root.n)
         winner = -1
         for _ in range(self.n_limit):
             end, winner = board.game_end_winner()

@@ -389,22 +389,33 @@ class SearchForest(object):
         # [evaluate, backup]  -- two captured graphs instead of one
         fuse = (self.K == 1 and getattr(evaluator, 'prior64', None) is None
                 and os.environ.get('RZ_FUSE_SELECT', '1') != '0')
-        value64 = getattr(evaluator, 'value64', None)
 
+        # value64 / prior64 are read after the evaluator has run: an evaluator may allocate them in its first call
+        # (RandomRolloutEvaluator) or re-allocate them for a forest of another size
         def mid():
             evaluator(self)
-            self.expand_backup_select(prior_is_log, noise_eps, noise_alpha, 0, value64=value64)
+            self.expand_backup_select(prior_is_log, noise_eps, noise_alpha, 0,
+                                      value64=getattr(evaluator, 'value64', None))
 
         def last():
             evaluator(self)
-            self.expand_backup(prior_is_log, noise_eps, noise_alpha, 0, value64=value64,
+            self.expand_backup(prior_is_log, noise_eps, noise_alpha, 0, value64=getattr(evaluator, 'value64', None),
                                prior64=getattr(evaluator, 'prior64', None))
+
+        def buffers():
+            # the evaluator's host-visible output buffers as a captured graph holds them: address and shape
+            return tuple(None if t is None else (t.data_ptr(), tuple(t.shape))
+                         for t in (getattr(evaluator, 'value64', None), getattr(evaluator, 'prior64', None)))
 
         # weights_version: a captured graph holds the weight pointers (and the fused head's filter taps) and the
         # evaluator's activation buffers by value, so repacked weights or re-allocated buffers need a new capture
-        # (NativeForward bumps it in both cases).  The cache entry keeps the evaluator alive: its id() is the key
-        key = (id(evaluator), getattr(evaluator, 'weights_version', 0), prior_is_log, float(noise_eps),
-               float(noise_alpha), fuse)
+        # (NativeForward bumps it in both cases); value64 / prior64 enter the key themselves.  The cache entry keeps
+        # the evaluator alive: its id() is the key
+        def cache_key():
+            return (id(evaluator), getattr(evaluator, 'weights_version', 0), prior_is_log, float(noise_eps),
+                    float(noise_alpha), fuse, buffers())
+
+        key = cache_key()
         graphs = self.__dict__.setdefault('_graphs', {})
         if key not in graphs and len(graphs) >= 8:
             graphs.clear()                                              # bounded cache
@@ -415,6 +426,7 @@ class SearchForest(object):
                 mid()                       # wave 1; leaves the leaves of wave 2 selected
                 n_waves -= 1
                 torch.cuda.synchronize()
+                key = cache_key()           # the buffers the warm-up call left are the ones the graphs capture
                 g_mid, g_last, g_mid8 = torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph(), torch.cuda.CUDAGraph()
                 with capture_graph(g_mid):
                     mid()
@@ -431,6 +443,7 @@ class SearchForest(object):
             wave()
             n_waves -= 1
             torch.cuda.synchronize()
+            key = cache_key()
             g = torch.cuda.CUDAGraph()
             with capture_graph(g):
                 wave()

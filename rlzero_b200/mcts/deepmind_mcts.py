@@ -23,7 +23,9 @@ of the descent and of ``best_child``) and draws the root's Dirichlet noise (:539
   same seed, bit for bit (``tests/golden/dm_mcts_shuffle.json``).  One tree, three small device-host
   copies per simulation: a checker, not the fast path;
 * ``child_shuffle=True`` (default, like the reference) without a ``random_state`` -- counter-based random
-  child order and root noise on the device, inside the captured wave graph (same distribution);
+  child order and root noise on the device, inside the captured wave graph (same distribution as the
+  reference; the child order and the device playouts are pinned draw for draw to
+  ``oracle/rollout_oracle.py``);
 * ``child_shuffle=False`` -- no shuffle, ties to the lowest action (the deterministic fixtures).
 
 The reference's quirks that change results are kept: the noise

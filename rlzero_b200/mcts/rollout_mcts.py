@@ -4,10 +4,12 @@ pure Monte-Carlo tree search (uniform priors, random playouts), the opponent
 (tools/train_alphazero.py:139-163).
 
 Search, expansion and backup are the kernels of ``AlphaZeroMCTS``; the leaf evaluator is
-``rz_eval_rollout`` (random playouts on the device, one warp per game).  The playouts use a
-counter-based RNG instead of the global ``np.random`` stream of the reference (:96-100), so moves
-agree with the reference in distribution, not draw by draw; with the deterministic rollout modes
-('first' / 'last') visit counts match the reference algorithm bit for bit (tests).
+``rz_eval_rollout`` (random playouts on the device, one warp per game).  The playouts draw from a
+counter-based Philox stream instead of the global ``np.random`` stream of the reference (:96-100), so
+moves agree with the reference in distribution, not draw by draw.  The device playouts themselves are
+pinned draw for draw to a restatement (``oracle/rollout_oracle.py``): for the same ``seed`` visit
+counts, value sums and the move are bit-identical to it (tests/test_gpu_rollout_parity.py).  With the
+deterministic rollout modes ('first' / 'last') visit counts match the reference algorithm bit for bit.
 """
 import numpy as np
 
