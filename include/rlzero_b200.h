@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define RZ_ABI_VERSION 9
+#define RZ_ABI_VERSION 10
 #define RZ_MAX_BOARD 19          /* rows live one per lane; A <= 362 (19x19 Go incl. the pass) */
 #define RZ_META_STRIDE 12
 #define RZ_GO_HIST 14            /* history planes a Go position carries besides the current board */
@@ -58,7 +58,13 @@ enum rz_meta {                   /* int32 words of a game's meta record */
 };                               /* words 10, 11 reserved.  Go also uses LAST_MOVE = last ACTION (the pass
                                     is H*W) and STONES = moves played (Position.n) */
 
-enum rz_status { RZ_ACTIVE = 0, RZ_ENDED_WIN = 1, RZ_ENDED_TIE = 2, RZ_IDLE = 3 };
+enum rz_status {
+  RZ_ACTIVE = 0,
+  RZ_ENDED_WIN = 1,
+  RZ_ENDED_TIE = 2,
+  RZ_IDLE = 3                    /* waiting for the other seat (rz_match_commit): the game runs, but this forest's
+                                    root is not the mover's; every tree kernel skips it like a finished game */
+};
 
 enum rz_fault {
   RZ_FAULT_ILLEGAL_MOVE = 1,     /* AssertionError in gomoku_env.py:51 */
@@ -343,6 +349,18 @@ int rz_tree_root_policy(const rz_tree_desc* t, double temperature, int32_t* visi
    then restarts the slot from an empty board. */
 int rz_tree_advance(const rz_tree_desc* t, const int32_t* moves, int keep_subtree, int max_carry,
                     const rz_traj_desc* traj, const float* pi, int auto_reset, void* stream);
+
+/* ---- evaluation matches: GameControl.start_play (rlzero/games/gomoku/game.py:61-94) for G games at once ----
+   Two forests, one per seat, over the same G games: tree g of each forest is game g.  In a running game exactly
+   one seat's root is RZ_ACTIVE (the mover's), the other's RZ_IDLE.  For every game whose seat-s root is ACTIVE
+   the move is moves_s[g] (rz_tree_root_policy's draw on that forest) or, when moves_s is NULL, the first
+   most-visited child of the root (RolloutMCTS.simulate, rollout_mcts.py:76-81).  The move is played and logged
+   at move_log[g * max_plies + ply]; both roots receive the new position and fresh trees; the mover's root turns
+   IDLE and the other ACTIVE, or both take the ended status and the winner.  An illegal move raises
+   RZ_FAULT_ILLEGAL_MOVE, an unexpanded mover root RZ_FAULT_NO_CHILDREN, in the mover's root meta (nothing is
+   played then).  Line games, AlphaZero flavour, one leaf per wave; max_plies >= the board's cells. */
+int rz_match_commit(const rz_tree_desc* seat0, const rz_tree_desc* seat1, const int32_t* moves0,
+                    const int32_t* moves1, int32_t* move_log, int max_plies, void* stream);
 
 /* ---- closed-form evaluators for parity tests (oracle/evaluators.py) ------- */
 int rz_eval_closed_form(const rz_tree_desc* t, int eval_id, float* prior, float* value,

@@ -11,7 +11,7 @@ import torch  # noqa: F401  -- loads libcudart.so.12 into the process before our
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'librlzero_b200.so')
 
-ABI_VERSION = 9
+ABI_VERSION = 10
 META_STRIDE = 12
 (META_PLAYER, META_LAST_MOVE, META_STONES, META_STATUS, META_WINNER, META_PLY, META_FAULT,
  META_EPISODE, META_KO, META_PASSES) = range(10)
@@ -116,6 +116,7 @@ SIGNATURES = {
     'rz_tree_best_child': (C.c_int, [_TD, _vp, _vp, _vp]),
     'rz_tree_root_policy': (C.c_int, [_TD, C.c_double, _vp, _vp, _vp, _vp, C.c_ulonglong, _vp]),
     'rz_tree_advance': (C.c_int, [_TD, _vp, C.c_int, C.c_int, _TJ, _vp, C.c_int, _vp]),
+    'rz_match_commit': (C.c_int, [_TD, _TD, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_eval_closed_form': (C.c_int, [_TD, C.c_int, _vp, _vp, _vp]),
     'rz_augment_equi': (C.c_int, [_GD, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_gather_rows': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, _vp]),

@@ -915,6 +915,78 @@ rz_advance_kernel(rz_tree_desc t, const int32_t* __restrict__ moves, int keep_su
 }
 
 // ---------------------------------------------------------------------------
+// Evaluation match (GameControl.start_play, game.py:61-94) for G games at once: tree g of both seats' forests is
+// game g, the mover's root is ACTIVE and the other seat's IDLE.  One warp per game plays the mover's move, hands the
+// position over and gives both seats fresh trees (neither player keeps a tree between moves, alphazero_mcts.py:158,
+// rollout_mcts.py:131).
+// ---------------------------------------------------------------------------
+template <class GM>
+__global__ void __launch_bounds__(RZ_TREE_THREADS)
+rz_match_commit_kernel(rz_tree_desc t0, rz_tree_desc t1, const int32_t* __restrict__ moves0,
+                       const int32_t* __restrict__ moves1, int32_t* __restrict__ move_log, int max_plies) {
+  const int g = blockIdx.x * RZ_TREE_WARPS + (threadIdx.x >> 5);
+  if (g >= t0.n_trees) return;
+  const int lane = rz_lane();
+  const rz_geom q = rz_geom_of(t0.game);
+  int32_t* m0 = t0.root_meta + (size_t)g * RZ_META_STRIDE;
+  int32_t* m1 = t1.root_meta + (size_t)g * RZ_META_STRIDE;
+  const int seat = m0[RZ_META_STATUS] == RZ_ACTIVE ? 0 : (m1[RZ_META_STATUS] == RZ_ACTIVE ? 1 : -1);
+  if (seat < 0) return;                       // game over
+  const rz_tree_desc& tm = seat ? t1 : t0;    // the mover's forest
+  const rz_tree_desc& to = seat ? t0 : t1;
+  int32_t* mm = seat ? m1 : m0;
+  int32_t* mo = seat ? m0 : m1;
+  const int32_t* moves = seat ? moves1 : moves0;
+  if (tm.n_nodes[g] == 0) {                   // no search ran on the mover's root: nothing to choose from
+    if (lane == 0) mm[RZ_META_FAULT] |= RZ_FAULT_NO_CHILDREN;
+    return;
+  }
+  int m;
+  if (moves) {
+    m = moves[g];
+  } else {
+    // the first most-visited child: max over (N desc, action asc) of the root's children (edge_N >= 0)
+    const size_t base = rz_edge_base(tm, g, 0);
+    int bn = -1, bs = 0x7fffffff;
+    for (int s = lane; s < tm.game.action_stride; s += 32) {
+      const int n = tm.edge_N[base + s];
+      if (n > bn) { bn = n; bs = s; }           // s ascends per lane: the first maximum of the lane
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const int n2 = __shfl_xor_sync(RZ_FULL, bn, o);
+      const int s2 = __shfl_xor_sync(RZ_FULL, bs, o);
+      if (n2 > bn || (n2 == bn && s2 < bs)) { bn = n2; bs = s2; }
+    }
+    m = bn >= 0 ? bs : -1;
+  }
+  typename GM::board b;
+  GM::load_root(b, tm, g);
+  if (m < 0 || GM::action_illegal(b, m, q)) {
+    if (lane == 0) mm[RZ_META_FAULT] |= RZ_FAULT_ILLEGAL_MOVE;
+    return;
+  }
+  const int ply = mm[RZ_META_PLY];
+  GM::play(b, m, q);
+  int winner;
+  const int status = GM::status(b, q, winner);
+  // both roots hold the position after the move; only the other seat's is searched next
+  GM::store_root(b, to, g);
+  GM::store_root(b, tm, g);
+  if (lane == 0) {
+    if (ply < max_plies) move_log[(size_t)g * max_plies + ply] = m;
+    GM::store_meta(b, mo);
+    GM::store_meta(b, mm);
+    mo[RZ_META_STATUS] = status;
+    mm[RZ_META_STATUS] = status == RZ_ACTIVE ? RZ_IDLE : status;
+    mo[RZ_META_WINNER] = mm[RZ_META_WINNER] = winner;
+    mo[RZ_META_PLY] = mm[RZ_META_PLY] = ply + 1;
+    rz_tree_fresh(to, g, 0, 0.0);
+    rz_tree_fresh(tm, g, 0, 0.0);
+  }
+}
+
+// ---------------------------------------------------------------------------
 // SearchNode.best_child (deepmind_mcts.py:153-175): max over the root's children of the key
 // (outcome[player] or 0, explore_count, total_reward); first maximum wins.
 // ---------------------------------------------------------------------------
@@ -1154,6 +1226,29 @@ extern "C" int rz_tree_advance(const rz_tree_desc* t, const int32_t* moves, int 
     rz_advance_kernel<rz_line_game><<<rz_tree_grid(t->n_trees), RZ_TREE_THREADS, smem, (cudaStream_t)stream>>>(
         *t, moves, keep_subtree, max_carry, td, traj != nullptr, pi, auto_reset, words);
   RZ_LAUNCH_CHECK("rz_tree_advance");
+  return 0;
+}
+
+extern "C" int rz_match_commit(const rz_tree_desc* seat0, const rz_tree_desc* seat1, const int32_t* moves0,
+                               const int32_t* moves1, int32_t* move_log, int max_plies, void* stream) {
+  if (rz_check_tree(seat0, "rz_match_commit (seat 0)") || rz_check_tree(seat1, "rz_match_commit (seat 1)")) return -1;
+  RZ_REQUIRE(memcmp(&seat0->game, &seat1->game, sizeof(rz_game_desc)) == 0,
+             "rz_match_commit: the seats' game descriptors differ");
+  RZ_REQUIRE(seat0->n_trees == seat1->n_trees, "rz_match_commit: n_trees %d vs %d", seat0->n_trees, seat1->n_trees);
+  RZ_REQUIRE(seat0->game.game_type != RZ_GAME_GO, "rz_match_commit: Go is not supported");
+  RZ_REQUIRE(seat0->flavour == RZ_FLAVOUR_ALPHAZERO && seat1->flavour == RZ_FLAVOUR_ALPHAZERO,
+             "rz_match_commit: the DeepMindMCTS flavour is not supported");
+  RZ_REQUIRE(seat0->leaves_per_tree <= 1 && seat1->leaves_per_tree <= 1,
+             "rz_match_commit: leaves_per_tree %d / %d (one leaf per wave only)", seat0->leaves_per_tree,
+             seat1->leaves_per_tree);
+  RZ_REQUIRE(move_log, "rz_match_commit: null move_log");
+  const int W = seat0->game.width > 0 ? seat0->game.width : seat0->game.board_size;
+  RZ_REQUIRE(max_plies >= seat0->game.board_size * W, "rz_match_commit: max_plies %d below the board's %d cells",
+             max_plies, seat0->game.board_size * W);
+  if (seat0->n_trees == 0) return 0;
+  rz_match_commit_kernel<rz_line_game><<<rz_tree_grid(seat0->n_trees), RZ_TREE_THREADS, 0, (cudaStream_t)stream>>>(
+      *seat0, *seat1, moves0, moves1, move_log, max_plies);
+  RZ_LAUNCH_CHECK("rz_match_commit");
   return 0;
 }
 

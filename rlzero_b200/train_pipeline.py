@@ -105,9 +105,14 @@ def augment_equi_device(forest_or_desc, rows, info, pi):
 class TrainPipeline(object):
 
     def __init__(self, board_size=6, n_in_row=4, n_playout=400, n_parallel_games=1, device='cuda', net=None,
-                 game_batch_num=64, check_freq=50, pure_mcts_playout_num=100, leaves_per_wave=1):
+                 game_batch_num=64, check_freq=50, pure_mcts_playout_num=100, leaves_per_wave=1,
+                 batched_evaluation=False):
         # leaves_per_wave > 1: leaf-parallel self-play search of the single-game path (an extension; the default is
         # the reference's sequential search)
+        # batched_evaluation: policy_evaluate plays its games at once on the device (BatchedMatch) instead of one after
+        # another through GameControl.start_play.  The two paths draw from different random streams, so their results
+        # agree in distribution, not game for game
+        self.batched_evaluation = bool(batched_evaluation)
         # params of the board and the game (tools/train_alphazero.py:19-26)
         self.board_size = board_size
         self.n_in_row = n_in_row
@@ -247,14 +252,22 @@ class TrainPipeline(object):
         return loss, entropy
 
     def policy_evaluate(self, n_games=10):
-        """Evaluate the trained policy against the pure MCTS player (:139-163)."""
+        """Evaluate the trained policy against the pure MCTS player (:139-163).  With ``batched_evaluation`` the
+        games run as one ``BatchedMatch`` whose draws follow ``np.random.seed`` through its ``seed``."""
         current_mcts_player = AlphaZeroPlayer(self.alphazero_agent.policy_value_fn, n_playout=self.n_playout,
                                               c_puct=self.c_puct)
         pure_mcts_player = RolloutPlayer(n_playout=self.pure_mcts_playout_num, c_puct=5)
-        win_cnt = defaultdict(int)
-        for i in range(n_games):
-            winner = self.game.start_play(current_mcts_player, pure_mcts_player, start_player=i % 2, is_shown=0)
-            win_cnt[winner] += 1
+        if self.batched_evaluation:
+            # every game starts with player1 (id 0), as start_play does whatever start_player says
+            from .match import BatchedMatch
+            match = BatchedMatch(current_mcts_player, pure_mcts_player, n_games, self.board_size, self.n_in_row,
+                                 device=self.device)
+            win_cnt = match.play(seed=int(np.random.randint(0, 2 ** 31 - 1)))['win_cnt']
+        else:
+            win_cnt = defaultdict(int)
+            for i in range(n_games):
+                winner = self.game.start_play(current_mcts_player, pure_mcts_player, start_player=i % 2, is_shown=0)
+                win_cnt[winner] += 1
         win_ratio = 1.0 * (win_cnt[1] + 0.5 * win_cnt[-1]) / n_games
         print('num_playouts:{}, win: {}, lose: {}, tie:{}'.format(self.pure_mcts_playout_num, win_cnt[1],
                                                                   win_cnt[2], win_cnt[-1]))
