@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define RZ_ABI_VERSION 10
+#define RZ_ABI_VERSION 11
 #define RZ_MAX_BOARD 19          /* rows live one per lane; A <= 362 (19x19 Go incl. the pass) */
 #define RZ_META_STRIDE 12
 #define RZ_GO_HIST 14            /* history planes a Go position carries besides the current board */
@@ -255,10 +255,6 @@ int rz_gomoku_encode_f32(const rz_game_desc* g, const uint32_t* rows, const int3
 /* the same planes channels-last, float32 [n][HW][4] (input of the fp32 trunk). */
 int rz_gomoku_encode_nhwc_f32(const rz_game_desc* g, const uint32_t* rows, const int32_t* meta,
                               float* planes, int n_games, void* stream);
-/* same planes as bf16 in the tensor-core trunk's layout [n][256][64]: position
-   p = y*16+x (x,y < 15 real, else zero), channels 0..3 = planes, 4..63 zero. */
-int rz_gomoku_encode_tc(const rz_game_desc* g, const uint32_t* rows, const int32_t* meta,
-                        void* act_bf16, int n_games, void* stream);
 
 /* ---- game dynamics: GoEnv (rlzero/games/go/go_env.py over pettingzoo go_base = MiniGo rules) ----
    Positions: rows [n][2][H] (black, white), hist [n][RZ_GO_HIST][H] = board_history planes 2..15
@@ -526,20 +522,15 @@ typedef struct rz_heads_desc {
   const void* wtc_lo;
 } rz_heads_desc;
 
-/* 3x3 convolution (padding 1) + bias (+ residual) (+ ReLU) on the tensor cores (tcgen05/TMEM/TMA):
-   act_in bf16 [n][256][c_in] tile layout (see rz_gomoku_encode_tc), c_in in {64,128};
-   weight bf16 [9][128][c_in] (tap = kh*3+kw, then out channel, then in channel); bias f32 [128];
-   residual/act_out bf16 [n][256][128] (residual may alias act_out, may be NULL).
-   n_ctas <= 0 picks one persistent CTA per SM.  nn.Conv2d + folded BatchNorm + ReLU of the trunk. */
-int rz_net_conv3x3_tc(const void* act_in, const void* weight, const float* bias, const void* residual,
-                      void* act_out, int n_boards, int board_size, int c_in, int relu, int n_ctas,
-                      void* stream);
-/* revision 2 of the same operator (same tensors, same results): the 9x128x128 weights stay resident
-   in shared memory, split over a CTA pair (cta_group = 2: tcgen05 cta_group::2 MMAs, cluster of 2),
-   and each 128-position activation tile is loaded once with its 17-row halo; the 9 taps are
-   row-shifted UMMA descriptors on that tile.  cta_group = 1 runs the same data path on single CTAs
-   (each computes 64 of the 128 output channels).  flags bit 0: set the base-offset field of the
-   shifted descriptors.  n_ctas <= 0 picks 148.
+/* 3x3 convolution (padding 1) + bias (+ residual) (+ ReLU) on the tensor cores (tcgen05/TMEM/TMA), revision 2:
+   nn.Conv2d + folded BatchNorm + ReLU of the trunk.
+   act_in bf16 [n][256][c_in] in the padded tile layout described at the top of rz_net_tc2.cu (position
+   p = y*16+x, zero pad squares), c_in in {64,128}; weight bf16 [9][128][c_in] (tap = kh*3+kw, then out channel,
+   then in channel); bias f32 [128]; residual/act_out bf16 [n][256][128] (residual may alias act_out, may be NULL).
+   The 9x128x128 weights stay resident in shared memory, split over a CTA pair (tcgen05 cta_group::2 MMAs, cluster
+   of 2; cta_group must be 2), and each 128-position activation tile is loaded once with its 17-row halo; the 9 taps
+   are row-shifted UMMA descriptors on that tile.  flags bit 0: set the base-offset field of the shifted
+   descriptors; bit 1 (2) is accepted and ignored.  n_ctas <= 0 picks 148.
    Programmatic dependent launch: this kernel, rev. 3, the stems, the heads and the tree kernels of a wave are launched
    with cudaLaunchAttributeProgrammaticStreamSerialization and call griddepcontrol.wait before they read or write
    anything another kernel of the stream touches (RZ_PDL=0 in the environment turns it off).  flags bit 9 (512; for
@@ -552,18 +543,14 @@ int rz_net_conv3x3_tc2(const void* act_in, const void* weight, const float* bias
 /* the last trunk layer with the heads' two 1x1 convolutions + ReLU (act_conv1 128->4, val_conv1 128->2,
    policy_value_net.py:41,47) applied in its epilogue: writes ONLY feat f32 [n][6][256] (filter, then
    position p = y*16+x); the trunk output never reaches HBM.  w1x1_host [6][128] / b1x1_host [6] are
-   HOST float32 arrays (copied into the launch parameters).  Feed feat to rz_net_heads(.., 2, ..). */
-int rz_net_conv3x3_tc2_head(const void* act_in, const void* weight, const float* bias, const void* residual,
-                            int n_boards, int board_size, int board_cols, int c_in, int relu,
-                            const float* w1x1_host, const float* b1x1_host, float* feat, int n_ctas,
-                            void* stream);
-/* the same with the kernel's mode flags: 16 = split input (act_in = [hi 0..63 | lo 0..63], the bf16 high parts and
+   HOST float32 arrays (copied into the launch parameters).  Feed feat to rz_net_heads(.., 2, ..).
+   flags 0, 512 (static weights, as above) or the kernel's mode flags: 16 = split input (act_in = [hi 0..63 | lo 0..63], the bf16 high parts and
    rounding residues of a 64-channel float32-accurate activation; weight = [tap][128][Whi 0..63 | Wlo 0..63]; three
    products per tap: hi*Whi + lo*Whi + hi*Wlo), 32 = the 1x1 head convolutions read the float32 accumulators instead
    of bf16-rounded activations.  Together: conv3 (64 -> 128) + act_conv1 / val_conv1 of the reference's own
    PolicyValueNet at float32-level accuracy on the tensor cores.  Likewise rz_net_conv3x3_tc2 accepts flags 8 =
-   split output (64 real output channels written as [hi 0..63 | lo 0..63]; needs flag 2), 64 = float32 output (act_out
-   is float [rows][128]; needs flag 2, no residual), 128 = only the first 96 input channels are issued, 256 = N = 64 MMAs
+   split output (64 real output channels written as [hi 0..63 | lo 0..63]), 64 = float32 output (act_out
+   is float [rows][128]; no residual), 128 = only the first 96 input channels are issued, 256 = N = 64 MMAs
    for a layer with 64 output channels (with flag 8; weight rows 0..31 / 64..95 hold output channels 0..31 / 32..63), and
    the `relu` argument of
    rz_net_stem_tc / rz_net_stem_tc_planes bit 1 = 32-channel float32-accurate stem: weight rows 0..31 / 32..63 hold
@@ -577,10 +564,10 @@ int rz_net_conv3x3_tc2_head_ex(const void* act_in, const void* weight, const flo
    memory across all layers (ping-pong halo tiles written by the epilogue, the rows next to the seam between the two
    CTAs also into the peer's tile through distributed shared memory); the weights of all layers stream through a ring
    of taps; the MMAs, their order and the epilogue arithmetic are those of rz_net_conv3x3_tc2, so the results are
-   bit-identical to n_layers launches of it followed by the fused-heads epilogue of rz_net_conv3x3_tc2_head.
+   bit-identical to n_layers launches of it followed by the fused-heads epilogue of rz_net_conv3x3_tc2_head_ex.
    act_in bf16 [n][256][128] (the stem's output); weights bf16 [n_layers][9][128][128] (layer, tap, out channel, in
    channel); biases f32 [n_layers][128]; bit l of relu_mask: ReLU after layer l; bit l of res_mask: layer l adds the
-   input of layer l-1 (the block's skip connection) before its ReLU; feat f32 [n][6][256] as _tc2_head.  n_layers <= 24.
+   input of layer l-1 (the block's skip connection) before its ReLU; feat f32 [n][6][256] as _tc2_head_ex.  n_layers <= 24.
    Weights and biases are STATIC in the sense of flag 512 above. */
 int rz_net_trunk_small(const void* act_in, const void* weights, const float* biases, int n_layers,
                        unsigned relu_mask, unsigned res_mask, int n_boards, int board_size, int board_cols,
@@ -638,12 +625,12 @@ int rz_net_conv3x3_f32(const float* in, const float* weight, const float* bias, 
 /* both heads from the 128-channel trunk output: logp f32 [n][AS] = log_softmax(policy logits)
    (0 in the padding), value f32 [n] = tanh(...).  act_is_tile_bf16 = 0: act is f32 [n][HW][128];
    1: bf16 padded layout [n][S*S][128]; 2: act is the f32 [n][6][S*S] feature tensor written by
-   rz_net_conv3x3_tc2_head / _tc3_head (the 1x1 convolutions are already applied); S = h->row_stride, or
+   rz_net_conv3x3_tc2_head_ex / _tc3_head (the 1x1 convolutions are already applied); S = h->row_stride, or
    when that is 0 the smallest of 8 / 16 / 20 above max(H, W). */
 int rz_net_heads(const rz_heads_desc* h, const void* act, int act_is_tile_bf16, float* logp,
                  float* value, int n_boards, void* stream);
 /* the heads' two 1x1 convolutions + ReLU alone (policy_value_net.py:41,47): act bf16 padded layout
-   [n*S*S][128] -> feat f32 [n][6][S*S], the tensor rz_net_conv3x3_tc2_head / _tc3_head write from their
+   [n*S*S][128] -> feat f32 [n][6][S*S], the tensor rz_net_conv3x3_tc2_head_ex / _tc3_head write from their
    epilogue (same summation order: bit-identical at the board's squares). */
 int rz_net_head_features(const rz_heads_desc* h, const void* act, float* feat, int n_boards, void* stream);
 /* the fully connected layers of both heads on the tensor cores (act_fc1 + log_softmax, val_fc1 + ReLU +

@@ -11,7 +11,7 @@ import torch  # noqa: F401  -- loads libcudart.so.12 into the process before our
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'librlzero_b200.so')
 
-ABI_VERSION = 10
+ABI_VERSION = 11
 META_STRIDE = 12
 (META_PLAYER, META_LAST_MOVE, META_STONES, META_STATUS, META_WINNER, META_PLY, META_FAULT,
  META_EPISODE, META_KO, META_PASSES) = range(10)
@@ -97,7 +97,6 @@ SIGNATURES = {
     'rz_gomoku_winner': (C.c_int, [_GD, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_gomoku_encode_f32': (C.c_int, [_GD, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_gomoku_encode_nhwc_f32': (C.c_int, [_GD, _vp, _vp, _vp, C.c_int, _vp]),
-    'rz_gomoku_encode_tc': (C.c_int, [_GD, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_go_reset': (C.c_int, [_GD, _vp, _vp, _vp, C.c_int, C.c_int, _vp]),
     'rz_go_step': (C.c_int, [_GD, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_go_legal_mask': (C.c_int, [_GD, _vp, _vp, _vp, C.c_int, _vp]),
@@ -158,12 +157,8 @@ SIGNATURES = {
     'rz_mz_select': (C.c_int, [C.POINTER(MzDesc), _vp]),
     'rz_mz_expand_backup': (C.c_int, [C.POINTER(MzDesc), _vp, _vp, _vp]),
     'rz_mz_gather': (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_longlong, _vp]),
-    'rz_net_conv3x3_tc': (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int,
-                                    C.c_int, _vp]),
     'rz_net_conv3x3_tc2': (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_int, _vp]),
-    'rz_net_conv3x3_tc2_head': (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp,
-                                          _vp, _vp, C.c_int, _vp]),
     'rz_debug_set_probe': (C.c_int, [_vp]),
     'rz_net_trunk_small_ex': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_uint, C.c_uint, C.c_uint, C.c_uint, C.c_int, C.c_int,
                                          C.c_int, C.c_int, _vp, _vp, _vp, _vp]),

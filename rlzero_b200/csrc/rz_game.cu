@@ -1,8 +1,6 @@
 // rlzero_b200 -- batched GomokuEnv kernels (one warp per game) and closed-form evaluators.
 // Reference: rlzero/games/gomoku/gomoku_env.py (reset 33-47, step 49-70, leagel_actions 72-73,
 // current_state 95-114, has_a_winner 116-170, game_end_winner 196-203).
-#include <cuda_bf16.h>
-
 #include "rz_board.cuh"
 #include "rz_go.cuh"
 
@@ -148,45 +146,6 @@ rz_gomoku_encode_nhwc_kernel(rz_game_desc gd, const uint32_t* rows, const int32_
     const int r = pos / W, c = pos - r * W;
     const float v = rz_plane_value(b, mine, theirs, plane, r, c, W);
     if (i < total) planes[(size_t)g * total + i] = v;
-  }
-}
-
-// bf16 [n][256 positions][64 channels]: position p = y*16 + x, channels 0..3 = the 4 planes.
-// One 16-byte store per (position, 8-channel group); only group 0 carries data.
-__global__ void __launch_bounds__(RZ_GAME_THREADS)
-rz_gomoku_encode_tc_kernel(rz_game_desc gd, const uint32_t* rows, const int32_t* meta,
-                           __nv_bfloat16* act, int n) {
-  const int g = blockIdx.x * RZ_GAME_WARPS + (threadIdx.x >> 5);
-  if (g >= n) return;
-  const int lane = rz_lane(), H = gd.board_size, W = gd.width > 0 ? gd.width : gd.board_size;
-  rz_wboard b;
-  rz_board_load(b, rows + (size_t)g * 2 * H, meta + (size_t)g * RZ_META_STRIDE, H);
-  const uint32_t mine = b.p[b.player], theirs = b.p[b.player ^ 1];
-  uint4* out = reinterpret_cast<uint4*>(act + (size_t)g * 256 * 64);
-  const float colour = (b.stones & 1) ? 0.0f : 1.0f;
-  for (int p0 = 0; p0 < 256; p0 += 32) {
-    const int p = p0 + lane;
-    const int y = p >> 4, x = p & 15;
-    const uint32_t mrow = __shfl_sync(RZ_FULL, mine, y & 31);
-    const uint32_t trow = __shfl_sync(RZ_FULL, theirs, y & 31);
-    const bool inside = (y < H) && (x < W);
-    float f0 = 0.f, f1 = 0.f, f2 = 0.f, f3 = 0.f;
-    if (inside) {
-      f0 = (float)((mrow >> x) & 1u);
-      f1 = (float)((trow >> x) & 1u);
-      f2 = (b.stones > 0 && b.last_move == y * W + x) ? 1.0f : 0.0f;
-      f3 = colour;
-    }
-    __nv_bfloat162 lo = __floats2bfloat162_rn(f0, f1), hi = __floats2bfloat162_rn(f2, f3);
-    uint4 v0;
-    v0.x = *reinterpret_cast<uint32_t*>(&lo);
-    v0.y = *reinterpret_cast<uint32_t*>(&hi);
-    v0.z = 0u; v0.w = 0u;
-    const uint4 z = make_uint4(0u, 0u, 0u, 0u);
-    uint4* dst = out + (size_t)p * 8;  // 64 bf16 = 8 x 16 B
-    dst[0] = v0;
-#pragma unroll
-    for (int j = 1; j < 8; ++j) dst[j] = z;
   }
 }
 
@@ -463,18 +422,6 @@ extern "C" int rz_gomoku_encode_nhwc_f32(const rz_game_desc* g, const uint32_t* 
   rz_gomoku_encode_nhwc_kernel<<<rz_grid(n_games, RZ_GAME_WARPS), RZ_GAME_THREADS, 0,
                                  (cudaStream_t)stream>>>(*g, rows, meta, planes, n_games);
   RZ_LAUNCH_CHECK("rz_gomoku_encode_nhwc_f32");
-  return 0;
-}
-
-extern "C" int rz_gomoku_encode_tc(const rz_game_desc* g, const uint32_t* rows, const int32_t* meta,
-                                   void* act_bf16, int n_games, void* stream) {
-  if (rz_check_line_game(g)) return -1;
-  RZ_REQUIRE(rows && meta && act_bf16 && n_games >= 0, "rz_gomoku_encode_tc: bad arguments");
-  RZ_REQUIRE(g->board_size <= 15, "rz_gomoku_encode_tc: the 16x16 tile layout holds boards up to 15x15");
-  if (n_games == 0) return 0;
-  rz_gomoku_encode_tc_kernel<<<rz_grid(n_games, RZ_GAME_WARPS), RZ_GAME_THREADS, 0,
-                               (cudaStream_t)stream>>>(*g, rows, meta, (__nv_bfloat16*)act_bf16, n_games);
-  RZ_LAUNCH_CHECK("rz_gomoku_encode_tc");
   return 0;
 }
 

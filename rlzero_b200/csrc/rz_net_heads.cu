@@ -9,7 +9,7 @@
 //
 // The fp32 convolution is the plain CUDA-core path used for the reference's stock network
 // (3 layers, <= 64 input channels) at any board size; the benchmark trunk runs on the tensor
-// cores (rz_net_tc.cu).  The heads kernel serves both (template on the activation layout).
+// cores (rz_net_tc2.cu).  The heads kernel serves both (template on the activation layout).
 #include <cuda_bf16.h>
 #include <string.h>
 
@@ -240,7 +240,7 @@ __global__ void __launch_bounds__(HEAD_THREADS, 2) rz_heads_kernel(const HeadsPa
   const int nb = min(HEAD_NB, p.n_boards - b0);
   if (kSrc == SRC_FEAT) {
     // phase 1': the 1x1 convolutions were applied by the last trunk layer's epilogue
-    // (rz_net_conv3x3_tc2_head): gather feat[b][f][y*16+x] (coalesced along x) into k-major order
+    // (rz_net_conv3x3_tc2_head_ex): gather feat[b][f][y*16+x] (coalesced along x) into k-major order
     const int FP = 6 * p.P;   // floats per board in feat[b][f][y*S+x]
     const float* feat = reinterpret_cast<const float*>(p.act) + (size_t)b0 * FP;
     // iterate over the padded positions of [bi][f] (coalesced), 4 loads in flight

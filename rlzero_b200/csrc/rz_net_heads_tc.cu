@@ -2,7 +2,7 @@
 //
 // Reference ops (rlzero/games/gomoku/policy_value_net.py): act_fc1 (4HW -> A) + log_softmax (:42-44),
 // val_fc1 (2HW -> 64) + ReLU, val_fc2 (64 -> 1), tanh (:48-51), applied to the 6 head features per square
-// that the last trunk layer's epilogue (rz_net_conv3x3_tc2_head / _tc3_head) or rz_net_head_features wrote.
+// that the last trunk layer's epilogue (rz_net_conv3x3_tc2_head_ex / _tc3_head) or rz_net_head_features wrote.
 //
 // The CUDA-core heads kernel (rz_net_heads.cu) spends 211 us on 8192 boards of 15x15 (3.8 GFLOP of fp32 FMAs
 // through shared memory) and 721 us at 19x19.  Here the two FCs are one GEMM per 128 boards:

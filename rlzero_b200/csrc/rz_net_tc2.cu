@@ -3,13 +3,21 @@
 //
 // Reference op: nn.Conv2d(C, 128, kernel_size=3, padding=1) (+ folded BatchNorm, residual add,
 // ReLU), trunk of rlzero/games/gomoku/policy_value_net.py:14-16,36-38 / the ResNet-N trunk of
-// SURVEY.md section 7.  Same tensors and layouts as rz_net_tc.cu (act[b][p = y*16+x][c] bf16 with
-// zero pad squares, w[tap][cout][cin]).
+// SURVEY.md section 7.
 //
-// Why: revision 1 streams a 128x64 activation tile AND a 128x64 weight tile from L2 for every
-// (tap, k-block) -- 128 B/clk/SM, 8.5-11 GB of L2->SM traffic per layer against 1.07 GB
-// algorithmic (profiles/r1_run4_*): it is L2-bandwidth bound at ~50 % tensor-pipe activity.
-// Here
+// Data layout (bf16, channels last, one 16x16 tile of positions per board):
+//   act[b][p][c], p = y*16 + x; squares with x >= H or y >= H hold ZERO in every activation
+//   tensor.  With row stride 16 > H the zero column x = 15 is at once the right halo of row y
+//   and the left halo of row y+1, and the zero row y = 15 is the bottom halo of board b and the
+//   top halo of board b+1, so the input of tap (dy,dx) for 128 consecutive output positions is
+//   simply the 128 consecutive rows starting dy*16+dx further on: no im2col buffer, no boundary
+//   code (rows before the tensor start are zero-filled by TMA).
+//   w[tap][cout][cin] (K-major B operand), tap = kh*3 + kw.
+//
+// Why: revision 1 of this convolution (since removed) streamed a 128x64 activation tile AND a
+// 128x64 weight tile from L2 for every (tap, k-block) -- 128 B/clk/SM, 8.5-11 GB of L2->SM traffic
+// per layer against 1.07 GB algorithmic (profiles/r1_run4_*): it was L2-bandwidth bound at ~50 %
+// tensor-pipe activity.  Here
 //   * the 9 x 128 x 128 weights stay in shared memory for the whole launch.  295 KB do not fit one
 //     SM, so two CTAs form a pair: each keeps the 64 output channels it contributes as the B
 //     operand of a cta_group::2 MMA (147 KB), the pair computes 256 positions x 128 channels;
@@ -20,10 +28,6 @@
 // for operands inside a tile (72 back-to-back tcgen05.mma per tile).  At the start of a launch the
 // first activation tile is requested before the weights, which complete on one mbarrier per tap, so
 // the first tile's MMAs begin after 16 KB of weights instead of all 147 KB.
-//
-// kCG = 2: the production kernel (cluster of 2).  kCG = 1: the same data path on a single CTA
-// (UMMA 128x64, each CTA computes one half of the output channels) -- kept as a bisecting aid
-// and for odd SM counts.
 #include <cuda_bf16.h>
 
 #include "rz_common.cuh"
@@ -47,7 +51,7 @@ struct Conv2Params {
   const float* bias;               // [128]
   const __nv_bfloat16* residual;   // [rows][128] or null
   __nv_bfloat16* out;              // [rows][128]  (flags bit 6: float [rows][128] instead)
-  int n_items;                     // kCG=2: boards; kCG=1: half boards
+  int n_items;                     // boards
   int board;                       // H (rows)
   int board_w;                     // W (columns)
   int kblocks;                     // Cin / 64
@@ -66,18 +70,13 @@ struct HeadTaps {
   float* feat;                     // [n_boards][6][256] float32, position index p = y*16 + x
 };
 
-// kDirect: the epilogue writes its output rows straight from registers with 256-bit global stores (one full
-// 32-byte sector per lane and instruction) instead of staging them in the A buffer for a TMA store, so the A
-// buffer goes back to the producer as soon as the tile's MMAs are done: the reload of the next-but-one tile
-// starts one epilogue earlier and has a whole MMA period to land.
-template <int kCG, bool kHead, bool kDirect>
+template <bool kHead>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
                       const __grid_constant__ CUtensorMap tmap_w,
                       const __grid_constant__ CUtensorMap tmap_out, const Conv2Params p,
                       const __grid_constant__ HeadTaps head) {
-  static_assert(!kHead || kCG == 2, "the fused 1x1 heads need all 128 channels of a row in one thread");
-  constexpr int ACC_N = (kCG == 2) ? 128 : 64;     // accumulator columns per buffer
+  constexpr int ACC_N = 128;                       // accumulator columns per buffer
   // fused-heads layer: 16 more columns (two slots of 8) carry the upper channel half's partial sums from one warp of a
   // lane quarter to the other; the allocation is a power of two
   constexpr int TMEM_COLS = kHead ? 512 : 2 * ACC_N;
@@ -96,8 +95,8 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
   // warp index and cluster rank through a shuffle: values the compiler can prove warp-uniform, so the
   // role branches below are uniform and the MMA issuer's operands live in uniform registers
   const int warp = rz::uniform_i32((int)(threadIdx.x >> 5)), lane = threadIdx.x & 31;
-  const uint32_t rank = (kCG == 2) ? rz::uniform_u32(rz::cluster_ctarank()) : 0u;
-  const int half = (kCG == 2) ? (int)rank : (int)(blockIdx.x & 1);   // which 64 output channels live here
+  const uint32_t rank = rz::uniform_u32(rz::cluster_ctarank());
+  const int half = (int)rank;                      // which 64 output channels live here
   const bool leader = rank == 0;
   const int worker = blockIdx.x >> 1, n_workers = gridDim.x >> 1;
 
@@ -116,23 +115,20 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
       rz::mbar_init(bar_afull + 8 * b, 1);
       rz::mbar_init(bar_aempty + 8 * b, 1);
       rz::mbar_init(bar_tfull + 8 * b, 1);
-      rz::mbar_init(bar_tempty + 8 * b, 8 * kCG);
+      rz::mbar_init(bar_tempty + 8 * b, 16);
     }
     rz::fence_barrier_init();
   }
-  if (warp == 1) {
-    if (kCG == 2) { rz::tmem_alloc_pair(rz::smem_u32(tmem_holder), TMEM_COLS); rz::tmem_relinquish_pair(); }
-    else          { rz::tmem_alloc(rz::smem_u32(tmem_holder), TMEM_COLS); rz::tmem_relinquish(); }
-  }
+  if (warp == 1) { rz::tmem_alloc_pair(rz::smem_u32(tmem_holder), TMEM_COLS); rz::tmem_relinquish_pair(); }
   if (threadIdx.x >= 64 && threadIdx.x < 192) s_bias[threadIdx.x - 64] = p.bias[threadIdx.x - 64];
   rz::tc_fence_before();
-  if (kCG == 2) rz::cluster_sync_all(); else __syncthreads();
+  rz::cluster_sync_all();
   rz::tc_fence_after();
   const uint32_t tmem_base = *tmem_holder;
 
   // first row of this CTA's 128 output positions for work item `item`
   auto row_of = [&](int item) -> int {
-    return (kCG == 2) ? item * 256 + (int)rank * TILE_M : item * TILE_M;
+    return item * 256 + (int)rank * TILE_M;
   };
 
   if (early_w && threadIdx.x != 0) rz::grid_dep_wait();   // thread 0 (the producer) first requests the weights
@@ -142,12 +138,11 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
     if (lane == 0) {
       auto load_weights = [&]() {
         for (int tap = 0; tap < 9; ++tap) {
-          const uint32_t l_btap = (kCG == 2) ? rz::mapa_shared(bar_btap + 8 * tap, 0) : bar_btap + 8 * tap;
-          if (leader) rz::mbar_expect_tx(bar_btap + 8 * tap, (uint32_t)(kCG * p.kblocks * B_TILE_BYTES));
+          const uint32_t l_btap = rz::mapa_shared(bar_btap + 8 * tap, 0);
+          if (leader) rz::mbar_expect_tx(bar_btap + 8 * tap, (uint32_t)(2 * p.kblocks * B_TILE_BYTES));
           for (int kb = 0; kb < p.kblocks; ++kb) {
             const uint32_t dst = smem_base + (uint32_t)(tap * 2 + kb) * B_TILE_BYTES;
-            if (kCG == 2) rz::tma_load_2d_pair(dst, &tmap_w, l_btap, kb * 64, tap * 128 + half * 64);
-            else          rz::tma_load_2d(dst, &tmap_w, l_btap, kb * 64, tap * 128 + half * 64);
+            rz::tma_load_2d_pair(dst, &tmap_w, l_btap, kb * 64, tap * 128 + half * 64);
           }
         }
       };
@@ -157,13 +152,12 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
       for (int item = worker; item < p.n_items; item += n_workers, ++it) {
         const int buf = it & 1;
         rz::mbar_wait(bar_aempty + 8 * buf, ((uint32_t)(it >> 1) & 1u) ^ 1u);
-        const uint32_t l_afull = (kCG == 2) ? rz::mapa_shared(bar_afull + 8 * buf, 0) : bar_afull + 8 * buf;
-        if (leader) rz::mbar_expect_tx(bar_afull + 8 * buf, (uint32_t)(kCG * p.kblocks * A_KB_BYTES));
+        const uint32_t l_afull = rz::mapa_shared(bar_afull + 8 * buf, 0);
+        if (leader) rz::mbar_expect_tx(bar_afull + 8 * buf, (uint32_t)(2 * p.kblocks * A_KB_BYTES));
         const int row0 = row_of(item) - HALO;
         for (int kb = 0; kb < p.kblocks; ++kb) {
           const uint32_t dst = a_base + (uint32_t)buf * A_BUF_BYTES + (uint32_t)kb * A_KB_BYTES;
-          if (kCG == 2) rz::tma_load_2d_pair(dst, &tmap_act, l_afull, kb * 64, row0);
-          else          rz::tma_load_2d(dst, &tmap_act, l_afull, kb * 64, row0);
+          rz::tma_load_2d_pair(dst, &tmap_act, l_afull, kb * 64, row0);
         }
         if (it == 0 && !early_w) load_weights();      // right behind the first activation tile
       }
@@ -172,10 +166,9 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
     // ===== MMA issuer: the whole warp of the leader CTA runs the loop (converged, uniform operands);
     // one elected lane issues each tcgen05.mma / commit =====
     if (leader) {
-      // flags bit 8 (pair kernel): the layer has only 64 output channels -- N = 64 MMAs (each CTA supplies the first 32
-      // rows of its weight tiles: output channels 0..31 / 32..63), accumulator columns 0..63
-      const uint32_t idesc = (kCG == 2 && (p.flags & 256)) ? rz::umma_idesc_bf16(256, 64)
-                                                           : rz::umma_idesc_bf16(kCG == 2 ? 256 : 128, ACC_N);
+      // flags bit 8: the layer has only 64 output channels -- N = 64 MMAs (each CTA supplies the first 32 rows of its
+      // weight tiles: output channels 0..31 / 32..63), accumulator columns 0..63
+      const uint32_t idesc = (p.flags & 256) ? rz::umma_idesc_bf16(256, 64) : rz::umma_idesc_bf16(256, ACC_N);
       const uint32_t issue = rz::elect_one();
       const uint32_t tmem_u = rz::uniform_u32(tmem_base);
       int it = 0;
@@ -208,17 +201,15 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
 #pragma unroll
             for (int kk = 0; kk < 4; ++kk) {
               if (kk < n_kk) {
-                if (kCG == 2) rz::umma_bf16_pair_pred(d_tmem, adesc + (uint64_t)(2 * kk), bdesc + (uint64_t)(2 * kk), idesc, acc, issue);
-                else          rz::umma_bf16_pred(d_tmem, adesc + (uint64_t)(2 * kk), bdesc + (uint64_t)(2 * kk), idesc, acc, issue);
+                rz::umma_bf16_pair_pred(d_tmem, adesc + (uint64_t)(2 * kk), bdesc + (uint64_t)(2 * kk), idesc, acc, issue);
                 acc = 1;
               }
             }
           }
         }
         // accumulator complete: both CTAs drain their half; the A buffers are recycled by the
-        // epilogues (they stage the output tile in them), not here
-        if (kCG == 2) rz::umma_commit_pair_pred(bar_tfull + 8 * buf, 3, issue);
-        else          rz::umma_commit_pred(bar_tfull + 8 * buf, issue);
+        // epilogues, not here
+        rz::umma_commit_pair_pred(bar_tfull + 8 * buf, 3, issue);
       }
     }
   } else if (!kHead) {
@@ -226,18 +217,19 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
     // row x half the channels per thread.  Two warps per scheduler and half the serial work per thread:
     // with a single warp per quarter the epilogue (TMEM drain, bias/residual/ReLU, bf16 packing, staging)
     // took longer than the tile's 72 MMAs and set the pace of the kernel (profiles/r1_run24_*).
-    // TMEM -> registers -> (+bias, +residual, ReLU, pad mask, bf16) -> shared-memory staging in the
-    // A buffer the tile's MMAs have just finished with -> TMA store.  The A buffer is handed back
-    // to the producer (a_empty) once the store has read it.
+    // TMEM -> registers -> (+bias, +residual, ReLU, pad mask, bf16) -> 256-bit global stores straight
+    // from registers (one full 32-byte sector per lane and instruction).  Nothing is staged in shared
+    // memory, so the A buffer goes back to the producer (a_empty) as soon as the tile's MMAs are done:
+    // the reload of the next-but-one tile starts one epilogue earlier and has a whole MMA period to land.
     const int q = warp & 3;
     const int hsel = (warp - 2) >> 2;
-    constexpr int HALF = ACC_N / 2;                 // columns per thread: 64 (pair) / 32 (single CTA)
+    constexpr int HALF = ACC_N / 2;                 // columns per thread
     constexpr int NCHH = HALF / 32;                 // 32-column TMEM chunks per thread
-    const int col0 = ((kCG == 2) ? 0 : half * 64) + hsel * HALF;   // first output channel of this thread
-    // flags bit 3 (split output, pair kernel): the layer has 64 real output channels (accumulator columns 0..63);
+    const int col0 = hsel * HALF;                   // first output channel of this thread
+    // flags bit 3 (split output): the layer has 64 real output channels (accumulator columns 0..63);
     // the row leaves as [hi 0..63 | lo 0..63], hi = bf16(x), lo = bf16(x - hi): warps with hsel = 0 write the high
     // parts, their partners read the SAME columns and write the rounding residues
-    const bool split_out = (kCG == 2) && (p.flags & 8);
+    const bool split_out = (p.flags & 8) != 0;
     const int csrc = split_out ? 0 : hsel * HALF;                    // first accumulator column this thread reads
     const int r_in_tile = q * 32 + lane;
     auto row_valid = [&](int item_) {
@@ -279,13 +271,12 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
         rz::tc_fence_before();
         __syncwarp();
         if (lane == 0) {
-          if (kCG == 2) rz::mbar_arrive_cluster_relaxed(rz::mapa_shared(bar_tempty + 8 * buf, 0));
-          else          rz::mbar_arrive(bar_tempty + 8 * buf);
+          rz::mbar_arrive_cluster_relaxed(rz::mapa_shared(bar_tempty + 8 * buf, 0));
           if (warp == 2) rz::mbar_arrive(bar_aempty + 8 * buf);
         }
         continue;
       }
-      if (kDirect && warp == 2 && lane == 0) rz::mbar_arrive(bar_aempty + 8 * buf);   // MMAs done: A tile is dead
+      if (warp == 2 && lane == 0) rz::mbar_arrive(bar_aempty + 8 * buf);   // MMAs done: A tile is dead
       // all of this thread's accumulator columns in flight at once, one wait
       uint32_t acc[NCHH][32];
 #pragma unroll
@@ -295,16 +286,7 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
       // accumulator drained: the MMA issuer may overwrite it (no memory payload -> relaxed)
       rz::tc_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (kCG == 2) rz::mbar_arrive_cluster_relaxed(rz::mapa_shared(bar_tempty + 8 * buf, 0));
-        else          rz::mbar_arrive(bar_tempty + 8 * buf);
-      }
-      // staging row: k-block (64 columns) `kbs` is a [128 rows][128 B] tile with the 128-byte swizzle of the
-      // absolute shared-memory address, as the TMA store expects; this thread owns 16-byte chunks c0.. of it
-      const int kbs = (hsel * HALF) >> 6;
-      const uint32_t chunk0 = (uint32_t)(((hsel * HALF) & 63) >> 3);
-      const uint32_t srow = a_base + (uint32_t)buf * A_BUF_BYTES + (uint32_t)kbs * (TILE_M * 128u) + (uint32_t)r_in_tile * 128u;
-      const uint32_t sw = (srow >> 7) & 7u;
+      if (lane == 0) rz::mbar_arrive_cluster_relaxed(rz::mapa_shared(bar_tempty + 8 * buf, 0));
       const float4* bias4 = reinterpret_cast<const float4*>(s_bias + (split_out ? csrc : col0));
       uint32_t pair8[8];
 #pragma unroll
@@ -331,7 +313,7 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
             }
             if (!valid) packed[e] = 0u;
           }
-          if (kDirect && (p.flags & 64)) {
+          if (p.flags & 64) {
             // float32 output (the training step of the reference's own network keeps conv3's activation and the data
             // gradients at accumulator precision): 8 channels = one 32-byte store
             uint32_t f8[8];
@@ -345,30 +327,16 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
               f8[e * 2 + 1] = valid ? __float_as_uint(v1) : 0u;
             }
             rz::st_global_v8(reinterpret_cast<float*>(p.out) + row * 128 + col0 + ch * 32 + j * 8, f8);
-          } else if (kDirect) {
+          } else {
 #pragma unroll
             for (int e = 0; e < 4; ++e) pair8[(j & 1) * 4 + e] = packed[e];
             if (j & 1) rz::st_global_v8(p.out + row * 128 + col0 + ch * 32 + (j - 1) * 8, pair8);
-          } else {
-            const uint32_t chunk = chunk0 + (uint32_t)(ch * 4 + j);
-            rz::st_shared_v4(srow + ((chunk ^ sw) << 4), packed[0], packed[1], packed[2], packed[3]);
           }
         }
       }
-      if (kDirect) continue;
-      rz::fence_proxy_async();              // staging writes -> visible to the TMA engine
-      rz::named_bar_sync(1, 256);           // the 8 epilogue warps
-      if (warp == 2 && lane == 0) {
-        const uint32_t stage = a_base + (uint32_t)buf * A_BUF_BYTES;
-        const int cb = (kCG == 2) ? 0 : half * 64;
-#pragma unroll
-        for (int kb = 0; kb < ACC_N / 64; ++kb)
-          rz::tma_store_2d(&tmap_out, stage + (uint32_t)kb * (TILE_M * 128u), cb + kb * 64, row0);
-        rz::tma_store_commit();
-        rz::tma_store_wait_read();
-        rz::mbar_arrive(bar_aempty + 8 * buf);   // this CTA's producer may refill the buffer
-      }
     }
+    // no bulk store is outstanding here, so this waits for nothing; dropping it changes the kernel's register
+    // allocation, which wants a measured A/B of its own
     if (warp == 2 && lane == 0) rz::tma_store_wait_all();
   } else {
     // ===== fused-heads layer (kHead): the same 8 epilogue warps; every thread turns its 64 channels of a row
@@ -478,20 +446,19 @@ rz_conv3x3_tc2_kernel(const __grid_constant__ CUtensorMap tmap_act,
   }
 
   rz::tc_fence_before();
-  if (kCG == 2) rz::cluster_sync_all(); else __syncthreads();
+  rz::cluster_sync_all();
   if (warp == 1) {
     rz::tc_fence_after();
-    if (kCG == 2) rz::tmem_dealloc_pair(tmem_base, TMEM_COLS);
-    else          rz::tmem_dealloc(tmem_base, TMEM_COLS);
+    rz::tmem_dealloc_pair(tmem_base, TMEM_COLS);
   }
 }
 
-template <int kCG, bool kHead, bool kDirect>
+template <bool kHead>
 int launch(const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& to, const Conv2Params& p,
            const HeadTaps& head, int ctas, cudaStream_t stream) {
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(rz_conv3x3_tc2_kernel<kCG, kHead, kDirect>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(rz_conv3x3_tc2_kernel<kHead>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e != cudaSuccess) { rz_set_error("rz_net_conv3x3_tc2: smem attribute: %s", cudaGetErrorString(e)); return -2; }
     attr_set = true;
   }
@@ -502,12 +469,12 @@ int launch(const CUtensorMap& ta, const CUtensorMap& tw, const CUtensorMap& to, 
   cfg.stream = stream;
   cudaLaunchAttribute attr[2];
   attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = kCG;
+  attr[0].val.clusterDim.x = 2;
   attr[0].val.clusterDim.y = 1;
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1 + rz_pdl_attr(&attr[1]);
-  cudaError_t e = cudaLaunchKernelEx(&cfg, rz_conv3x3_tc2_kernel<kCG, kHead, kDirect>, ta, tw, to, p, head);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, rz_conv3x3_tc2_kernel<kHead>, ta, tw, to, p, head);
   if (e != cudaSuccess) { rz_set_error("rz_net_conv3x3_tc2: launch failed: %s", cudaGetErrorString(e)); return -2; }
   return 0;
 }
@@ -523,15 +490,13 @@ static int conv2_entry(const void* act_in, const void* weight, const float* bias
   RZ_REQUIRE(board_size >= 1 && board_size <= 15, "rz_net_conv3x3_tc2: board_size %d not in [1,15]", board_size);
   RZ_REQUIRE(board_cols >= 1 && board_cols <= 15, "rz_net_conv3x3_tc2: board_cols %d not in [1,15]", board_cols);
   RZ_REQUIRE(c_in == 64 || c_in == 128, "rz_net_conv3x3_tc2: c_in %d (64 or 128)", c_in);
-  RZ_REQUIRE(cta_group == 1 || cta_group == 2, "rz_net_conv3x3_tc2: cta_group %d (1 or 2)", cta_group);
+  RZ_REQUIRE(cta_group == 2, "rz_net_conv3x3_tc2: cta_group %d (the kernel runs on CTA pairs: 2)", cta_group);
   RZ_REQUIRE(act_in != act_out, "rz_net_conv3x3_tc2: in-place convolution is not supported");
-  RZ_REQUIRE(!(flags & (8 | 16)) || (cta_group == 2 && c_in == 128),
-             "rz_net_conv3x3_tc2: the split modes (flags 8 / 16) need the pair kernel and c_in = 128");
-  RZ_REQUIRE(!(flags & 8) || (flags & 2) || feat, "rz_net_conv3x3_tc2: split output (flag 8) needs the direct-store epilogue (flag 2)");
-  RZ_REQUIRE(!(flags & 256) || ((flags & 8) && cta_group == 2), "rz_net_conv3x3_tc2: N = 64 (flag 256) goes with the split output (flag 8)");
+  RZ_REQUIRE(!(flags & (8 | 16)) || c_in == 128, "rz_net_conv3x3_tc2: the split modes (flags 8 / 16) need c_in = 128");
+  RZ_REQUIRE(!(flags & 256) || (flags & 8), "rz_net_conv3x3_tc2: N = 64 (flag 256) goes with the split output (flag 8)");
   RZ_REQUIRE(!(flags & 128) || !(flags & 16), "rz_net_conv3x3_tc2: flags 128 (96 input channels) and 16 (split input) exclude each other");
-  RZ_REQUIRE(!(flags & 64) || ((flags & 2) && cta_group == 2 && !(flags & 8) && !residual && !feat),
-             "rz_net_conv3x3_tc2: float32 output (flag 64) needs the direct-store pair kernel, no residual, no split output");
+  RZ_REQUIRE(!(flags & 64) || (!(flags & 8) && !residual && !feat),
+             "rz_net_conv3x3_tc2: float32 output (flag 64) needs no residual and no split output");
   if (n_boards == 0) return 0;
   static HeadTaps head;   // ~3 KB: filled per call, copied into the launch parameters
   CUtensorMap tmap_act, tmap_w, tmap_out;
@@ -544,25 +509,23 @@ static int conv2_entry(const void* act_in, const void* weight, const float* bias
   p.bias = bias;
   p.residual = (const __nv_bfloat16*)residual;
   p.out = (__nv_bfloat16*)act_out;
-  p.n_items = cta_group == 2 ? n_boards : n_boards * 2;
+  p.n_items = n_boards;
   p.board = board_size;
   p.board_w = board_cols;
   p.kblocks = c_in / 64;
   p.relu = relu;
   p.flags = flags;
   int ctas = n_ctas > 0 ? n_ctas : 148;
-  ctas &= ~1;                                       // workers are CTA pairs in both modes
+  ctas &= ~1;                                       // workers are CTA pairs
   if (ctas < 2) ctas = 2;
   if (ctas / 2 > p.n_items) ctas = 2 * p.n_items;   // every worker gets at least one item
   if (feat) {
     for (int i = 0; i < 6 * 128; ++i) head.w[i] = w1x1_host[i];
     for (int i = 0; i < 6; ++i) head.b[i] = b1x1_host[i];
     head.feat = feat;
-    return launch<2, true, false>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream);
+    return launch<true>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream);
   }
-  if (cta_group == 2 && (flags & 2)) return launch<2, false, true>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream);
-  return cta_group == 2 ? launch<2, false, false>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream)
-                        : launch<1, false, false>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream);
+  return launch<false>(tmap_act, tmap_w, tmap_out, p, head, ctas, (cudaStream_t)stream);
 }
 
 extern "C" int rz_net_conv3x3_tc2(const void* act_in, const void* weight, const float* bias,
@@ -572,15 +535,6 @@ extern "C" int rz_net_conv3x3_tc2(const void* act_in, const void* weight, const 
   RZ_REQUIRE(act_out, "rz_net_conv3x3_tc2: null output");
   return conv2_entry(act_in, weight, bias, residual, act_out, n_boards, board_size, board_cols, c_in, relu, cta_group, flags,
                      n_ctas, nullptr, nullptr, nullptr, stream);
-}
-
-extern "C" int rz_net_conv3x3_tc2_head(const void* act_in, const void* weight, const float* bias,
-                                       const void* residual, int n_boards, int board_size, int board_cols,
-                                       int c_in, int relu, const float* w1x1_host, const float* b1x1_host,
-                                       float* feat, int n_ctas, void* stream) {
-  RZ_REQUIRE(w1x1_host && b1x1_host && feat, "rz_net_conv3x3_tc2_head: null head argument");
-  return conv2_entry(act_in, weight, bias, residual, nullptr, n_boards, board_size, board_cols, c_in, relu, 2, 0, n_ctas,
-                     w1x1_host, b1x1_host, feat, stream);
 }
 
 extern "C" int rz_net_conv3x3_tc2_head_ex(const void* act_in, const void* weight, const float* bias,

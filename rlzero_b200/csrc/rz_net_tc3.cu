@@ -9,7 +9,7 @@
 //
 // Layout: act[row][c] bf16 with row = board*P + y*S + x, P = S*S, S = 16 (boards up to 15x15) or
 // 20 (up to 19x19); squares with x >= W or y >= H hold zero, which gives every tap its halo (see
-// rz_net_tc.cu).  Tiles are 128 consecutive rows and need not be aligned to boards (P = 400 is not
+// rz_net_tc2.cu).  Tiles are 128 consecutive rows and need not be aligned to boards (P = 400 is not
 // a multiple of 128); the tensor is padded to a multiple of 256 rows.
 //
 // What changes against revision 2, and why: the halo tile of stride 20 has 128 + 2*21 = 170 rows;

@@ -17,7 +17,7 @@
 //   * the weights of all layers stream through an 8-slot ring of taps (16 KB per CTA and tap), the producer running up
 //     to 8 taps ahead across layer boundaries; they are static, so the stream starts before the grid dependency
 //     resolves (programmatic dependent launch, rz_common.cuh);
-//   * the last layer's epilogue applies the heads' 1x1 convolutions exactly as rz_net_conv3x3_tc2_head does.
+//   * the last layer's epilogue applies the heads' 1x1 convolutions exactly as rz_net_conv3x3_tc2_head_ex does.
 // One pair per board: n_boards pairs run side by side (up to 74 at once on 148 SMs).
 #include <cuda_bf16.h>
 
@@ -277,7 +277,7 @@ rz_trunk_small_kernel(const __grid_constant__ CUtensorMap tmap_act, const __grid
         if (lane == 0) rz::mbar_arrive_cluster(l_aready);
         if (p.probe && board == 0 && leader && warp == 2 && lane == 0) p.probe[l * 8 + 7] = rz::globaltimer_ns();
       } else {
-        // the heads' 1x1 convolutions on the bf16-rounded activations of the last layer, as rz_net_conv3x3_tc2_head:
+        // the heads' 1x1 convolutions on the bf16-rounded activations of the last layer, as rz_net_conv3x3_tc2_head_ex:
         // channels in ascending order, the upper half's partial sums handed over through the (dead) input tile
         float hacc[6];
 #pragma unroll

@@ -156,8 +156,8 @@ class NativeForward(object):
     graph_capturable = True
     prior_is_log = True       # the network emits log-probabilities (policy_value_net.py:44)
 
-    def __init__(self, module, mode=None, max_batch=1, device='cuda', n_ctas=0, conv_rev=2, fused_stem=True,
-                 fused_head=True, game_type=None, row_stride=None, heads_tc=True):
+    def __init__(self, module, mode=None, max_batch=1, device='cuda', n_ctas=0, fused_head=True, game_type=None,
+                 row_stride=None, heads_tc=True):
         if not torch.cuda.is_available():
             raise L.NativeLibraryError('NativeForward needs a CUDA device (no CPU fallback)')
         self.lib = L.load()
@@ -210,22 +210,19 @@ class NativeForward(object):
         self.mode = mode
         self.n_ctas = int(n_ctas)
         # the heads' 1x1 convolutions inside the last trunk layer's epilogue (rz_net_tc2.cu, kHead)
-        self.fused_head = bool(fused_head) and int(conv_rev) >= 2
+        self.fused_head = bool(fused_head)
         self.weights_version = 0
-        self.fused_stem = bool(fused_stem)  # encoder + first conv in one kernel (rz_net_stem.cu)
         # the heads' fully connected layers on the tensor cores (rz_net_heads_tc.cu; bf16 hi/lo split, fp32-level
         # accuracy); False keeps the CUDA-core heads kernel
         self.heads_tc = (bool(heads_tc) and mode == 'tc') or mode == 'tc32'
-        # 3: rz_net_tc3.cu (any row stride; forced for 19x19); 2: rz_net_tc2.cu (stride 16); 1: rz_net_tc.cu
-        self.conv_rev = int(conv_rev)
-        # rz_net_conv3x3_tc2 flags: bit 1 = direct-store epilogue, the default (853 k vs 840 k sims/s sustained on
-        # one box, profiles/r1_run24_bench_ab.log; bit-identical tensors); RZ_CONV_FLAGS=0 selects the staged TMA store
         import os
         # boards up to which the one-launch trunk of rz_net_trunk_small.cu is used (one CTA pair per board, 74 pairs at a
         # time on 148 SMs; measured crossover with the per-layer kernels near 200 boards, profiles/r2_run43_crossover.log);
         # RZ_SMALL_BATCH_MAX=0 turns it off
         self.small_batch_max = int(os.environ.get('RZ_SMALL_BATCH_MAX', '148'))
-        self.conv_flags = int(os.environ.get('RZ_CONV_FLAGS', '514'))   # 2 | 512: direct store, static weights
+        # flags of the 128 -> 128 rz_net_conv3x3_tc2 launches, read by MuZeroNative and bench.py too: 512 = static
+        # weights (include/rlzero_b200.h); bit 1 (2) is accepted and ignored
+        self.conv_flags = 514
         self.max_batch = 0
         self.refresh_weights()
         self._alloc(max_batch)
@@ -417,7 +414,6 @@ class NativeForward(object):
         if self.mode in ('tc', 'tc32'):
             bf = torch.bfloat16
             rows = (n * self.P + 255) // 256 * 256          # the convolutions work on pairs of 128-row tiles
-            self.act0 = torch.zeros(n, 256, 64, dtype=bf, device=dev) if self.S == 16 else None
             self.bufs = [torch.zeros(rows, 128, dtype=bf, device=dev) for _ in range(2)]
             self.feat = torch.zeros(n, 6, self.P, dtype=torch.float32, device=dev)
         else:
@@ -434,7 +430,14 @@ class NativeForward(object):
             return L.GameDesc(self.H, 1, self.A, self.AS, self.W, self.game_type, 0.0, 0, rs)
         return L.GameDesc(self.H, min(k, max(self.H, self.W)), self.A, self.AS, self.W, self.game_type, 0.0, 0, rs)
 
-    def _trunk_and_heads(self, n, logp, value, stem_done=False):
+    def _tc_stem(self):
+        """The fused encoder + first convolution (rz_net_stem.cu) that starts every tensor-core forward."""
+        if self.stem is None:
+            raise ValueError("mode 'tc' needs a first layer the fused stem takes: 4 input planes without BatchNorm, "
+                             "or Go's 17 planes")
+        return self.stem
+
+    def _trunk_and_heads(self, n, logp, value):
         s = L.stream_ptr()
         lib = self.lib
         if self.mode == 'tc32' and self.trunk_small is not None and n <= self.small_batch_max:
@@ -461,8 +464,7 @@ class NativeForward(object):
             L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
                     'rz_net_heads_tc')
             return
-        if (self.mode == 'tc' and stem_done and self.trunk_small is not None and n <= self.small_batch_max
-                and self.fused_head and self.conv_rev == 2):
+        if self.mode == 'tc' and self.trunk_small is not None and n <= self.small_batch_max and self.fused_head:
             # few boards (a sequential search evaluates ONE): the whole trunk in one launch, one CTA pair per board
             ts = self.trunk_small
             L.check(lib.rz_net_trunk_small(
@@ -477,23 +479,21 @@ class NativeForward(object):
                         'rz_net_heads')
             return
         if self.mode == 'tc':
-            # ping-pong: the residual of a block is the buffer its second conv overwrites
-            src, outs = self.act0, self.bufs
-            cur = 0 if stem_done else -1   # index in outs holding the latest activation, -1 = act0
-            for i, l in enumerate(self.layers):
-                if stem_done and i == 0:
-                    continue
-                dst = 0 if cur != 0 else 1
+            # ping-pong behind the stem, which wrote bufs[0]: the residual of a block is the buffer its second conv
+            # overwrites.  The layer layout picks the kernel: rz_net_tc2.cu for stride 16, rz_net_tc3.cu otherwise.
+            outs = self.bufs
+            cur = 0   # index in outs holding the latest activation
+            for i, l in enumerate(self.layers[1:], 1):
+                dst = 1 - cur
                 res = None
                 if l['skip'] is not None:
                     # skip always refers to the activation two layers back = the other buffer
                     res = outs[dst]
-                inp = src if cur < 0 else outs[cur]
-                rev3 = (self.conv_rev == 3 or self.S != 16) and l['cin'] == 128
+                inp = outs[cur]
                 w1p = self.w1x1_host.ctypes.data_as(C.c_void_p)
                 b1p = self.b1x1_host.ctypes.data_as(C.c_void_p)
-                if self.fused_head and i == len(self.layers) - 1 and l['cin'] == 128:
-                    if rev3:
+                if self.fused_head and i == len(self.layers) - 1:
+                    if self.S != 16:
                         L.check(lib.rz_net_conv3x3_tc3_head(
                             L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res), n, self.H, self.W, self.S,
                             int(l['relu']) | 2, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc3_head')
@@ -508,20 +508,14 @@ class NativeForward(object):
                         L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(self.feat), 2, L.ptr(logp),
                                                  L.ptr(value), n, s), 'rz_net_heads')
                     return
-                if rev3:
+                if self.S != 16:
                     L.check(lib.rz_net_conv3x3_tc3(L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res),
                                                    L.ptr(outs[dst]), n, self.H, self.W, self.S, int(l['relu']) | 2,
                                                    self.n_ctas, s), 'rz_net_conv3x3_tc3')
-                elif self.S != 16:
-                    raise ValueError('19x19 boards need the fused stem (the generic first layer is stride-16 only)')
-                elif self.conv_rev >= 2:
+                else:
                     L.check(lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res),
                                                    L.ptr(outs[dst]), n, self.H, self.W, l['cin'],
                                                    int(l['relu']), 2, self.conv_flags, self.n_ctas, s), 'rz_net_conv3x3_tc2')
-                else:
-                    L.check(lib.rz_net_conv3x3_tc(L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res),
-                                                  L.ptr(outs[dst]), n, self.H, l['cin'], int(l['relu']),
-                                                  self.n_ctas, s), 'rz_net_conv3x3_tc')
                 cur = dst
             if self.heads_tc:
                 L.check(lib.rz_net_head_features(C.byref(self.hdesc), L.ptr(outs[cur]), L.ptr(self.feat), n, s),
@@ -556,12 +550,11 @@ class NativeForward(object):
                 return 3                                    # stem, conv2 + conv3 + 1x1 heads in one launch, FC heads
             return 4                                        # stem, conv2, conv3 + 1x1 heads, FC heads
         if (n is not None and self.mode == 'tc' and self.trunk_small is not None and n <= self.small_batch_max
-                and self.fused_head and self.conv_rev == 2 and self.stem is not None and self.fused_stem):
+                and self.fused_head):
             return 3                                        # stem, one-launch trunk + 1x1 heads, FC heads
         n_conv = len(self.layers)
-        fused = self.mode == 'tc' and self.stem is not None and self.fused_stem
         heads = 2 if (self.heads_tc and not self.fused_head) else 1   # [1x1 features +] FC heads
-        return (1 + n_conv - 1 if fused else 1 + n_conv) + heads  # [stem | encode + conv0] + convs + heads
+        return (n_conv if self.mode == 'tc' else 1 + n_conv) + heads  # [stem + convs | encode + convs] + heads
 
     def forward_boards(self, rows, meta, n, logp=None, value=None, hist=None):
         """Positions in the device board layout -> (logp [n][AS], value [n]) float32 tensors.
@@ -570,7 +563,6 @@ class NativeForward(object):
         logp = self.logp if logp is None else logp
         value = self.value if value is None else value
         g = self._gdesc()
-        stem_done = False
         if self.game_type == L.GAME_GO:
             st = self.stem
             if hist is None:
@@ -578,32 +570,23 @@ class NativeForward(object):
             L.check(self.lib.rz_net_stem_go_tc(C.byref(g), L.ptr(rows), L.ptr(hist), L.ptr(meta), L.ptr(st['w']),
                                                L.ptr(st['b']), L.ptr(self.bufs[0]), n, int(st['relu']), 0,
                                                L.stream_ptr()), 'rz_net_stem_go_tc')
-            stem_done = True
-        elif self.mode in ('tc', 'tc32') and self.stem is not None and self.fused_stem:
-            st = self.stem
+        elif self.mode in ('tc', 'tc32'):
+            st = self._tc_stem()
             L.check(self.lib.rz_net_stem_tc(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(st['w']), L.ptr(st['b']),
                                             L.ptr(self.bufs[0]), n, int(st['relu']), 0, L.stream_ptr()),
                     'rz_net_stem_tc')
-            stem_done = True
-        elif self.mode == 'tc':
-            if self.S != 16:
-                raise ValueError('19x19 boards need the fused stem')
-            L.check(self.lib.rz_gomoku_encode_tc(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(self.act0), n,
-                                                 L.stream_ptr()), 'rz_gomoku_encode_tc')
         else:
             L.check(self.lib.rz_gomoku_encode_nhwc_f32(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(self.act0),
                                                        n, L.stream_ptr()), 'rz_gomoku_encode_nhwc_f32')
-        self._trunk_and_heads(n, logp, value, stem_done)
+        self._trunk_and_heads(n, logp, value)
         return logp[:n], value[:n]
 
     def forward_planes(self, planes):
         """[n,4,H,W] float planes (current_state format) -> (logp [n][A], value [n]).  Used by
-        AlphaZeroAgent.policy_value / predict (alphazero_agent.py:48-57,88-97); the plane -> kernel
-        layout repack is a handful of torch ops (off the search path)."""
+        AlphaZeroAgent.policy_value / predict (alphazero_agent.py:48-57,88-97)."""
         x = torch.as_tensor(planes, dtype=torch.float32, device=self.device)
         n = x.shape[0]
         self._alloc(n)
-        stem_done = False
         if self.game_type == L.GAME_GO:
             st = self.stem
             xc = x.contiguous()
@@ -611,25 +594,17 @@ class NativeForward(object):
             L.check(self.lib.rz_net_stem_go_tc_planes(C.byref(g), L.ptr(xc), L.ptr(st['w']), L.ptr(st['b']),
                                                       L.ptr(self.bufs[0]), n, int(st['relu']), 0, L.stream_ptr()),
                     'rz_net_stem_go_tc_planes')
-            stem_done = True
-        elif self.mode in ('tc', 'tc32') and self.stem is not None and self.fused_stem:
+        elif self.mode in ('tc', 'tc32'):
             # same kernel (and therefore bit-identical stem outputs) as forward_boards
-            st = self.stem
+            st = self._tc_stem()
             xc = x.contiguous()
             g = self._gdesc()
             L.check(self.lib.rz_net_stem_tc_planes(C.byref(g), L.ptr(xc), L.ptr(st['w']), L.ptr(st['b']),
                                                    L.ptr(self.bufs[0]), n, int(st['relu']), 0, L.stream_ptr()),
                     'rz_net_stem_tc_planes')
-            stem_done = True
-        elif self.mode == 'tc':
-            if self.S != 16:
-                raise ValueError('19x19 boards need the fused stem')
-            self.act0[:n].zero_()
-            t = self.act0[:n].view(n, 16, 16, 64)
-            t[:, :self.H, :self.W, :4] = x.permute(0, 2, 3, 1).to(torch.bfloat16)
         else:
             self.act0[:n] = x.permute(0, 2, 3, 1).reshape(n, self.HW, 4)
-        self._trunk_and_heads(n, self.logp, self.value, stem_done)
+        self._trunk_and_heads(n, self.logp, self.value)
         return self.logp[:n, :self.A], self.value[:n]
 
     def __call__(self, forest):

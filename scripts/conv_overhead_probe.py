@@ -18,7 +18,7 @@ def main():
     torch.manual_seed(0)
     w = (torch.randn(9, 128, 128, device='cuda') * 0.03).to(torch.bfloat16).contiguous()
     b = torch.zeros(128, device='cuda')
-    flags = (4 if 'noepilogue' in sys.argv else 0) | (2 if 'direct' in sys.argv else 0)
+    flags = 4 if 'noepilogue' in sys.argv else 0
     pts = []
     for rounds in (4, 8, 16, 32, 64, 110):
         B = 74 * rounds

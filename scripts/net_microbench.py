@@ -40,13 +40,6 @@ def main():
 
     flops_alg = 2.0 * B * H * H * 128 * 128 * 9
     flops_issued = 2.0 * B * 256 * 128 * 128 * 9
-    if nf.S == 16:
-        def conv():
-            L.check(lib.rz_net_conv3x3_tc(L.ptr(x), L.ptr(l['w']), L.ptr(l['b']), None, L.ptr(y), B, H, 128, 1,
-                                          ctas, L.stream_ptr()))
-        ms = timeit(conv)
-        print(json.dumps({'kernel': 'conv3x3_tc', 'B': B, 'ms': ms, 'TFLOPs_algorithmic': flops_alg / ms / 1e9,
-                          'TFLOPs_issued': flops_issued / ms / 1e9}))
     z = nf.bufs[1]
     for name, res in (('conv3x3_tc3', None), ('conv3x3_tc3+residual', z)):
         def conv3():
@@ -75,12 +68,12 @@ def main():
     import ctypes as C
 
     def conv_head():
-        L.check(lib.rz_net_conv3x3_tc2_head(L.ptr(x), L.ptr(l['w']), L.ptr(l['b']), L.ptr(z), B, H, H, 128, 1,
-                                            nf.w1x1_host.ctypes.data_as(C.c_void_p),
-                                            nf.b1x1_host.ctypes.data_as(C.c_void_p), L.ptr(nf.feat), ctas,
-                                            L.stream_ptr()))
+        L.check(lib.rz_net_conv3x3_tc2_head_ex(L.ptr(x), L.ptr(l['w']), L.ptr(l['b']), L.ptr(z), B, H, H, 128, 1, 0,
+                                               nf.w1x1_host.ctypes.data_as(C.c_void_p),
+                                               nf.b1x1_host.ctypes.data_as(C.c_void_p), L.ptr(nf.feat), ctas,
+                                               L.stream_ptr()))
     ms = timeit(conv_head)
-    print(json.dumps({'kernel': 'conv3x3_tc2_head+residual', 'ms': ms, 'TFLOPs_issued': flops_issued / ms / 1e9}))
+    print(json.dumps({'kernel': 'conv3x3_tc2_head_ex+residual', 'ms': ms, 'TFLOPs_issued': flops_issued / ms / 1e9}))
     rows = torch.zeros(B, 2, H, dtype=torch.int32, device='cuda')
     meta = torch.zeros(B, 12, dtype=torch.int32, device='cuda')
     meta[:, 1] = -1

@@ -33,6 +33,20 @@ def test_header_symbols_exported(lib):
     assert sorted(_lib.SIGNATURES) == syms
 
 
+def test_superseded_convolutions_are_not_exported(lib):
+    """Revision 1 of the trunk convolution, its plane encoder and the flag-less fused-heads entry point are gone
+    (rz_net_conv3x3_tc2 / rz_net_stem_tc / rz_net_conv3x3_tc2_head_ex do their work)."""
+    for s in ('rz_net_conv3x3_tc', 'rz_gomoku_encode_tc', 'rz_net_conv3x3_tc2_head'):
+        assert not hasattr(lib, s), s
+
+
+def test_conv3x3_tc2_rejects_single_cta_groups(lib):
+    """rz_net_conv3x3_tc2 runs on CTA pairs only: cta_group 1 is rejected on the host before any launch."""
+    dummy = C.c_void_p(16)
+    rc = lib.rz_net_conv3x3_tc2(dummy, dummy, dummy, None, C.c_void_p(32), 1, 15, 15, 128, 1, 1, 514, 0, None)
+    assert rc != 0 and b'cta_group' in lib.rz_last_error()
+
+
 def test_abi_version_and_struct_sizes(lib):
     from rlzero_b200 import _lib
     assert lib.rz_abi_version() == _lib.ABI_VERSION

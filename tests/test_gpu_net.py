@@ -24,7 +24,7 @@ def _from_tile(t, h):
     return t.reshape(n, 16, 16, c)[:, :h, :h, :].permute(0, 3, 1, 2).float()
 
 
-@pytest.mark.parametrize('rev', ['v1', 'v2_pair', 'v2_single', 'v3'])
+@pytest.mark.parametrize('rev', ['v2_pair', 'v3'])
 @pytest.mark.parametrize('n,h,cin,relu,res', [(1, 15, 128, 1, 0), (3, 15, 128, 1, 1), (5, 9, 64, 0, 0),
                                               (300, 15, 128, 1, 1), (2, 3, 64, 1, 0), (37, 15, 64, 1, 0)])
 def test_conv3x3_tc_matches_torch(n, h, cin, relu, res, rev):
@@ -59,13 +59,9 @@ def test_conv3x3_tc_matches_torch(n, h, cin, relu, res, rev):
         L.check(lib.rz_net_conv3x3_tc3(L.ptr(xt), L.ptr(wt), L.ptr(b.contiguous()), L.ptr(rt), L.ptr(out),
                                        n, h, h, 16, relu, 0, L.stream_ptr()), 'conv3')
         out = out[:n]
-    elif rev == 'v1':
-        L.check(lib.rz_net_conv3x3_tc(L.ptr(xt), L.ptr(wt), L.ptr(b.contiguous()), L.ptr(rt), L.ptr(out),
-                                      n, h, cin, relu, 0, L.stream_ptr()), 'conv')
     else:
         L.check(lib.rz_net_conv3x3_tc2(L.ptr(xt), L.ptr(wt), L.ptr(b.contiguous()), L.ptr(rt), L.ptr(out),
-                                       n, h, h, cin, relu, 2 if rev == 'v2_pair' else 1, 0, 0, L.stream_ptr()),
-                'conv2')
+                                       n, h, h, cin, relu, 2, 0, 0, L.stream_ptr()), 'conv2')
     torch.cuda.synchronize()
     got = _from_tile(out, h).double()
     err = (got - ref).abs().max().item()
@@ -265,9 +261,9 @@ def test_agent_api_shapes():
 
 
 @pytest.mark.parametrize('size,n', [(15, 70), (9, 33), (6, 5)])
-def test_fused_stem_matches_encode_plus_conv(size, n):
-    """rz_net_stem_tc (planes built from the bitboards inside the kernel, K = 36) against
-    rz_gomoku_encode_tc + the generic convolution, and against PyTorch on current_state planes."""
+def test_stem_kernel_matches_torch_and_planes_stem(size, n):
+    """rz_net_stem_tc (planes built from the bitboards inside the kernel, K = 36) against PyTorch on
+    current_state planes, with zero pad squares, and bit-identical to the planes-fed stem."""
     from oracle import pyoracle
     from rlzero_b200 import _lib as L
     from rlzero_b200.games.gomoku.gomoku_env import GomokuEnv
@@ -286,25 +282,14 @@ def test_fused_stem_matches_encode_plus_conv(size, n):
         envs.append(e)
     rows = torch.cat([e.device_state()[0] for e in envs]).cuda()
     meta = torch.cat([e.device_state()[1] for e in envs]).cuda()
-    # row_stride=16: this test compares against the legacy stride-16 encode + conv route (a 6x6 board would
-    # otherwise use the 8-stride layout, covered by test_row_stride_8_*)
+    # row_stride=16: the 8-stride layout a 6x6 board would otherwise use is covered by test_row_stride_8_*
     nf = NativeForward(net, max_batch=n, row_stride=16)
     lib, g = L.load(), nf._gdesc()
     st = nf.stem
     fused = torch.full((n, 256, 128), 3.0, dtype=torch.bfloat16, device='cuda')
     L.check(lib.rz_net_stem_tc(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(st['w']), L.ptr(st['b']), L.ptr(fused),
                                n, 1, 0, L.stream_ptr()), 'stem')
-    act0 = torch.zeros(n, 256, 64, dtype=torch.bfloat16, device='cuda')
-    L.check(lib.rz_gomoku_encode_tc(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(act0), n, L.stream_ptr()), 'enc')
-    l0 = nf.layers[0]
-    plain = torch.full((n, 256, 128), 5.0, dtype=torch.bfloat16, device='cuda')
-    L.check(lib.rz_net_conv3x3_tc2(L.ptr(act0), L.ptr(l0['w']), L.ptr(l0['b']), None, L.ptr(plain), n, size, size,
-                                   64, 1, 2, 0, 0, L.stream_ptr()), 'conv')
     torch.cuda.synchronize()
-    # same bf16 products, fp32 accumulation in a different order: equal up to one bf16 ulp
-    d = (fused.float() - plain.float()).abs()
-    assert d.max().item() <= 2.0 ** -7 * max(1.0, plain.float().abs().max().item())
-    assert (d == 0).float().mean().item() > 0.98
     full = fused.reshape(n, 16, 16, 128).float()
     assert full[:, size:].abs().max().item() == 0.0 and full[:, :, size:].abs().max().item() == 0.0
     # against PyTorch on the reference's observation planes (weights rounded to bf16 like the kernel's)
@@ -313,13 +298,8 @@ def test_fused_stem_matches_encode_plus_conv(size, n):
     ref = torch.relu(torch.nn.functional.conv2d(planes, wq, net.stem.bias.detach(), padding=1))
     got = _from_tile(fused, size)
     assert (got - ref).abs().max().item() <= 2.0 ** -8 * max(1.0, ref.abs().max().item()) + 1e-6
-    # and the whole forward through both routes
     lp1, v1 = nf.forward_boards(rows, meta, n)
     lp1, v1 = lp1.clone(), v1.clone()
-    nf2 = NativeForward(net, max_batch=n, fused_stem=False, row_stride=16)
-    lp2, v2 = nf2.forward_boards(rows, meta, n)
-    assert (lp1[:, :size * size] - lp2[:, :size * size]).abs().max().item() < 2e-3
-    assert (v1 - v2).abs().max().item() < 2e-3
     # the planes-fed variant of the kernel (AlphaZeroAgent.policy_value_fn on a host env) is
     # bit-identical to the bitboard-fed one: search parity with a Python-side evaluator relies on it
     lp3, v3 = nf.forward_planes(planes.cpu().numpy())
@@ -328,7 +308,7 @@ def test_fused_stem_matches_encode_plus_conv(size, n):
 
 @pytest.mark.parametrize('size,blocks,n', [(15, 2, 70), (9, 1, 37), (6, 1, 3)])
 def test_fused_head_matches_separate_heads(size, blocks, n):
-    """The 1x1 head convolutions inside the last layer's epilogue (rz_net_conv3x3_tc2_head) give
+    """The 1x1 head convolutions inside the last layer's epilogue (rz_net_conv3x3_tc2_head_ex) give
     the same logits / values as storing the trunk output and running the heads kernel on it."""
     from rlzero_b200.games.gomoku.policy_value_net import NativeForward, ResNetPolicyValueNet
     torch.manual_seed(size + 1)
@@ -510,16 +490,14 @@ def test_conv3x3_tc3_any_stride_matches_torch(n, h, w, relu, res, S):
     assert out[n * S * S:].abs().max().item() == 0.0 if out.shape[0] > n * S * S else True
 
 
-@pytest.mark.parametrize('size,blocks,n', [(19, 3, 9), (15, 2, 6)])
-def test_resnet_forward_rev3_vs_torch_and_rev2(size, blocks, n):
-    """Whole forward on the revision-3 convolution: 19x19 against PyTorch fp32 (1e-3), and at 15x15
-    bit-identical to the revision-2 path (same MMAs in a different order of k-blocks would NOT be
-    identical, so this only checks closeness there)."""
+def test_resnet_forward_rev3_19x19_vs_torch():
+    """Whole 19x19 forward on the revision-3 convolution (row stride 20) against PyTorch fp32 (1e-3)."""
     from rlzero_b200.games.gomoku.policy_value_net import NativeForward, ResNetPolicyValueNet
+    size, blocks, n = 19, 3, 9
     torch.manual_seed(size)
     net = ResNetPolicyValueNet(size, n_blocks=blocks).cuda().eval()
-    nf = NativeForward(net, max_batch=n, conv_rev=3)
-    assert nf.mode == 'tc' and nf.S == (20 if size > 15 else 16)
+    nf = NativeForward(net, max_batch=n)
+    assert nf.mode == 'tc' and nf.S == 20
     x = _random_boards(n, size, 5)
     logp, v = (t.cpu() for t in nf.forward_planes(x))
     ref = ResNetPolicyValueNet(size, n_blocks=blocks).eval()
@@ -529,21 +507,33 @@ def test_resnet_forward_rev3_vs_torch_and_rev2(size, blocks, n):
     assert (logp.exp() - lt.exp()).abs().max().item() < 1e-3
     assert (v - vt.reshape(-1)).abs().max().item() < 1e-3
     # fused head on/off agree exactly on this path too
-    nf_b = NativeForward(net, max_batch=n, conv_rev=3, fused_head=False)
+    nf_b = NativeForward(net, max_batch=n, fused_head=False)
     lb, vb = (t.cpu() for t in nf_b.forward_planes(x))
     assert torch.equal(lb, logp) and torch.equal(vb, v)
-    if size <= 15:
-        nf2 = NativeForward(net, max_batch=n, conv_rev=2)
-        l2, v2 = (t.cpu() for t in nf2.forward_planes(x))
-        assert (l2.exp() - logp.exp()).abs().max().item() < 1e-4 and (v2 - v).abs().max().item() < 1e-3
+
+
+def test_tc_trunk_without_a_fusable_stem_is_rejected():
+    """Mode 'tc' starts every forward with the fused stem (4 planes without BatchNorm, or Go's 17): a trunk with any
+    other first layer still constructs -- MuZeroNative packs its dynamics trunk this way -- but does not run."""
+    from rlzero_b200.games.gomoku.policy_value_net import NativeForward, ResNetPolicyValueNet
+    from rlzero_b200.games.gomoku.gomoku_env import GomokuEnv
+    nf = NativeForward(ResNetPolicyValueNet(9, n_blocks=1, in_planes=8).cuda().eval())
+    assert nf.mode == 'tc' and nf.stem is None
+    e = GomokuEnv(9, 5)
+    e.reset()
+    rows, meta = e.device_state()[0].cuda(), e.device_state()[1].cuda()
+    with pytest.raises(ValueError, match='fused stem'):
+        nf.forward_boards(rows, meta, 1)
+    with pytest.raises(ValueError, match='fused stem'):
+        nf.forward_planes(np.zeros((1, 8, 9, 9), dtype=np.float32))
 
 
 @pytest.mark.parametrize('h,w,a,blocks,n', [(6, 7, 7, 3, 300), (6, 6, None, 2, 5), (3, 3, None, 1, 17), (7, 7, None, 1, 130)])
-def test_row_stride_8_forward_vs_torch_and_stride_16(h, w, a, blocks, n):
+def test_row_stride_8_forward_vs_torch_and_tc2_stride_16(h, w, a, blocks, n):
     """Boards up to 7x7 (Connect Four 6x7 = BASELINE config 2, TicTacToe 3x3) run on the 8-stride padded layout
-    (64 rows per board instead of 256): whole forward within 1e-3 of PyTorch fp32, fused head on/off and
-    planes-/bitboard-fed stems bit-identical, and the same network forced onto the 16-stride layout agrees (same
-    bf16 products; the accumulation order inside one MMA chain is the same, so the trunk is in fact identical)."""
+    (64 rows per board instead of 256, revision 3): whole forward within 1e-3 of PyTorch fp32, fused head on/off and
+    planes-/bitboard-fed stems bit-identical, and the same network forced onto the 16-stride layout, where revision 2
+    runs, agrees (same bf16 products; revision 2 sums them tap-outer, revision 3 k-block-outer)."""
     from rlzero_b200.games.gomoku.policy_value_net import NativeForward, ResNetPolicyValueNet
     torch.manual_seed(h * 10 + w)
     kw = dict(board_width=w, n_actions=a) if a is not None else dict(board_width=w)
@@ -564,7 +554,7 @@ def test_row_stride_8_forward_vs_torch_and_stride_16(h, w, a, blocks, n):
     assert nf_b.S == 8
     lb, vb = (t.cpu() for t in nf_b.forward_planes(x))
     assert torch.equal(lb[:, :A], logp[:, :A]) and torch.equal(vb, v)
-    nf16 = NativeForward(net, max_batch=n, row_stride=16, conv_rev=3)
+    nf16 = NativeForward(net, max_batch=n, row_stride=16)
     assert nf16.S == 16
     l16, v16 = (t.cpu() for t in nf16.forward_planes(x))
     assert (l16[:, :A].exp() - logp[:, :A].exp()).abs().max().item() < 1e-4 and (v16 - v).abs().max().item() < 1e-3
