@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define RZ_ABI_VERSION 11
+#define RZ_ABI_VERSION 12
 #define RZ_MAX_BOARD 19          /* rows live one per lane; A <= 362 (19x19 Go incl. the pass) */
 #define RZ_META_STRIDE 12
 #define RZ_GO_HIST 14            /* history planes a Go position carries besides the current board */
@@ -543,7 +543,7 @@ int rz_net_conv3x3_tc2(const void* act_in, const void* weight, const float* bias
 /* the last trunk layer with the heads' two 1x1 convolutions + ReLU (act_conv1 128->4, val_conv1 128->2,
    policy_value_net.py:41,47) applied in its epilogue: writes ONLY feat f32 [n][6][256] (filter, then
    position p = y*16+x); the trunk output never reaches HBM.  w1x1_host [6][128] / b1x1_host [6] are
-   HOST float32 arrays (copied into the launch parameters).  Feed feat to rz_net_heads(.., 2, ..).
+   HOST float32 arrays (copied into the launch parameters).  Feed feat to rz_net_heads_tc.
    flags 0, 512 (static weights, as above) or the kernel's mode flags: 16 = split input (act_in = [hi 0..63 | lo 0..63], the bf16 high parts and
    rounding residues of a 64-channel float32-accurate activation; weight = [tap][128][Whi 0..63 | Wlo 0..63]; three
    products per tap: hi*Whi + lo*Whi + hi*Wlo), 32 = the 1x1 head convolutions read the float32 accumulators instead
@@ -622,13 +622,10 @@ int rz_net_stem_go_tc_planes(const rz_game_desc* g, const float* planes, const v
 int rz_net_conv3x3_f32(const float* in, const float* weight, const float* bias, const float* residual,
                        float* out, int n_boards, int board_size, int c_in, int c_out, int relu,
                        void* stream);
-/* both heads from the 128-channel trunk output: logp f32 [n][AS] = log_softmax(policy logits)
-   (0 in the padding), value f32 [n] = tanh(...).  act_is_tile_bf16 = 0: act is f32 [n][HW][128];
-   1: bf16 padded layout [n][S*S][128]; 2: act is the f32 [n][6][S*S] feature tensor written by
-   rz_net_conv3x3_tc2_head_ex / _tc3_head (the 1x1 convolutions are already applied); S = h->row_stride, or
-   when that is 0 the smallest of 8 / 16 / 20 above max(H, W). */
-int rz_net_heads(const rz_heads_desc* h, const void* act, int act_is_tile_bf16, float* logp,
-                 float* value, int n_boards, void* stream);
+/* both heads on CUDA cores from the fp32 trunk output act f32 [n][HW][128] (channels last, as
+   rz_net_conv3x3_f32 writes it): logp f32 [n][AS] = log_softmax(policy logits) (0 in the padding),
+   value f32 [n] = tanh(...). */
+int rz_net_heads(const rz_heads_desc* h, const float* act, float* logp, float* value, int n_boards, void* stream);
 /* the heads' two 1x1 convolutions + ReLU alone (policy_value_net.py:41,47): act bf16 padded layout
    [n*S*S][128] -> feat f32 [n][6][S*S], the tensor rz_net_conv3x3_tc2_head_ex / _tc3_head write from their
    epilogue (same summation order: bit-identical at the board's squares). */

@@ -11,7 +11,7 @@ import torch  # noqa: F401  -- loads libcudart.so.12 into the process before our
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'librlzero_b200.so')
 
-ABI_VERSION = 11
+ABI_VERSION = 12
 META_STRIDE = 12
 (META_PLAYER, META_LAST_MOVE, META_STONES, META_STATUS, META_WINNER, META_PLY, META_FAULT,
  META_EPISODE, META_KO, META_PASSES) = range(10)
@@ -176,7 +176,7 @@ SIGNATURES = {
     'rz_net_stem_go_tc_planes': (C.c_int, [_GD, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     'rz_net_conv3x3_f32': (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, _vp]),
-    'rz_net_heads': (C.c_int, [C.POINTER(HeadsDesc), _vp, C.c_int, _vp, _vp, C.c_int, _vp]),
+    'rz_net_heads': (C.c_int, [C.POINTER(HeadsDesc), _vp, _vp, _vp, C.c_int, _vp]),
     'rz_net_head_features': (C.c_int, [C.POINTER(HeadsDesc), _vp, _vp, C.c_int, _vp]),
     'rz_net_heads_tc': (C.c_int, [C.POINTER(HeadsDesc), _vp, _vp, _vp, C.c_int, _vp]),
 }

@@ -8,8 +8,8 @@
 // weights are stored transposed ([in][out]) so that threads over `out` read them coalesced.
 //
 // The fp32 convolution is the plain CUDA-core path used for the reference's stock network
-// (3 layers, <= 64 input channels) at any board size; the benchmark trunk runs on the tensor
-// cores (rz_net_tc2.cu).  The heads kernel serves both (template on the activation layout).
+// (3 layers, <= 64 input channels) at any board size, and the heads kernel finishes it.  The
+// tensor-core trunks end in rz_net_heads_tc.cu, fed by the head-features kernel below.
 #include <cuda_bf16.h>
 #include <string.h>
 
@@ -143,7 +143,7 @@ constexpr int HEAD_THREADS = 256;
 constexpr int HEAD_C = 128;
 
 struct HeadsParams {
-  const void* act;        // trunk output: bf16 [B][256][128] (tile layout) or fp32 [B][HW][128]
+  const void* act;        // trunk output: fp32 [B][HW][128] (heads) or bf16 [B*P][128] (padded layout, features)
   const float* w1x1;      // [6][128]: 4 policy + 2 value 1x1 filters
   const float* b1x1;      // [6]
   const float* wp;        // [4*HW + 4][AS] policy FC, transposed + padded (4 zero rows at the end)
@@ -155,7 +155,7 @@ struct HeadsParams {
   float* logp;            // [B][AS]
   float* value;           // [B]
   int n_boards, H, W, HW, A, AS;   // H x W squares (HW), A policy outputs
-  int S, P;                        // padded layout of tile / feature sources: row stride S, P = S*S rows per board
+  int S, P;                        // padded layout of a bf16 source: row stride S, P = S*S rows per board
 };
 
 // 256-bit read-only global load: one full 32-byte sector per lane (sm_100 LDG.E.256)
@@ -223,9 +223,6 @@ __device__ __forceinline__ int feat_slot(int k, int bi) {
   return k * HEAD_NB + ((((bi >> 2) ^ (k & 3)) << 2) | (bi & 3));
 }
 
-enum { SRC_F32 = 0, SRC_TILE = 1, SRC_FEAT = 2 };
-
-template <int kSrc>
 __global__ void __launch_bounds__(HEAD_THREADS, 2) rz_heads_kernel(const HeadsParams p) {
   rz::grid_dep_wait();     // programmatic dependent launch: see rz_common.cuh
   rz::grid_dep_launch();
@@ -234,45 +231,21 @@ __global__ void __launch_bounds__(HEAD_THREADS, 2) rz_heads_kernel(const HeadsPa
   float* s_f = sm;                              // [6*HW][NB]  k-major features (policy 4*HW, then value 2*HW)
   float* s_lg = s_f + 6 * HW * HEAD_NB;         // [NB][AS]    logits
   float* s_h = s_lg + HEAD_NB * p.AS;           // [NB][64]    value hidden
-  float* s_w = s_h + HEAD_NB * 64;              // [6][128]    1x1 filters (not for SRC_FEAT)
+  float* s_w = s_h + HEAD_NB * 64;              // [6][128]    1x1 filters
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const int b0 = blockIdx.x * HEAD_NB;
   const int nb = min(HEAD_NB, p.n_boards - b0);
-  if (kSrc == SRC_FEAT) {
-    // phase 1': the 1x1 convolutions were applied by the last trunk layer's epilogue
-    // (rz_net_conv3x3_tc2_head_ex): gather feat[b][f][y*16+x] (coalesced along x) into k-major order
-    const int FP = 6 * p.P;   // floats per board in feat[b][f][y*S+x]
-    const float* feat = reinterpret_cast<const float*>(p.act) + (size_t)b0 * FP;
-    // iterate over the padded positions of [bi][f] (coalesced), 4 loads in flight
-    for (int i0 = tid; i0 < HEAD_NB * FP; i0 += 4 * HEAD_THREADS) {
-      float v[4];
+  for (int i = tid; i < 6 * HEAD_C; i += HEAD_THREADS) s_w[i] = p.w1x1[i];
+  __syncthreads();
+  // phase 1: 1x1 convolutions + ReLU  (policy_value_net.py:41, 47); boards beyond nb hold zeros
+  for (int i = tid; i < HEAD_NB * HW; i += HEAD_THREADS) {
+    const int bi = i % HEAD_NB, pos = i / HEAD_NB;
+    float acc[6];
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int i = i0 + u * HEAD_THREADS;
-        const int bi = i / FP;
-        v[u] = (i < HEAD_NB * FP && bi < nb) ? feat[i] : 0.0f;
-      }
+    for (int f = 0; f < 6; ++f) acc[f] = p.b1x1[f];
+    if (bi < nb) conv1x1_position<false>(p.act, b0 + bi, pos, p.W, HW, p.S, p.P, s_w, acc);
 #pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        const int i = i0 + u * HEAD_THREADS;
-        const int bi = i / FP, r = i - bi * FP;
-        const int f = r / p.P, t = r - f * p.P, y = t / p.S, x = t - y * p.S;
-        if (i < HEAD_NB * FP && x < p.W && y < p.H) s_f[feat_slot(f * HW + y * p.W + x, bi)] = v[u];
-      }
-    }
-  } else {
-    for (int i = tid; i < 6 * HEAD_C; i += HEAD_THREADS) s_w[i] = p.w1x1[i];
-    __syncthreads();
-    // phase 1: 1x1 convolutions + ReLU  (policy_value_net.py:41, 47); boards beyond nb hold zeros
-    for (int i = tid; i < HEAD_NB * HW; i += HEAD_THREADS) {
-      const int bi = i % HEAD_NB, pos = i / HEAD_NB;
-      float acc[6];
-#pragma unroll
-      for (int f = 0; f < 6; ++f) acc[f] = p.b1x1[f];
-      if (bi < nb) conv1x1_position<kSrc == SRC_TILE>(p.act, b0 + bi, pos, p.W, HW, p.S, p.P, s_w, acc);
-#pragma unroll
-      for (int f = 0; f < 6; ++f) s_f[feat_slot(f * HW + pos, bi)] = bi < nb ? fmaxf(acc[f], 0.0f) : 0.0f;
-    }
+    for (int f = 0; f < 6; ++f) s_f[feat_slot(f * HW + pos, bi)] = bi < nb ? fmaxf(acc[f], 0.0f) : 0.0f;
   }
   __syncthreads();
   // phase 2: policy FC (:43).  Thread (half, t): output columns t and t+128 of every 256-column
@@ -414,15 +387,6 @@ size_t heads_smem(int HW, int AS) {
   return sizeof(float) * ((size_t)HEAD_NB * 6 * HW + (size_t)HEAD_NB * AS + HEAD_NB * 64 + 6 * HEAD_C);
 }
 
-template <int kSrc>
-int heads_launch(const HeadsParams& p, size_t smem, int grid, cudaStream_t stream) {
-  cudaError_t e = cudaFuncSetAttribute(rz_heads_kernel<kSrc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) { rz_set_error("rz_net_heads: smem attribute: %s", cudaGetErrorString(e)); return -2; }
-  rz_launch_pdl(rz_heads_kernel<kSrc>, grid, HEAD_THREADS, smem, stream, p);
-  RZ_LAUNCH_CHECK("rz_net_heads");
-  return 0;
-}
-
 }  // namespace
 
 extern "C" int rz_net_conv3x3_f32(const float* in, const float* weight, const float* bias,
@@ -470,32 +434,29 @@ extern "C" int rz_net_conv3x3_f32(const float* in, const float* weight, const fl
   return 0;
 }
 
-extern "C" int rz_net_heads(const rz_heads_desc* h, const void* act, int act_is_tile_bf16, float* logp,
-                            float* value, int n_boards, void* stream) {
+extern "C" int rz_net_heads(const rz_heads_desc* h, const float* act, float* logp, float* value, int n_boards,
+                            void* stream) {
   RZ_REQUIRE(h && act && logp && value, "rz_net_heads: null argument");
   RZ_REQUIRE(h->w1x1 && h->b1x1 && h->wp && h->bp && h->wv1 && h->bv1 && h->wv2 && h->bv2,
              "rz_net_heads: null weight pointer");
   RZ_REQUIRE(h->board_size >= 1 && h->board_size <= RZ_MAX_BOARD, "rz_net_heads: board_size %d", h->board_size);
   const int W = h->width > 0 ? h->width : h->board_size;
   RZ_REQUIRE(W >= 1 && W <= RZ_MAX_BOARD, "rz_net_heads: width %d", W);
-  RZ_REQUIRE(!act_is_tile_bf16 || (h->board_size <= 19 && W <= 19), "rz_net_heads: padded layouts hold boards up to 19x19");
   const int HW = h->board_size * W;
   const int A = h->n_actions > 0 ? h->n_actions : HW;
   RZ_REQUIRE(h->action_stride >= A && (h->action_stride & 31) == 0, "rz_net_heads: action_stride %d", h->action_stride);
   if (n_boards <= 0) return 0;
   HeadsParams p;
+  memset(&p, 0, sizeof(p));
   p.act = act; p.w1x1 = h->w1x1; p.b1x1 = h->b1x1; p.wp = h->wp; p.bp = h->bp; p.wv1 = h->wv1;
   p.bv1 = h->bv1; p.wv2 = h->wv2; p.bv2 = h->bv2; p.logp = logp; p.value = value;
   p.n_boards = n_boards; p.H = h->board_size; p.W = W; p.HW = HW; p.A = A; p.AS = h->action_stride;
-  p.S = rz_row_stride(h->board_size, W, h->row_stride);
-  RZ_REQUIRE(!act_is_tile_bf16 || p.S != 0, "rz_net_heads: row_stride %d does not hold a %dx%d board", h->row_stride,
-             h->board_size, W);
-  p.P = p.S * p.S;
   const size_t smem = heads_smem(HW, p.AS);
-  const int grid = (n_boards + HEAD_NB - 1) / HEAD_NB;
-  if (act_is_tile_bf16 == 2) return heads_launch<SRC_FEAT>(p, smem, grid, (cudaStream_t)stream);
-  if (act_is_tile_bf16 == 1) return heads_launch<SRC_TILE>(p, smem, grid, (cudaStream_t)stream);
-  return heads_launch<SRC_F32>(p, smem, grid, (cudaStream_t)stream);
+  cudaError_t e = cudaFuncSetAttribute(rz_heads_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) { rz_set_error("rz_net_heads: smem attribute: %s", cudaGetErrorString(e)); return -2; }
+  rz_launch_pdl(rz_heads_kernel, (n_boards + HEAD_NB - 1) / HEAD_NB, HEAD_THREADS, smem, (cudaStream_t)stream, p);
+  RZ_LAUNCH_CHECK("rz_net_heads");
+  return 0;
 }
 
 extern "C" int rz_net_head_features(const rz_heads_desc* h, const void* act, float* feat, int n_boards,

@@ -16,7 +16,6 @@
 // Accumulators live in TMEM: columns [0, AS) policy logits, [AS, AS+64) value hidden units; the epilogue
 // (one thread per board row) adds the biases, does log_softmax / ReLU-FC2-tanh straight from TMEM.
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include "rz_common.cuh"
 #include "rz_tc.cuh"
@@ -504,13 +503,6 @@ rz_heads_tc4_kernel(const __grid_constant__ CUtensorMap tmap_whi, const __grid_c
   if (warp == 0) { rz::tc_fence_after(); rz::tmem_dealloc(tmem_base, (uint32_t)p.tmem_cols); }
 }
 
-// RZ_HEADS_CLUSTER=0: the single-CTA kernel for every action stride (A/B runs, bisecting)
-static bool getenv_flag_off() {
-  static int off = -1;
-  if (off < 0) { const char* e = getenv("RZ_HEADS_CLUSTER"); off = (e && e[0] == '0') ? 1 : 0; }
-  return off == 1;
-}
-
 }  // namespace
 
 extern "C" int rz_net_heads_tc(const rz_heads_desc* h, const float* feat, float* logp, float* value,
@@ -551,7 +543,7 @@ extern "C" int rz_net_heads_tc(const rz_heads_desc* h, const float* feat, float*
   if (rz::make_tmap_2d(&t_wlo, wlo, (uint64_t)AS, (uint64_t)KP, (uint32_t)p.w_box)) return -1;
   if (rz::make_tmap_2d(&t_vhi, whi + (size_t)AS * KP, 64, (uint64_t)KP, 64)) return -1;
   if (rz::make_tmap_2d(&t_vlo, wlo + (size_t)AS * KP, 64, (uint64_t)KP, 64)) return -1;
-  if (AS <= 256 && p.live_per_plane > 0 && !getenv_flag_off()) {
+  if (AS <= 256 && p.live_per_plane > 0) {
     // the cluster-of-four split-K kernel
     const size_t smem4 = 2 * (2 * HT_A_BYTES + slot) + HT_CTRL_BYTES;
     static size_t attr_smem4 = 0;

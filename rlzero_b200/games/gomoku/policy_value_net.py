@@ -157,7 +157,7 @@ class NativeForward(object):
     prior_is_log = True       # the network emits log-probabilities (policy_value_net.py:44)
 
     def __init__(self, module, mode=None, max_batch=1, device='cuda', n_ctas=0, fused_head=True, game_type=None,
-                 row_stride=None, heads_tc=True):
+                 row_stride=None):
         if not torch.cuda.is_available():
             raise L.NativeLibraryError('NativeForward needs a CUDA device (no CPU fallback)')
         self.lib = L.load()
@@ -212,16 +212,11 @@ class NativeForward(object):
         # the heads' 1x1 convolutions inside the last trunk layer's epilogue (rz_net_tc2.cu, kHead)
         self.fused_head = bool(fused_head)
         self.weights_version = 0
-        # the heads' fully connected layers on the tensor cores (rz_net_heads_tc.cu; bf16 hi/lo split, fp32-level
-        # accuracy); False keeps the CUDA-core heads kernel
-        self.heads_tc = (bool(heads_tc) and mode == 'tc') or mode == 'tc32'
-        import os
         # boards up to which the one-launch trunk of rz_net_trunk_small.cu is used (one CTA pair per board, 74 pairs at a
-        # time on 148 SMs; measured crossover with the per-layer kernels near 200 boards, profiles/r2_run43_crossover.log);
-        # RZ_SMALL_BATCH_MAX=0 turns it off
-        self.small_batch_max = int(os.environ.get('RZ_SMALL_BATCH_MAX', '148'))
-        # flags of the 128 -> 128 rz_net_conv3x3_tc2 launches, read by MuZeroNative and bench.py too: 512 = static
-        # weights (include/rlzero_b200.h); bit 1 (2) is accepted and ignored
+        # time on 148 SMs; measured crossover with the per-layer kernels near 200 boards, profiles/r2_run43_crossover.log)
+        self.small_batch_max = 148
+        # flags of the 128 -> 128 rz_net_conv3x3_tc2 launches, read by bench.py too: 512 = static weights
+        # (include/rlzero_b200.h); bit 1 (2) is accepted and ignored
         self.conv_flags = 514
         self.max_batch = 0
         self.refresh_weights()
@@ -330,7 +325,7 @@ class NativeForward(object):
             bv1=m.val_fc1.bias.detach().float().contiguous().to(dev),
             wv2=m.val_fc2.weight.detach().reshape(64).float().contiguous().to(dev),
             bv2=m.val_fc2.bias.detach().float().contiguous().to(dev))
-        if self.heads_tc:
+        if self.mode != 'f32':
             # both FCs as one K-major matrix over the padded feature row k' = f*P + y*S + x (rz_heads_desc.wtc_hi)
             S, Pp, A = self.S, self.P, self.A
             KP = (6 * Pp + 63) // 64 * 64
@@ -437,95 +432,44 @@ class NativeForward(object):
                              "or Go's 17 planes")
         return self.stem
 
+    def _one_launch(self, n):
+        """Whether ``n`` boards run the trunk behind the stem in one launch (rz_net_trunk_small.cu) instead of one
+        launch per layer: few boards (a sequential search evaluates ONE), a layout the one-launch kernel takes, and in
+        mode 'tc' the fused heads epilogue, which that kernel always applies."""
+        return (self.trunk_small is not None and n <= self.small_batch_max
+                and (self.mode == 'tc32' or self.fused_head))
+
+    def _conv(self, layer, inp, res, out, n):
+        """One 128 -> 128 trunk layer on the tensor cores.  The layer layout picks the kernel: rz_net_tc2.cu for
+        stride 16, rz_net_tc3.cu otherwise (bit 1 of its `relu`, like flag 512 of tc2: static weights)."""
+        s = L.stream_ptr()
+        if self.S == 16:
+            L.check(self.lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res),
+                                                L.ptr(out), n, self.H, self.W, layer['cin'], int(layer['relu']), 2,
+                                                self.conv_flags, self.n_ctas, s), 'rz_net_conv3x3_tc2')
+        else:
+            L.check(self.lib.rz_net_conv3x3_tc3(L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res),
+                                                L.ptr(out), n, self.H, self.W, self.S, int(layer['relu']) | 2,
+                                                self.n_ctas, s), 'rz_net_conv3x3_tc3')
+
+    def _conv_head(self, layer, inp, res, n):
+        """``_conv`` of the last trunk layer with the heads' 1x1 convolutions in its epilogue: writes ``self.feat``."""
+        s = L.stream_ptr()
+        w1p = self.w1x1_host.ctypes.data_as(C.c_void_p)
+        b1p = self.b1x1_host.ctypes.data_as(C.c_void_p)
+        if self.S == 16:
+            L.check(self.lib.rz_net_conv3x3_tc2_head_ex(
+                L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res), n, self.H, self.W, layer['cin'],
+                int(layer['relu']), 512, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc2_head_ex')
+        else:
+            L.check(self.lib.rz_net_conv3x3_tc3_head(
+                L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res), n, self.H, self.W, self.S,
+                int(layer['relu']) | 2, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc3_head')
+
     def _trunk_and_heads(self, n, logp, value):
         s = L.stream_ptr()
         lib = self.lib
-        if self.mode == 'tc32' and self.trunk_small is not None and n <= self.small_batch_max:
-            # few boards: conv2 + conv3 + the 1x1 heads in one launch (rz_net_trunk_small_ex), then the FC heads
-            ts = self.trunk_small
-            L.check(lib.rz_net_trunk_small_ex(
-                L.ptr(self.bufs[0]), L.ptr(ts['w']), L.ptr(ts['b']), ts['n'], ts['relu_mask'], ts['res_mask'],
-                ts['n64_mask'], ts['split_in_mask'], ts['head_f32'], n, self.H, self.W,
-                self.w1x1_host.ctypes.data_as(C.c_void_p), self.b1x1_host.ctypes.data_as(C.c_void_p), L.ptr(self.feat), s),
-                'rz_net_trunk_small_ex')
-            L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
-                    'rz_net_heads_tc')
-            return
-        if self.mode == 'tc32':
-            # conv2 (one K = 128 pass, split output) and conv3 (three products per tap, fp32 features), then the heads
-            l2, l3 = self.layers[1], self.layers[2]
-            L.check(lib.rz_net_conv3x3_tc2(L.ptr(self.bufs[0]), L.ptr(l2['w']), L.ptr(l2['b']), None, L.ptr(self.bufs[1]),
-                                           n, self.H, self.W, 128, int(l2['relu']), 2, 2 | 8 | 256 | 512, self.n_ctas, s),
-                    'rz_net_conv3x3_tc2')
-            L.check(lib.rz_net_conv3x3_tc2_head_ex(
-                L.ptr(self.bufs[1]), L.ptr(l3['w']), L.ptr(l3['b']), None, n, self.H, self.W, 128, int(l3['relu']),
-                16 | 32 | 512, self.w1x1_host.ctypes.data_as(C.c_void_p), self.b1x1_host.ctypes.data_as(C.c_void_p),
-                L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc2_head_ex')
-            L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
-                    'rz_net_heads_tc')
-            return
-        if self.mode == 'tc' and self.trunk_small is not None and n <= self.small_batch_max and self.fused_head:
-            # few boards (a sequential search evaluates ONE): the whole trunk in one launch, one CTA pair per board
-            ts = self.trunk_small
-            L.check(lib.rz_net_trunk_small(
-                L.ptr(self.bufs[0]), L.ptr(ts['w']), L.ptr(ts['b']), ts['n'], ts['relu_mask'], ts['res_mask'], n,
-                self.H, self.W, self.w1x1_host.ctypes.data_as(C.c_void_p), self.b1x1_host.ctypes.data_as(C.c_void_p),
-                L.ptr(self.feat), s), 'rz_net_trunk_small')
-            if self.heads_tc:
-                L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
-                        'rz_net_heads_tc')
-            else:
-                L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(self.feat), 2, L.ptr(logp), L.ptr(value), n, s),
-                        'rz_net_heads')
-            return
-        if self.mode == 'tc':
-            # ping-pong behind the stem, which wrote bufs[0]: the residual of a block is the buffer its second conv
-            # overwrites.  The layer layout picks the kernel: rz_net_tc2.cu for stride 16, rz_net_tc3.cu otherwise.
-            outs = self.bufs
-            cur = 0   # index in outs holding the latest activation
-            for i, l in enumerate(self.layers[1:], 1):
-                dst = 1 - cur
-                res = None
-                if l['skip'] is not None:
-                    # skip always refers to the activation two layers back = the other buffer
-                    res = outs[dst]
-                inp = outs[cur]
-                w1p = self.w1x1_host.ctypes.data_as(C.c_void_p)
-                b1p = self.b1x1_host.ctypes.data_as(C.c_void_p)
-                if self.fused_head and i == len(self.layers) - 1:
-                    if self.S != 16:
-                        L.check(lib.rz_net_conv3x3_tc3_head(
-                            L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res), n, self.H, self.W, self.S,
-                            int(l['relu']) | 2, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc3_head')
-                    else:
-                        L.check(lib.rz_net_conv3x3_tc2_head_ex(
-                            L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res), n, self.H, self.W, l['cin'],
-                            int(l['relu']), 512, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc2_head_ex')
-                    if self.heads_tc:
-                        L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value),
-                                                    n, s), 'rz_net_heads_tc')
-                    else:
-                        L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(self.feat), 2, L.ptr(logp),
-                                                 L.ptr(value), n, s), 'rz_net_heads')
-                    return
-                if self.S != 16:
-                    L.check(lib.rz_net_conv3x3_tc3(L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res),
-                                                   L.ptr(outs[dst]), n, self.H, self.W, self.S, int(l['relu']) | 2,
-                                                   self.n_ctas, s), 'rz_net_conv3x3_tc3')
-                else:
-                    L.check(lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(l['w']), L.ptr(l['b']), L.ptr(res),
-                                                   L.ptr(outs[dst]), n, self.H, self.W, l['cin'],
-                                                   int(l['relu']), 2, self.conv_flags, self.n_ctas, s), 'rz_net_conv3x3_tc2')
-                cur = dst
-            if self.heads_tc:
-                L.check(lib.rz_net_head_features(C.byref(self.hdesc), L.ptr(outs[cur]), L.ptr(self.feat), n, s),
-                        'rz_net_head_features')
-                L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
-                        'rz_net_heads_tc')
-            else:
-                L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(outs[cur]), 1, L.ptr(logp), L.ptr(value), n, s),
-                        'rz_net_heads')
-        else:
+        if self.mode == 'f32':
             outs = self.bufs
             hist = []   # buffer index holding the output of layer i
             inp = self.act0
@@ -540,21 +484,59 @@ class NativeForward(object):
                                                int(l['relu']), s), 'rz_net_conv3x3_f32')
                 hist.append(dst)
                 inp = outs[dst]
-            L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(inp), 0, L.ptr(logp), L.ptr(value), n, s),
-                    'rz_net_heads')
+            L.check(lib.rz_net_heads(C.byref(self.hdesc), L.ptr(inp), L.ptr(logp), L.ptr(value), n, s), 'rz_net_heads')
+            return
+        # the tensor-core modes: trunk behind the stem (which wrote bufs[0]) -> head features in self.feat -> FC heads
+        w1p = self.w1x1_host.ctypes.data_as(C.c_void_p)
+        b1p = self.b1x1_host.ctypes.data_as(C.c_void_p)
+        if self._one_launch(n):
+            # the whole trunk in one launch, one CTA pair per board (tc32: conv2 + conv3 + the 1x1 heads)
+            ts = self.trunk_small
+            if self.mode == 'tc32':
+                L.check(lib.rz_net_trunk_small_ex(
+                    L.ptr(self.bufs[0]), L.ptr(ts['w']), L.ptr(ts['b']), ts['n'], ts['relu_mask'], ts['res_mask'],
+                    ts['n64_mask'], ts['split_in_mask'], ts['head_f32'], n, self.H, self.W, w1p, b1p,
+                    L.ptr(self.feat), s), 'rz_net_trunk_small_ex')
+            else:
+                L.check(lib.rz_net_trunk_small(
+                    L.ptr(self.bufs[0]), L.ptr(ts['w']), L.ptr(ts['b']), ts['n'], ts['relu_mask'], ts['res_mask'], n,
+                    self.H, self.W, w1p, b1p, L.ptr(self.feat), s), 'rz_net_trunk_small')
+        elif self.mode == 'tc32':
+            # conv2 (one K = 128 pass, split output) and conv3 (three products per tap, fp32 features)
+            l2, l3 = self.layers[1], self.layers[2]
+            L.check(lib.rz_net_conv3x3_tc2(L.ptr(self.bufs[0]), L.ptr(l2['w']), L.ptr(l2['b']), None, L.ptr(self.bufs[1]),
+                                           n, self.H, self.W, 128, int(l2['relu']), 2, 2 | 8 | 256 | 512, self.n_ctas, s),
+                    'rz_net_conv3x3_tc2')
+            L.check(lib.rz_net_conv3x3_tc2_head_ex(
+                L.ptr(self.bufs[1]), L.ptr(l3['w']), L.ptr(l3['b']), None, n, self.H, self.W, 128, int(l3['relu']),
+                16 | 32 | 512, w1p, b1p, L.ptr(self.feat), self.n_ctas, s), 'rz_net_conv3x3_tc2_head_ex')
+        else:
+            # ping-pong: the residual of a block is the buffer its second conv overwrites
+            outs = self.bufs
+            cur = 0   # index in outs holding the latest activation
+            for i, l in enumerate(self.layers[1:], 1):
+                # skip always refers to the activation two layers back = the other buffer
+                res = outs[1 - cur] if l['skip'] is not None else None
+                if self.fused_head and i == len(self.layers) - 1:
+                    self._conv_head(l, outs[cur], res, n)
+                    break
+                self._conv(l, outs[cur], res, outs[1 - cur], n)
+                cur = 1 - cur
+            else:
+                L.check(lib.rz_net_head_features(C.byref(self.hdesc), L.ptr(outs[cur]), L.ptr(self.feat), n, s),
+                        'rz_net_head_features')
+        L.check(lib.rz_net_heads_tc(C.byref(self.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value), n, s),
+                'rz_net_heads_tc')
 
     def kernels_per_forward(self, n=None):
         """Kernel launches of one forward_boards call of ``n`` boards (for bench.py's gpu_launches)."""
-        if self.mode == 'tc32':
-            if n is not None and self.trunk_small is not None and n <= self.small_batch_max:
-                return 3                                    # stem, conv2 + conv3 + 1x1 heads in one launch, FC heads
-            return 4                                        # stem, conv2, conv3 + 1x1 heads, FC heads
-        if (n is not None and self.mode == 'tc' and self.trunk_small is not None and n <= self.small_batch_max
-                and self.fused_head):
+        if n is not None and self._one_launch(n):
             return 3                                        # stem, one-launch trunk + 1x1 heads, FC heads
-        n_conv = len(self.layers)
-        heads = 2 if (self.heads_tc and not self.fused_head) else 1   # [1x1 features +] FC heads
-        return (n_conv if self.mode == 'tc' else 1 + n_conv) + heads  # [stem + convs | encode + convs] + heads
+        if self.mode == 'tc32':
+            return 4                                        # stem, conv2, conv3 + 1x1 heads, FC heads
+        if self.mode == 'f32':
+            return 1 + len(self.layers) + 1                 # encode, convs, heads
+        return len(self.layers) + (1 if self.fused_head else 2)   # stem + convs, [1x1 features +] FC heads
 
     def forward_boards(self, rows, meta, n, logp=None, value=None, hist=None):
         """Positions in the device board layout -> (logp [n][AS], value [n]) float32 tensors.

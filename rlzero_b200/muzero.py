@@ -11,7 +11,7 @@ board-game setting: reward 0, discount 1, values negated between plies.  PARITY 
                      last channel is replaced by the one-hot plane of the action;  f = the reference's
                      policy / value heads (rlzero/games/gomoku/policy_value_net.py:19-25,41-51).
 * ``MuZeroNative``   the same three functions on the tensor cores through the C ABI
-                     (rz_net_stem_tc, rz_net_conv3x3_tc2/3, rz_net_heads, rz_mz_gather).
+                     (rz_net_stem_tc, rz_net_conv3x3_tc2/3, rz_net_heads_tc, rz_mz_gather).
 * ``MuZeroSearch``   G latent-space trees in HBM + the per-move loop
                      h -> f -> rz_mz_root -> 50 x (rz_mz_select -> rz_mz_gather -> g -> f -> rz_mz_expand_backup),
                      captured as one CUDA graph.  Hidden states live node-major (pool[node][tree]) so the
@@ -141,13 +141,12 @@ class MuZeroNative(object):
         self.net = net
         self.G = int(n_trees)
         self.device = torch.device(device)
-        self.n_ctas = int(n_ctas)
         self.game_type = int(game_type)
         # weight packing (BatchNorm folded, bf16 [tap][cout][cin]) through the AlphaZero packer
         self.h = NativeForward(_TrunkView(net, net.repr_stem, net.repr_blocks), mode='tc', max_batch=1,
-                               device=device, game_type=game_type, fused_head=False)
+                               device=device, n_ctas=n_ctas, game_type=game_type)
         self.g = NativeForward(_TrunkView(net, net.dyn_in, net.dyn_blocks), mode='tc', max_batch=1,
-                               device=device, game_type=game_type, fused_head=False)
+                               device=device, n_ctas=n_ctas, game_type=game_type)
         if self.h.stem is None:
             raise ValueError('the representation stem must take the 4 observation planes (fused encoder + stem)')
         self.H, self.W, self.S, self.P = self.h.H, self.h.W, self.h.S, self.h.P
@@ -171,26 +170,16 @@ class MuZeroNative(object):
     def hbm_bytes(self):
         return sum(t.numel() * t.element_size() for t in [self.pool] + self.bufs)
 
-    def _conv(self, layer, inp, res, out):
-        s = L.stream_ptr()
-        if self.S == 16:
-            L.check(self.lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res),
-                                                L.ptr(out), self.G, self.H, self.W, 128, int(layer['relu']), 2, self.h.conv_flags,
-                                                self.n_ctas, s), 'rz_net_conv3x3_tc2')
-        else:
-            L.check(self.lib.rz_net_conv3x3_tc3(L.ptr(inp), L.ptr(layer['w']), L.ptr(layer['b']), L.ptr(res),
-                                                L.ptr(out), self.G, self.H, self.W, self.S, int(layer['relu']),
-                                                self.n_ctas, s), 'rz_net_conv3x3_tc3')
-
-    def _blocks(self, layers, x, other, final_out):
-        """Residual blocks layers[1:] on the activation in ``x`` (``other`` = scratch); the last conv
+    def _blocks(self, nf, x, other, final_out):
+        """Residual blocks nf.layers[1:] on the activation in ``x`` (``other`` = scratch); the last conv
         writes ``final_out``.  Returns nothing; with no blocks the caller wrote final_out already."""
+        layers = nf.layers
         n_blocks = (len(layers) - 1) // 2
         for b in range(n_blocks):
             c1, c2 = layers[1 + 2 * b], layers[2 + 2 * b]
-            self._conv(c1, x, None, other)
+            nf._conv(c1, x, None, other, self.G)
             last = b == n_blocks - 1
-            self._conv(c2, other, x, final_out if last else x)      # residual may alias the output
+            nf._conv(c2, other, x, final_out if last else x, self.G)      # residual may alias the output
 
     def representation(self, rows, meta, slot=0):
         """h(observation of the device positions) -> pool[slot]."""
@@ -202,7 +191,7 @@ class MuZeroNative(object):
         L.check(self.lib.rz_net_stem_tc(C.byref(g), L.ptr(rows), L.ptr(meta), L.ptr(st['w']), L.ptr(st['b']),
                                         L.ptr(first_out), self.G, int(st['relu']), 0, L.stream_ptr()),
                 'rz_net_stem_tc')
-        self._blocks(nf.layers, self.bufs[0], self.bufs[1], self.pool[slot])
+        self._blocks(nf, self.bufs[0], self.bufs[1], self.pool[slot])
 
     def dynamics(self, parent, action, slot):
         """g(pool[parent[g]][g], action[g]) -> pool[slot] for every tree g."""
@@ -211,21 +200,17 @@ class MuZeroNative(object):
         nf = self.g
         n_blocks = (len(nf.layers) - 1) // 2
         first_out = self.pool[slot] if n_blocks == 0 else self.bufs[1]
-        self._conv(nf.layers[0], self.bufs[0], None, first_out)
-        self._blocks(nf.layers, self.bufs[1], self.bufs[0], self.pool[slot])
+        nf._conv(nf.layers[0], self.bufs[0], None, first_out, self.G)
+        self._blocks(nf, self.bufs[1], self.bufs[0], self.pool[slot])
 
     def prediction(self, slot, logp=None, value=None):
         """f(pool[slot]) -> (log-probabilities [G][AS], value [G])."""
         logp = self.logp if logp is None else logp
         value = self.value if value is None else value
-        if self.h.heads_tc:
-            L.check(self.lib.rz_net_head_features(C.byref(self.h.hdesc), L.ptr(self.pool[slot]), L.ptr(self.feat),
-                                                  self.G, L.stream_ptr()), 'rz_net_head_features')
-            L.check(self.lib.rz_net_heads_tc(C.byref(self.h.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value),
-                                             self.G, L.stream_ptr()), 'rz_net_heads_tc')
-        else:
-            L.check(self.lib.rz_net_heads(C.byref(self.h.hdesc), L.ptr(self.pool[slot]), 1, L.ptr(logp),
-                                          L.ptr(value), self.G, L.stream_ptr()), 'rz_net_heads')
+        L.check(self.lib.rz_net_head_features(C.byref(self.h.hdesc), L.ptr(self.pool[slot]), L.ptr(self.feat),
+                                              self.G, L.stream_ptr()), 'rz_net_head_features')
+        L.check(self.lib.rz_net_heads_tc(C.byref(self.h.hdesc), L.ptr(self.feat), L.ptr(logp), L.ptr(value),
+                                         self.G, L.stream_ptr()), 'rz_net_heads_tc')
         return logp, value
 
     def unroll(self, rows, meta, actions):
@@ -252,7 +237,7 @@ class MuZeroNative(object):
         return logp, value
 
     def kernels_per_simulation(self):
-        return 1 + len(self.g.layers) + (2 if self.h.heads_tc else 1)      # gather + convolutions + heads
+        return 1 + len(self.g.layers) + 2      # gather + convolutions + head features + FC heads
 
     def hidden_state(self, slot):
         """pool[slot] as float32 [G, 128, H, W] (tests)."""
@@ -348,7 +333,7 @@ class MuZeroSearch(object):
 
     def kernels_per_move(self):
         nat = self.native
-        return (len(nat.h.layers) + (3 if nat.h.heads_tc else 2)) + self.cfg.num_simulations * (2 + nat.kernels_per_simulation())
+        return (len(nat.h.layers) + 3) + self.cfg.num_simulations * (2 + nat.kernels_per_simulation())
 
     # ------------------------------------------------------------------- search
     def run(self, rows, meta, legal=None, add_noise=True, use_graph=True, move_ids=None):

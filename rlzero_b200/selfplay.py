@@ -4,8 +4,9 @@ This is ``GameControl.start_self_play`` + ``AlphaZeroPlayer.get_action`` + ``Alp
 (rlzero/games/gomoku/game.py:96-134, rlzero/mcts/alphazero_mcts.py:73-165) for thousands of
 games at once, entirely on the device:
 
-    per wave  : rz_tree_select -> rz_net_stem_tc (encoder + first conv) -> 20 x rz_net_conv3x3_tc2 -> rz_net_heads
-                -> rz_tree_expand_backup                          (one CUDA graph, replayed)
+    per wave  : rz_tree_select -> rz_net_stem_tc (encoder + first conv) -> 20 x rz_net_conv3x3_tc2 (the last
+                with the heads' 1x1 convolutions) -> rz_net_heads_tc -> rz_tree_expand_backup
+                                                                  (one CUDA graph, replayed)
     per move  : rz_tree_root_policy (pi, sampled move) -> rz_tree_advance (record ply, play the
                 move, re-root with the kept subtree, finish episode -> z -> ring, restart slot)
 

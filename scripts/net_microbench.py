@@ -58,13 +58,9 @@ def main():
         print(json.dumps({'kernel': name, 'B': B, 'ms': ms, 'TFLOPs_algorithmic': flops_alg / ms / 1e9,
                           'TFLOPs_issued': flops_issued / ms / 1e9}))
 
-    def heads():
-        L.check(lib.rz_net_heads(nf.hdesc, L.ptr(x), 1, L.ptr(nf.logp), L.ptr(nf.value), B, L.stream_ptr()))
-    print(json.dumps({'kernel': 'heads<tile>', 'ms': timeit(heads)}))
-
-    def heads_feat():
-        L.check(lib.rz_net_heads(nf.hdesc, L.ptr(nf.feat), 2, L.ptr(nf.logp), L.ptr(nf.value), B, L.stream_ptr()))
-    print(json.dumps({'kernel': 'heads<feat>', 'ms': timeit(heads_feat)}))
+    def heads_tc():
+        L.check(lib.rz_net_heads_tc(nf.hdesc, L.ptr(nf.feat), L.ptr(nf.logp), L.ptr(nf.value), B, L.stream_ptr()))
+    print(json.dumps({'kernel': 'heads_tc', 'ms': timeit(heads_tc)}))
     import ctypes as C
 
     def conv_head():

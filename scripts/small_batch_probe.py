@@ -34,5 +34,5 @@ for G in [int(g) for g in os.environ.get('RZ_GS', '1,8,64,512').split(',')]:
     e1.record()
     torch.cuda.synchronize()
     us = e0.elapsed_time(e1) * 1000 / 400
-    print(json.dumps({'games': G, 'us_per_wave': us, 'sims_per_s': G / us * 1e6, 'pdl': os.environ.get('RZ_PDL', '1'),
-                      'small_batch_max': os.environ.get('RZ_SMALL_BATCH_MAX', 'default')}), flush=True)
+    print(json.dumps({'games': G, 'us_per_wave': us, 'sims_per_s': G / us * 1e6, 'pdl': os.environ.get('RZ_PDL', '1')}),
+          flush=True)

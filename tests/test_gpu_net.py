@@ -614,10 +614,10 @@ def test_row_stride_8_stem_bitboards_vs_planes_and_torch(size, n):
 
 @pytest.mark.parametrize('h,w,a,planes,n', [(15, 15, None, 4, 300), (15, 15, None, 4, 1), (19, 19, 362, 17, 131),
                                             (6, 7, 7, 4, 257), (3, 3, None, 4, 5), (9, 9, None, 4, 128)])
-def test_heads_on_the_tensor_cores_match_the_fp32_heads(h, w, a, planes, n):
+def test_heads_on_the_tensor_cores_match_float64_heads(h, w, a, planes, n):
     """rz_net_heads_tc (both FCs as one tcgen05 GEMM over the padded feature row, bf16 hi/lo split) against the
-    CUDA-core fp32 heads kernel on the same features: float32-level agreement (the split drops only the lo*lo
-    term), for every padded layout (S = 8 / 16 / 20), AS = 32 ... 384 (two N pieces for Go), partial last tile;
+    heads' FC layers in float64 on the same features: float32-level agreement (the split drops only the lo*lo term),
+    for every padded layout (S = 8 / 16 / 20), AS = 32 ... 384 (two N pieces for Go), partial last tile;
     fused-head and separate-feature routes are bit-identical."""
     from rlzero_b200.games.gomoku.policy_value_net import NativeForward, ResNetPolicyValueNet
     torch.manual_seed(h * 31 + n)
@@ -630,20 +630,24 @@ def test_heads_on_the_tensor_cores_match_the_fp32_heads(h, w, a, planes, n):
         net.val_fc1.weight.mul_(4.0)
         net.val_fc2.weight.mul_(4.0)
     x = np.random.RandomState(n).randint(0, 2, size=(n, planes, h, w)).astype(np.float32)
-    tc = NativeForward(net, max_batch=n, heads_tc=True)
-    cc = NativeForward(net, max_batch=n, heads_tc=False)
-    assert tc.heads_tc and not cc.heads_tc
+    tc = NativeForward(net, max_batch=n)
     lt, vt = (t.clone() for t in tc.forward_planes(x))
-    lc, vc = (t.clone() for t in cc.forward_planes(x))
     A = tc.A
     assert torch.isfinite(lt).all() and torch.isfinite(vt).all()
-    # a few float32 ulps of the largest |log p| (the scaled heads reach ~30): two fp32 summation orders differ by that
-    assert (lt[:, :A] - lc[:, :A]).abs().max().item() < 1e-4, (lt[:, :A] - lc[:, :A]).abs().max().item()
-    assert (lt[:, :A].exp() - lc[:, :A].exp()).abs().max().item() < 1e-5
-    assert (vt - vc).abs().max().item() < 1e-5
+    # the features the kernel consumed, at the board squares of the padded layout, in the reference's flatten order
+    fe = tc.feat[:n].double().view(n, 6, tc.S, tc.S)[:, :, :h, :w]
+    with torch.no_grad():
+        d = {k: t.double() for k, t in net.state_dict().items()}
+        lc = torch.log_softmax(fe[:, :4].reshape(n, -1) @ d['act_fc1.weight'].t() + d['act_fc1.bias'], dim=1)
+        hid = torch.relu(fe[:, 4:].reshape(n, -1) @ d['val_fc1.weight'].t() + d['val_fc1.bias'])
+        vc = torch.tanh(hid @ d['val_fc2.weight'].t() + d['val_fc2.bias']).reshape(-1)
+    # a few float32 ulps of the largest |log p| (the scaled heads reach ~30)
+    assert (lt[:, :A] - lc).abs().max().item() < 1e-4, (lt[:, :A] - lc).abs().max().item()
+    assert (lt[:, :A].double().exp() - lc.exp()).abs().max().item() < 1e-5
+    assert (vt.double() - vc).abs().max().item() < 1e-5
     assert torch.allclose(lt[:, :A].exp().sum(1), torch.ones(n, device='cuda'), atol=1e-4)
     assert tc.logp[:n, A:].abs().max().item() == 0.0 if tc.AS > A else True
-    tb = NativeForward(net, max_batch=n, heads_tc=True, fused_head=False)
+    tb = NativeForward(net, max_batch=n, fused_head=False)
     lb, vb = tb.forward_planes(x)
     assert torch.equal(lb, lt) and torch.equal(vb, vt)
     # against PyTorch fp32 end to end
