@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define RZ_ABI_VERSION 12
+#define RZ_ABI_VERSION 13
 #define RZ_MAX_BOARD 19          /* rows live one per lane; A <= 362 (19x19 Go incl. the pass) */
 #define RZ_META_STRIDE 12
 #define RZ_GO_HIST 14            /* history planes a Go position carries besides the current board */
@@ -420,15 +420,23 @@ int rz_learn_adam(float* param, const float* grad, float* exp_avg, float* exp_av
                   float beta2, float eps, float weight_decay, int step, void* stream);
 
 /* ---- the same step for the 128-channel ResNet trunk on the tensor cores (rz_learn_tc.cu) -------------------------
-   bf16 activations / gradients in the padded 16-stride layout [n*256][128] of the inference path (boards up to 15x15),
-   fp32 statistics and parameter gradients.  Forward convolution and data gradient are rz_net_conv3x3_tc2 (the latter
-   with w_bwd below); the heads run through the float32 kernels above after rz_learn_tile_to_nhwc. */
+   bf16 activations / gradients in the padded position layout of the inference path, fp32 statistics and parameter
+   gradients.  Row stride S = 16 up to 15x15 ([n*256][128]; forward convolution and data gradient through
+   rz_net_conv3x3_tc2) or 20 up to 19x19 ([round_up(n*400, 256)][128]; rz_net_conv3x3_tc3); the data gradient runs
+   with w_bwd below; the heads run through the float32 kernels above after rz_learn_tile_to_nhwc[_ex].  The _ex entry
+   points take the row stride (16 or 20, anything else is an error naming row_stride); each plain entry point is the
+   S = 16 call of its _ex form.  Tensors of stride S have round_up(n*S*S, 256) rows; a row is off the board when its
+   x >= W, its y >= H, or the row is >= n*S*S, and off-board rows are written as zero. */
 /* dw [128][128][3][3] fp32 = sum over positions of dy[p][co] * x[p + d(tap)][ci]: tcgen05 GEMM with MN-major operands
    (the reduction index is the tile row), accumulators in TMEM for the whole launch, CTA triples (one per filter row)
    sharing position tiles through L2.  x, dy: bf16 [n*256][128] with zero pad squares.  scratch: 49 * 9 * 128 * 128
    floats (per-split partials, folded in a fixed order).  n_ctas <= 0 picks 147. */
 int rz_learn_conv_wgrad_tc(const void* x, const void* dy, float* dw_oihw, float* scratch, long long scratch_floats,
                            int n_boards, int n_ctas, void* stream);
+/* the same at row stride S (16 or 20): x tiles carry an (S + 1)-row halo, ceil(n*S*S / 128) position tiles, which at
+   S = 20 straddle boards (harmless: pad squares are zero); x, dy bf16 [round_up(n*S*S, 256)][128] */
+int rz_learn_conv_wgrad_tc_ex(const void* x, const void* dy, float* dw_oihw, float* scratch, long long scratch_floats,
+                              int n_boards, int row_stride, int n_ctas, void* stream);
 /* nn.Conv2d weight fp32 [128][128][3][3] -> bf16 w_fwd [tap][cout][cin] (rz_net_conv3x3_tc2's layout) and w_bwd
    [8-tap][cin][cout]: rz_net_conv3x3_tc2(dy, w_bwd, zero bias, residual = skip gradient, ...) is the data gradient */
 int rz_learn_pack_conv_tc(const float* w_oihw, void* w_fwd, void* w_bwd, void* stream);
@@ -441,6 +449,9 @@ int rz_net_pack_conv_bn_tc(const float* w_oihw, const float* conv_bias, const fl
                            void* stream);
 /* stem weight fp32 [128][4][3][3] -> bf16 [128][64] (k = tap*4 + plane, rz_net_stem_tc's layout) */
 int rz_learn_pack_stem_tc(const float* w_oihw, void* w_stem, void* stream);
+/* in_planes 4: the same; in_planes 17 (Go): fp32 [128][17][3][3] -> bf16 [128][192] (k = tap*17 + plane, zero from 153:
+   rz_net_stem_go_tc's layout) */
+int rz_learn_pack_stem_tc_ex(const float* w_oihw, int in_planes, void* w_stem, void* stream);
 /* nn.BatchNorm2d in training mode + skip + ReLU: batch statistics of y over the board squares (biased variance),
    running_mean / running_var updated (momentum, unbiased variance; may be NULL), out = relu((y - mean) * invstd *
    gamma + beta (+ skip)), zero off the board.  stats [4][128] receives mean, invstd, gamma * invstd, beta - mean *
@@ -452,9 +463,19 @@ int rz_learn_bn_forward(const void* y, const void* skip, void* out, const float*
    xhat * dgamma / N) (bf16, zero off the board); dz_out (may be NULL) receives dz, the gradient into the skip */
 int rz_learn_bn_backward(const void* dout, const void* act, const void* y, const float* stats, float* dgamma, float* dbeta,
                          void* dy, void* dz_out, float* scratch, int n_boards, int board_rows, int board_cols, void* stream);
+/* both at row stride S (boards up to S - 1 squares a side; the statistics still count n * H * W squares) */
+int rz_learn_bn_forward_ex(const void* y, const void* skip, void* out, const float* gamma, const float* beta,
+                           float* running_mean, float* running_var, float eps, float momentum, float* stats, float* scratch,
+                           int n_boards, int board_rows, int board_cols, int row_stride, void* stream);
+int rz_learn_bn_backward_ex(const void* dout, const void* act, const void* y, const float* stats, float* dgamma,
+                            float* dbeta, void* dy, void* dz_out, float* scratch, int n_boards, int board_rows,
+                            int board_cols, int row_stride, void* stream);
 /* float32 observation planes [n][4][H][W] -> bf16 tile [n*256][128] (channels 0..3, rest zero): the stem's input as the
    x operand of rz_learn_conv_wgrad_tc (its result's input channels 0..3 are the stem's weight gradient) */
 int rz_learn_planes_to_tile(const float* planes, void* tile, int n_boards, int board_rows, int board_cols, void* stream);
+/* float32 planes [n][n_planes][H][W] (n_planes 4 or 17) -> bf16 tile of stride S, channels 0..n_planes-1 */
+int rz_learn_planes_to_tile_ex(const float* planes, int n_planes, void* tile, int n_boards, int board_rows, int board_cols,
+                               int row_stride, void* stream);
 /* float32 channels-last [n][HW][C] -> bf16 tiles holding the values as (high, low) pairs (hi = bf16(x), lo = bf16(x - hi)):
    mode 0: tile_a[:, 0:C] = hi, tile_a[:, C:2C] = lo (2C <= 128; the layer input); mode 1: tile_a[:, 0:C] = hi,
    tile_b[:, 0:C] = lo (the output gradient).  Two rz_learn_conv_wgrad_tc launches (x pair-tile against the high and the
@@ -475,11 +496,17 @@ int rz_learn_tile_grad_mask_split(float* grad_a, const float* grad_b, const void
                                   void* hi_out, void* lo_out, int n_boards, void* stream);
 /* out[c] = sum over the rows of a bf16 tile [n*256][128] (a bias gradient); scratch: 148 * 2 * 256 floats */
 int rz_learn_tile_colsum(const void* tile, float* out, float* scratch, int n_boards, void* stream);
+int rz_learn_tile_colsum_ex(const void* tile, float* out, float* scratch, int n_boards, int row_stride, void* stream);
 /* grad = dout * (act > 0) on bf16 tiles (ReLU without BatchNorm: the stem) */
 int rz_learn_relu_bwd_bf16(const void* dout, const void* act, void* grad, int n_boards, void* stream);
+int rz_learn_relu_bwd_bf16_ex(const void* dout, const void* act, void* grad, int n_boards, int row_stride, void* stream);
 /* bf16 padded tile layout [n*256][128] <-> float32 [n][HW][128] */
 int rz_learn_tile_to_nhwc(const void* tile, float* out, int n_boards, int board_rows, int board_cols, void* stream);
 int rz_learn_nhwc_to_tile(const float* in, void* tile, int n_boards, int board_rows, int board_cols, void* stream);
+int rz_learn_tile_to_nhwc_ex(const void* tile, float* out, int n_boards, int board_rows, int board_cols, int row_stride,
+                             void* stream);
+int rz_learn_nhwc_to_tile_ex(const float* in, void* tile, int n_boards, int board_rows, int board_cols, int row_stride,
+                             void* stream);
 
 /* ---- pure-MCTS opponent: random playouts (rlzero/mcts/rollout_mcts.py:49-74,96-108) ---------
    prior: uniform over the leaf's legal moves; value: the reference's _evaluate on a uniformly random

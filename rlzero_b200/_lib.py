@@ -11,7 +11,7 @@ import torch  # noqa: F401  -- loads libcudart.so.12 into the process before our
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'librlzero_b200.so')
 
-ABI_VERSION = 12
+ABI_VERSION = 13
 META_STRIDE = 12
 (META_PLAYER, META_LAST_MOVE, META_STONES, META_STATUS, META_WINNER, META_PLY, META_FAULT,
  META_EPISODE, META_KO, META_PASSES) = range(10)
@@ -150,6 +150,17 @@ SIGNATURES = {
     'rz_learn_tile_grad_mask_split': (C.c_int, [_vp, _vp, _vp, C.c_int, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_learn_tile_to_nhwc': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     'rz_learn_nhwc_to_tile': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
+    'rz_learn_conv_wgrad_tc_ex': (C.c_int, [_vp, _vp, _vp, _vp, C.c_longlong, C.c_int, C.c_int, C.c_int, _vp]),
+    'rz_learn_pack_stem_tc_ex': (C.c_int, [_vp, C.c_int, _vp, _vp]),
+    'rz_learn_bn_forward_ex': (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_float, C.c_float, _vp, _vp, C.c_int,
+                                         C.c_int, C.c_int, C.c_int, _vp]),
+    'rz_learn_bn_backward_ex': (C.c_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int,
+                                          _vp]),
+    'rz_learn_planes_to_tile_ex': (C.c_int, [_vp, C.c_int, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),
+    'rz_learn_tile_colsum_ex': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, _vp]),
+    'rz_learn_relu_bwd_bf16_ex': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, _vp]),
+    'rz_learn_tile_to_nhwc_ex': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),
+    'rz_learn_nhwc_to_tile_ex': (C.c_int, [_vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, _vp]),
     'rz_eval_rollout': (C.c_int, [_TD, C.c_int, C.c_ulonglong, C.c_int, _vp, _vp, _vp]),
     'rz_eval_rollout_dm': (C.c_int, [_TD, C.c_int, C.c_ulonglong, C.c_int, _vp, _vp, _vp]),
     'rz_sizeof_mz_desc': (C.c_int, []),

@@ -2,11 +2,13 @@
 //
 // Reference op: AlphaZeroAgent.learn (rlzero/games/gomoku/alphazero_agent.py:59-86) -- loss.backward() +
 // optimizer.step() -- for the ResNet-N policy-value net of SURVEY.md section 7 (conv3x3 + BatchNorm2d in training
-// mode + skip + ReLU).  Activations and gradients travel as bf16 in the padded 16-stride position layout of the
-// inference path ([board*256 + y*16 + x][128 channels], zero at x = 15 / y = 15 / beyond the board), statistics,
-// reductions and parameter gradients are fp32.
+// mode + skip + ReLU).  Activations and gradients travel as bf16 in the padded position layout of the inference path
+// ([board*S*S + y*S + x][128 channels], zero at x >= W / y >= H and in the tail rows up to the multiple of 256 rows),
+// statistics, reductions and parameter gradients are fp32.  The row stride S is 16 for boards up to 15x15 and 20 for
+// 16x16 .. 19x19 (the Go boards of config 4); the _ex entry points take it, the plain ones are their S = 16 calls.
 //
-//   forward convolution   rz_net_conv3x3_tc2 (rz_net_tc2.cu), raw output (bias, no ReLU)
+//   forward convolution   rz_net_conv3x3_tc2 (rz_net_tc2.cu) at S = 16, rz_net_conv3x3_tc3 (rz_net_tc3.cu) at S = 20,
+//                         raw output (bias, no ReLU)
 //   data gradient         the SAME kernel with the weights transposed and the taps mirrored (rz_learn_pack_conv_tc)
 //   weight gradient       rz_conv_wgrad_tc_kernel below: dW[tap][co][ci] = sum_p dy[p][co] * x[p + d(tap)][ci], a
 //                         GEMM whose reduction runs over the POSITIONS.  Both operands are stored position-major
@@ -16,7 +18,10 @@
 //                         so no transpose is ever materialised; the 9 taps are row-shifted descriptors on one halo tile
 //                         of x, as in the forward kernel.  fp32 accumulators stay in TMEM for the whole launch (3 taps
 //                         x 128 columns per CTA); CTAs form triples (one per filter row) that walk the same position
-//                         tiles, so HBM sees each tile once and L2 serves the other two.
+//                         tiles, so HBM sees each tile once and L2 serves the other two.  Templated on S: an (S + 1)-row
+//                         halo, filter rows S rows apart; at S = 20 a tile may straddle two boards (pad squares are 0).
+//   stem                  forward: the inference stem fed from float32 planes (4 planes, or the 17 of GoEnv.observe);
+//                         weight gradient: the kernel above with the planes as channels 0 .. P-1 of a tile
 //   BatchNorm             batch statistics / normalise + skip + ReLU / the two backward reductions / the backward
 //                         apply as row-parallel kernels (a warp owns a row of 128 channels = 256 B).
 #include <cuda_bf16.h>
@@ -30,15 +35,22 @@ namespace {
 // weight gradient on tcgen05
 // ---------------------------------------------------------------------------------------------------------
 constexpr int WG_TILE = 128;                        // positions per tile (the K extent of one stage)
-constexpr int WG_HALO = 17;
-constexpr int WG_XROWS = WG_TILE + 2 * WG_HALO;     // 162
 constexpr int WG_DY_HALF = WG_TILE * 128;           // 16384 B: [128 rows][64 channels]
-constexpr int WG_X_HALF = WG_XROWS * 128;           // 20736 B
-constexpr int WG_STAGE = 2 * WG_DY_HALF + 2 * WG_X_HALF;   // 74240 B
 constexpr int WG_STAGES = 3;
-constexpr int WG_CTRL = WG_STAGES * WG_STAGE;       // 222720
-constexpr int WG_SMEM = WG_CTRL + 1024 + 1024;      // + control block + alignment slack
 constexpr int WG_THREADS = 192;                     // producer warp, MMA warp, 4 drain warps
+
+// the stage geometry of row stride S: x tiles carry an (S + 1)-row halo on each side
+//   S = 16: 162-row x tiles, stages of 74240 B, 224768 B of shared memory
+//   S = 20: 170-row x tiles, stages of 76288 B, 230912 B (the 232448 B limit allows no fourth stage at either stride)
+template <int kS>
+struct WgGeo {
+  static constexpr int HALO = kS + 1;
+  static constexpr int XROWS = WG_TILE + 2 * HALO;
+  static constexpr int X_HALF = XROWS * 128;
+  static constexpr int STAGE = 2 * WG_DY_HALF + 2 * X_HALF;
+  static constexpr int CTRL = WG_STAGES * STAGE;
+  static constexpr int SMEM = CTRL + 1024 + 1024;   // + control block + alignment slack
+};
 
 // MN-major SWIZZLE_128B operand: start address, LBO = byte distance between the two 64-channel halves, SBO = 1024 B
 // between 8-row groups along K (cute::UMMA::make_umma_desc<Major::MN> for Layout_MN_SW128_Atom)
@@ -63,15 +75,18 @@ struct WgradParams {
   int n_splits;
 };
 
+template <int kS>
 __global__ void __launch_bounds__(WG_THREADS, 1)
 rz_conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid_constant__ CUtensorMap tmap_dy,
                         const WgradParams p) {
+  using G = WgGeo<kS>;
+  static_assert(G::SMEM <= 232448, "shared memory budget");
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (rz::smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* al = smem_raw + (base - rz::smem_u32(smem_raw));
-  const uint32_t ctrl = base + WG_CTRL;
+  const uint32_t ctrl = base + G::CTRL;
   const uint32_t bar_full = ctrl, bar_empty = ctrl + 32, bar_done = ctrl + 64;
-  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(al + WG_CTRL + 96);
+  uint32_t* tmem_holder = reinterpret_cast<uint32_t*>(al + G::CTRL + 96);
   const int warp = rz::uniform_i32((int)(threadIdx.x >> 5)), lane = threadIdx.x & 31;
   const int split = blockIdx.x / 3, row_grp = blockIdx.x % 3;       // filter row dy = row_grp - 1
 
@@ -94,12 +109,12 @@ rz_conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid
       for (int it = 0; it < n_my; ++it) {
         const int st = it % WG_STAGES;
         rz::mbar_wait(bar_empty + 8 * st, ((uint32_t)(it / WG_STAGES) & 1u) ^ 1u);
-        rz::mbar_expect_tx(bar_full + 8 * st, (uint32_t)WG_STAGE);
+        rz::mbar_expect_tx(bar_full + 8 * st, (uint32_t)G::STAGE);
         const int row0 = (split + it * p.n_splits) * WG_TILE;
-        const uint32_t sb = base + (uint32_t)st * WG_STAGE;
+        const uint32_t sb = base + (uint32_t)st * G::STAGE;
         for (int h = 0; h < 2; ++h) {
           rz::tma_load_2d(sb + (uint32_t)h * WG_DY_HALF, &tmap_dy, bar_full + 8 * st, h * 64, row0);
-          rz::tma_load_2d(sb + 2u * WG_DY_HALF + (uint32_t)h * WG_X_HALF, &tmap_x, bar_full + 8 * st, h * 64, row0 - WG_HALO);
+          rz::tma_load_2d(sb + 2u * WG_DY_HALF + (uint32_t)h * G::X_HALF, &tmap_x, bar_full + 8 * st, h * 64, row0 - G::HALO);
         }
       }
     }
@@ -111,14 +126,14 @@ rz_conv_wgrad_tc_kernel(const __grid_constant__ CUtensorMap tmap_x, const __grid
       const int st = it % WG_STAGES;
       rz::mbar_wait(bar_full + 8 * st, (uint32_t)(it / WG_STAGES) & 1u);
       rz::tc_fence_after();
-      const uint32_t dyb = base + (uint32_t)st * WG_STAGE, xb = dyb + 2u * WG_DY_HALF;
+      const uint32_t dyb = base + (uint32_t)st * G::STAGE, xb = dyb + 2u * WG_DY_HALF;
 #pragma unroll 1
       for (int t = 0; t < 3; ++t) {
-        const int shift = WG_HALO + (row_grp - 1) * 16 + (t - 1);        // rows into the halo tile of x
+        const int shift = G::HALO + (row_grp - 1) * kS + (t - 1);        // rows into the halo tile of x
 #pragma unroll
         for (int ks = 0; ks < WG_TILE / 16; ++ks) {
           const uint64_t adesc = umma_desc_mn_sw128(dyb + (uint32_t)ks * 2048u, WG_DY_HALF);
-          const uint64_t bdesc = umma_desc_mn_sw128(xb + (uint32_t)(shift + ks * 16) * 128u, WG_X_HALF);
+          const uint64_t bdesc = umma_desc_mn_sw128(xb + (uint32_t)(shift + ks * 16) * 128u, G::X_HALF);
           rz::umma_bf16_pred(tmem_u + (uint32_t)(t * 128), adesc, bdesc, idesc, (it > 0 || ks > 0) ? 1u : 0u, issue);
         }
       }
@@ -204,6 +219,15 @@ __global__ void rz_pack_stem_tc_kernel(const float* __restrict__ w, __nv_bfloat1
   if (k < 36) { const int tap = k >> 2, pl = k & 3; v = w[((size_t)co * 4 + pl) * 9 + tap]; }
   ws[i] = __float2bfloat16_rn(v);
 }
+// Go stem: fp32 [128][17][3][3] -> bf16 [128][192], k = tap*17 + plane, zero from 153 (rz_net_stem_go_tc's layout)
+__global__ void rz_pack_stem_go_tc_kernel(const float* __restrict__ w, __nv_bfloat16* __restrict__ ws) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= 128 * 192) return;
+  const int k = i % 192, co = i / 192;
+  float v = 0.0f;
+  if (k < 153) { const int tap = k / 17, pl = k % 17; v = w[((size_t)co * 17 + pl) * 9 + tap]; }
+  ws[i] = __float2bfloat16_rn(v);
+}
 
 // ---------------------------------------------------------------------------------------------------------
 // row-parallel helpers: a warp owns a row (128 channels bf16 = 256 B), a lane 4 channels
@@ -225,6 +249,26 @@ __device__ __forceinline__ void st_bf16x4(__nv_bfloat16* p, const f4& r) {
 __device__ __forceinline__ bool row_on_board(long long row, int H, int W) {
   const int pos = (int)(row & 255);
   return (pos & 15) < W && (pos >> 4) < H;
+}
+// row r of the padded layout of stride kS (row = board*S*S + y*S + x) -> board, y, x
+template <int kS>
+__device__ __forceinline__ void row_pos(long long r, long long& b, int& y, int& x) {
+  if (kS == 16) {
+    const int pos = (int)(r & 255);
+    b = r >> 8; y = pos >> 4; x = pos & 15;
+  } else {
+    b = r / (kS * kS);
+    const int pos = (int)(r - b * (kS * kS));
+    y = pos / kS; x = pos - y * kS;
+  }
+}
+// a board square: x < W, y < H, and not one of the tail rows n*S*S .. round_up(n*S*S, 256) (there are none at S = 16)
+template <int kS>
+__device__ __forceinline__ bool row_on_board_s(long long r, int H, int W, long long n_valid) {
+  long long b;
+  int y, x;
+  row_pos<kS>(r, b, y, x);
+  return (kS == 16 || r < n_valid) && x < W && y < H;
 }
 
 // per-block partial sums of two per-channel quantities over the rows: part[blk][2][128]
@@ -315,16 +359,18 @@ rz_bn_finalize_kernel(const float* __restrict__ part, int n_blocks, double count
 }
 
 // a = relu(y * scale + shift (+ skip)), zero off the board
+template <int kS>
 __global__ void __launch_bounds__(256)
 rz_bn_apply_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict__ scale, const float* __restrict__ shift,
-                   const __nv_bfloat16* __restrict__ skip, __nv_bfloat16* __restrict__ out, long long rows, int H, int W) {
+                   const __nv_bfloat16* __restrict__ skip, __nv_bfloat16* __restrict__ out, long long rows,
+                   long long n_valid, int H, int W) {
   const int lane = threadIdx.x & 31, c0 = lane * 4;
   float sc[4], sh[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) { sc[e] = scale[c0 + e]; sh[e] = shift[c0 + e]; }
   for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     f4 o;
-    if (row_on_board(r, H, W)) {
+    if (row_on_board_s<kS>(r, H, W, n_valid)) {
       const f4 yv = ld_bf16x4(y + r * 128 + c0);
 #pragma unroll
       for (int e = 0; e < 4; ++e) o.v[e] = fmaf(yv.v[e], sc[e], sh[e]);
@@ -344,19 +390,20 @@ rz_bn_apply_kernel(const __nv_bfloat16* __restrict__ y, const float* __restrict_
 }
 
 // dy = scale * (dz - c1 - xhat * c2), dz = dout * (a > 0); optionally dz itself (the gradient that flows into the skip)
+template <int kS>
 __global__ void __launch_bounds__(256)
 rz_bn_bwd_apply_kernel(const __nv_bfloat16* __restrict__ dout, const __nv_bfloat16* __restrict__ a,
                        const __nv_bfloat16* __restrict__ y, const float* __restrict__ mean,
                        const float* __restrict__ invstd, const float* __restrict__ scale, const float* __restrict__ c1,
                        const float* __restrict__ c2, __nv_bfloat16* __restrict__ dy, __nv_bfloat16* __restrict__ dz_out,
-                       long long rows, int H, int W) {
+                       long long rows, long long n_valid, int H, int W) {
   const int lane = threadIdx.x & 31, c0 = lane * 4;
   float mu[4], is[4], sc[4], k1[4], k2[4];
 #pragma unroll
   for (int e = 0; e < 4; ++e) { mu[e] = mean[c0 + e]; is[e] = invstd[c0 + e]; sc[e] = scale[c0 + e]; k1[e] = c1[c0 + e]; k2[e] = c2[c0 + e]; }
   for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     f4 o, z;
-    if (row_on_board(r, H, W)) {
+    if (row_on_board_s<kS>(r, H, W, n_valid)) {
       const f4 dv = ld_bf16x4(dout + r * 128 + c0), av = ld_bf16x4(a + r * 128 + c0), yv = ld_bf16x4(y + r * 128 + c0);
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
@@ -386,26 +433,30 @@ rz_relu_bwd_bf16_kernel(const __nv_bfloat16* __restrict__ dout, const __nv_bfloa
   }
 }
 
-// padded bf16 tile layout [n*256][128] <-> float32 [n][HW][128]
+// padded bf16 tile layout [round_up(n*S*S, 256)][128] <-> float32 [n][HW][128]
+template <int kS>
 __global__ void __launch_bounds__(256)
 rz_tile_to_nhwc_kernel(const __nv_bfloat16* __restrict__ tile, float* __restrict__ out, int n, int H, int W) {
   const int lane = threadIdx.x & 31, c0 = lane * 4, HW = H * W;
   const long long rows = (long long)n * HW;
   for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     const int b = (int)(r / HW), pos = (int)(r - (long long)b * HW);
-    const f4 v = ld_bf16x4(tile + ((long long)b * 256 + (pos / W) * 16 + pos % W) * 128 + c0);
+    const f4 v = ld_bf16x4(tile + ((long long)b * (kS * kS) + (pos / W) * kS + pos % W) * 128 + c0);
     *reinterpret_cast<float4*>(out + r * 128 + c0) = make_float4(v.v[0], v.v[1], v.v[2], v.v[3]);
   }
 }
+template <int kS>
 __global__ void __launch_bounds__(256)
-rz_nhwc_to_tile_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__ tile, int n, int H, int W) {
+rz_nhwc_to_tile_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__ tile, long long rows, int n, int H, int W) {
   const int lane = threadIdx.x & 31, c0 = lane * 4, HW = H * W;
-  const long long rows = (long long)n * 256;
+  const long long n_valid = (long long)n * (kS * kS);
   for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     f4 o;
-    if (row_on_board(r, H, W)) {
-      const int pos = (int)(r & 255);
-      const float4 v = *reinterpret_cast<const float4*>(in + ((r >> 8) * HW + (pos >> 4) * W + (pos & 15)) * 128 + c0);
+    if (row_on_board_s<kS>(r, H, W, n_valid)) {
+      long long b;
+      int y, x;
+      row_pos<kS>(r, b, y, x);
+      const float4 v = *reinterpret_cast<const float4*>(in + (b * HW + y * W + x) * 128 + c0);
       o.v[0] = v.x; o.v[1] = v.y; o.v[2] = v.z; o.v[3] = v.w;
     } else {
       o.v[0] = o.v[1] = o.v[2] = o.v[3] = 0.0f;
@@ -414,20 +465,25 @@ rz_nhwc_to_tile_kernel(const float* __restrict__ in, __nv_bfloat16* __restrict__
   }
 }
 
-// float32 observation planes [n][4][H][W] -> bf16 tile layout [n*256][128], channels 0..3 (the rest zero): the stem's
-// input as an operand of the tensor-core weight-gradient kernel (planes are 0/1: exact in bf16)
+// float32 observation planes [n][n_planes][H][W] -> bf16 tile layout [round_up(n*S*S, 256)][128], channels
+// 0..n_planes-1 (the rest zero): the stem's input as an operand of the tensor-core weight-gradient kernel (planes are
+// 0/1: exact in bf16)
+template <int kS>
 __global__ void __launch_bounds__(256)
-rz_planes_to_tile_kernel(const float* __restrict__ planes, __nv_bfloat16* __restrict__ tile, int n, int H, int W) {
+rz_planes_to_tile_kernel(const float* __restrict__ planes, int n_planes, __nv_bfloat16* __restrict__ tile, long long rows,
+                         int n, int H, int W) {
   const int lane = threadIdx.x & 31, c0 = lane * 4, HW = H * W;
-  const long long rows = (long long)n * 256;
+  const long long n_valid = (long long)n * (kS * kS);
   for (long long r = (long long)blockIdx.x * 8 + (threadIdx.x >> 5); r < rows; r += (long long)gridDim.x * 8) {
     f4 o;
     o.v[0] = o.v[1] = o.v[2] = o.v[3] = 0.0f;
-    if (lane == 0 && row_on_board(r, H, W)) {
-      const int pos = (int)(r & 255);
-      const float* src = planes + (r >> 8) * 4 * HW + (pos >> 4) * W + (pos & 15);
+    if (c0 < n_planes && row_on_board_s<kS>(r, H, W, n_valid)) {
+      long long b;
+      int y, x;
+      row_pos<kS>(r, b, y, x);
+      const float* src = planes + (b * n_planes + c0) * HW + y * W + x;
 #pragma unroll
-      for (int e = 0; e < 4; ++e) o.v[e] = src[e * HW];
+      for (int e = 0; e < 4; ++e) if (c0 + e < n_planes) o.v[e] = src[e * HW];
     }
     st_bf16x4(tile + r * 128 + c0, o);
   }
@@ -528,38 +584,62 @@ inline int row_grid(long long rows) {
 }
 constexpr int BN_BLOCKS = 148 * 2;
 
+// rows of a tensor in the padded layout of stride S: round_up(n*S*S, 256) (n*256 at S = 16)
+inline long long layout_rows(int n_boards, int S) { return ((long long)n_boards * S * S + 255) / 256 * 256; }
+
+template <int kS>
+int wgrad_launch(const void* x, const void* dy, float* dw_oihw, float* scratch, int n_boards, int splits, int n_tiles,
+                 cudaStream_t st) {
+  static bool attr_set = false;
+  if (!attr_set) {
+    cudaError_t e = cudaFuncSetAttribute(rz_conv_wgrad_tc_kernel<kS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         WgGeo<kS>::SMEM);
+    if (e != cudaSuccess) { rz_set_error("rz_learn_conv_wgrad_tc_ex: smem attribute: %s", cudaGetErrorString(e)); return -2; }
+    attr_set = true;
+  }
+  // the tensor maps end at n*S*S rows: TMA fills the halo before row 0 and a partial last tile with zeros
+  CUtensorMap tmap_x, tmap_dy;
+  if (rz::make_tmap_2d(&tmap_x, x, (uint64_t)n_boards * kS * kS, 128, WgGeo<kS>::XROWS)) return -1;
+  if (rz::make_tmap_2d(&tmap_dy, dy, (uint64_t)n_boards * kS * kS, 128, WG_TILE)) return -1;
+  WgradParams p;
+  p.part = scratch; p.n_tiles = n_tiles; p.n_splits = splits;
+  rz_conv_wgrad_tc_kernel<kS><<<splits * 3, WG_THREADS, WgGeo<kS>::SMEM, st>>>(tmap_x, tmap_dy, p);
+  rz_wgrad_tc_final_kernel<<<(9 * 128 * 128 + 255) / 256, 256, 0, st>>>(scratch, dw_oihw, splits);
+  RZ_LAUNCH_CHECK("rz_learn_conv_wgrad_tc_ex");
+  return 0;
+}
+
 }  // namespace
+
+#define RZ_REQUIRE_STRIDE(fn, S) RZ_REQUIRE((S) == 16 || (S) == 20, fn ": row_stride %d (16 or 20)", (S))
+#define RZ_REQUIRE_BOARD(fn, H, W, S)                                                                              \
+  RZ_REQUIRE((H) >= 1 && (H) < (S) && (W) >= 1 && (W) < (S), fn ": board %dx%d does not fit row_stride %d", (H), (W), (S))
 
 // =========================================================================================================
 // C ABI
 // =========================================================================================================
-extern "C" int rz_learn_conv_wgrad_tc(const void* x, const void* dy, float* dw_oihw, float* scratch,
-                                      long long scratch_floats, int n_boards, int n_ctas, void* stream) {
-  RZ_REQUIRE(x && dy && dw_oihw && scratch && n_boards >= 1, "rz_learn_conv_wgrad_tc: bad arguments");
+extern "C" int rz_learn_conv_wgrad_tc_ex(const void* x, const void* dy, float* dw_oihw, float* scratch,
+                                         long long scratch_floats, int n_boards, int row_stride, int n_ctas,
+                                         void* stream) {
+  RZ_REQUIRE(x && dy && dw_oihw && scratch && n_boards >= 1, "rz_learn_conv_wgrad_tc_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_conv_wgrad_tc_ex", row_stride);
   int ctas = n_ctas > 0 ? n_ctas : 147;
   ctas = ctas / 3 * 3;
   if (ctas < 3) ctas = 3;
-  const int n_tiles = n_boards * 2;
+  const long long n_tiles = ((long long)n_boards * row_stride * row_stride + WG_TILE - 1) / WG_TILE;
+  RZ_REQUIRE(n_tiles < (1LL << 30), "rz_learn_conv_wgrad_tc_ex: %d boards", n_boards);
   int splits = ctas / 3;
-  if (splits > n_tiles) splits = n_tiles;
-  RZ_REQUIRE(scratch_floats >= (long long)splits * 9 * 128 * 128, "rz_learn_conv_wgrad_tc: scratch holds %lld floats, %lld needed",
+  if (splits > n_tiles) splits = (int)n_tiles;
+  RZ_REQUIRE(scratch_floats >= (long long)splits * 9 * 128 * 128, "rz_learn_conv_wgrad_tc_ex: scratch holds %lld floats, %lld needed",
              scratch_floats, (long long)splits * 9 * 128 * 128);
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(rz_conv_wgrad_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, WG_SMEM);
-    if (e != cudaSuccess) { rz_set_error("rz_learn_conv_wgrad_tc: smem attribute: %s", cudaGetErrorString(e)); return -2; }
-    attr_set = true;
-  }
-  CUtensorMap tmap_x, tmap_dy;
-  if (rz::make_tmap_2d(&tmap_x, x, (uint64_t)n_boards * 256, 128, WG_XROWS)) return -1;
-  if (rz::make_tmap_2d(&tmap_dy, dy, (uint64_t)n_boards * 256, 128, WG_TILE)) return -1;
-  WgradParams p;
-  p.part = scratch; p.n_tiles = n_tiles; p.n_splits = splits;
   cudaStream_t st = (cudaStream_t)stream;
-  rz_conv_wgrad_tc_kernel<<<splits * 3, WG_THREADS, WG_SMEM, st>>>(tmap_x, tmap_dy, p);
-  rz_wgrad_tc_final_kernel<<<(9 * 128 * 128 + 255) / 256, 256, 0, st>>>(scratch, dw_oihw, splits);
-  RZ_LAUNCH_CHECK("rz_learn_conv_wgrad_tc");
-  return 0;
+  return row_stride == 16 ? wgrad_launch<16>(x, dy, dw_oihw, scratch, n_boards, splits, (int)n_tiles, st)
+                          : wgrad_launch<20>(x, dy, dw_oihw, scratch, n_boards, splits, (int)n_tiles, st);
+}
+
+extern "C" int rz_learn_conv_wgrad_tc(const void* x, const void* dy, float* dw_oihw, float* scratch,
+                                      long long scratch_floats, int n_boards, int n_ctas, void* stream) {
+  return rz_learn_conv_wgrad_tc_ex(x, dy, dw_oihw, scratch, scratch_floats, n_boards, 16, n_ctas, stream);
 }
 
 extern "C" int rz_learn_pack_conv_tc(const float* w_oihw, void* w_fwd, void* w_bwd, void* stream) {
@@ -581,36 +661,61 @@ extern "C" int rz_net_pack_conv_bn_tc(const float* w_oihw, const float* conv_bia
   return 0;
 }
 
-extern "C" int rz_learn_pack_stem_tc(const float* w_oihw, void* w_stem, void* stream) {
-  RZ_REQUIRE(w_oihw && w_stem, "rz_learn_pack_stem_tc: null argument");
-  rz_pack_stem_tc_kernel<<<(128 * 64 + 255) / 256, 256, 0, (cudaStream_t)stream>>>(w_oihw, (__nv_bfloat16*)w_stem);
-  RZ_LAUNCH_CHECK("rz_learn_pack_stem_tc");
+extern "C" int rz_learn_pack_stem_tc_ex(const float* w_oihw, int in_planes, void* w_stem, void* stream) {
+  RZ_REQUIRE(w_oihw && w_stem, "rz_learn_pack_stem_tc_ex: null argument");
+  RZ_REQUIRE(in_planes == 4 || in_planes == 17, "rz_learn_pack_stem_tc_ex: in_planes %d (4 or 17)", in_planes);
+  if (in_planes == 4)
+    rz_pack_stem_tc_kernel<<<(128 * 64 + 255) / 256, 256, 0, (cudaStream_t)stream>>>(w_oihw, (__nv_bfloat16*)w_stem);
+  else
+    rz_pack_stem_go_tc_kernel<<<(128 * 192 + 255) / 256, 256, 0, (cudaStream_t)stream>>>(w_oihw, (__nv_bfloat16*)w_stem);
+  RZ_LAUNCH_CHECK("rz_learn_pack_stem_tc_ex");
   return 0;
 }
 
-extern "C" int rz_learn_bn_forward(const void* y, const void* skip, void* out, const float* gamma, const float* beta,
-                                   float* running_mean, float* running_var, float eps, float momentum, float* stats,
-                                   float* scratch, int n_boards, int board_rows, int board_cols, void* stream) {
-  RZ_REQUIRE(y && out && gamma && beta && stats && scratch && n_boards >= 1, "rz_learn_bn_forward: bad arguments");
-  RZ_REQUIRE(board_rows >= 1 && board_rows <= 15 && board_cols >= 1 && board_cols <= 15, "rz_learn_bn_forward: board %dx%d", board_rows, board_cols);
-  const long long rows = (long long)n_boards * 256;
+extern "C" int rz_learn_pack_stem_tc(const float* w_oihw, void* w_stem, void* stream) {
+  return rz_learn_pack_stem_tc_ex(w_oihw, 4, w_stem, stream);
+}
+
+extern "C" int rz_learn_bn_forward_ex(const void* y, const void* skip, void* out, const float* gamma, const float* beta,
+                                      float* running_mean, float* running_var, float eps, float momentum, float* stats,
+                                      float* scratch, int n_boards, int board_rows, int board_cols, int row_stride,
+                                      void* stream) {
+  RZ_REQUIRE(y && out && gamma && beta && stats && scratch && n_boards >= 1, "rz_learn_bn_forward_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_bn_forward_ex", row_stride);
+  RZ_REQUIRE_BOARD("rz_learn_bn_forward_ex", board_rows, board_cols, row_stride);
+  const long long rows = layout_rows(n_boards, row_stride), n_valid = (long long)n_boards * row_stride * row_stride;
   const int blocks = row_grid(rows) < BN_BLOCKS ? row_grid(rows) : BN_BLOCKS;
   cudaStream_t st = (cudaStream_t)stream;
   rz_bn_reduce_kernel<0><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)y, nullptr, nullptr, nullptr, nullptr, rows, scratch);
   // stats: [4][128] = mean, invstd, scale, shift
   rz_bn_finalize_kernel<<<1, 1024, 0, st>>>(scratch, blocks, (double)n_boards * board_rows * board_cols, 0, gamma, beta, eps,
                                           momentum, running_mean, running_var, stats, stats + 128, stats + 256, stats + 384);
-  rz_bn_apply_kernel<<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)y, stats + 256, stats + 384,
-                                                    (const __nv_bfloat16*)skip, (__nv_bfloat16*)out, rows, board_rows, board_cols);
-  RZ_LAUNCH_CHECK("rz_learn_bn_forward");
+  if (row_stride == 16)
+    rz_bn_apply_kernel<16><<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)y, stats + 256, stats + 384,
+                                                          (const __nv_bfloat16*)skip, (__nv_bfloat16*)out, rows, n_valid,
+                                                          board_rows, board_cols);
+  else
+    rz_bn_apply_kernel<20><<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)y, stats + 256, stats + 384,
+                                                          (const __nv_bfloat16*)skip, (__nv_bfloat16*)out, rows, n_valid,
+                                                          board_rows, board_cols);
+  RZ_LAUNCH_CHECK("rz_learn_bn_forward_ex");
   return 0;
 }
 
-extern "C" int rz_learn_bn_backward(const void* dout, const void* act, const void* y, const float* stats, float* dgamma,
-                                    float* dbeta, void* dy, void* dz_out, float* scratch, int n_boards, int board_rows,
-                                    int board_cols, void* stream) {
-  RZ_REQUIRE(dout && act && y && stats && dgamma && dbeta && dy && scratch && n_boards >= 1, "rz_learn_bn_backward: bad arguments");
-  const long long rows = (long long)n_boards * 256;
+extern "C" int rz_learn_bn_forward(const void* y, const void* skip, void* out, const float* gamma, const float* beta,
+                                   float* running_mean, float* running_var, float eps, float momentum, float* stats,
+                                   float* scratch, int n_boards, int board_rows, int board_cols, void* stream) {
+  return rz_learn_bn_forward_ex(y, skip, out, gamma, beta, running_mean, running_var, eps, momentum, stats, scratch,
+                                n_boards, board_rows, board_cols, 16, stream);
+}
+
+extern "C" int rz_learn_bn_backward_ex(const void* dout, const void* act, const void* y, const float* stats, float* dgamma,
+                                       float* dbeta, void* dy, void* dz_out, float* scratch, int n_boards, int board_rows,
+                                       int board_cols, int row_stride, void* stream) {
+  RZ_REQUIRE(dout && act && y && stats && dgamma && dbeta && dy && scratch && n_boards >= 1, "rz_learn_bn_backward_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_bn_backward_ex", row_stride);
+  RZ_REQUIRE_BOARD("rz_learn_bn_backward_ex", board_rows, board_cols, row_stride);
+  const long long rows = layout_rows(n_boards, row_stride), n_valid = (long long)n_boards * row_stride * row_stride;
   const int blocks = row_grid(rows) < BN_BLOCKS ? row_grid(rows) : BN_BLOCKS;
   cudaStream_t st = (cudaStream_t)stream;
   rz_bn_reduce_kernel<1><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)y, (const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
@@ -618,20 +723,48 @@ extern "C" int rz_learn_bn_backward(const void* dout, const void* act, const voi
   float* coef = scratch + (size_t)BN_BLOCKS * 256;        // c1, c2
   rz_bn_finalize_kernel<<<1, 1024, 0, st>>>(scratch, blocks, (double)n_boards * board_rows * board_cols, 1, nullptr, nullptr, 0.0f,
                                           0.0f, nullptr, nullptr, dgamma, dbeta, coef, coef + 128);
-  rz_bn_bwd_apply_kernel<<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
-                                                        (const __nv_bfloat16*)y, stats, stats + 128, stats + 256, coef, coef + 128,
-                                                        (__nv_bfloat16*)dy, (__nv_bfloat16*)dz_out, rows, board_rows, board_cols);
-  RZ_LAUNCH_CHECK("rz_learn_bn_backward");
+  if (row_stride == 16)
+    rz_bn_bwd_apply_kernel<16><<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
+                                                              (const __nv_bfloat16*)y, stats, stats + 128, stats + 256, coef,
+                                                              coef + 128, (__nv_bfloat16*)dy, (__nv_bfloat16*)dz_out, rows,
+                                                              n_valid, board_rows, board_cols);
+  else
+    rz_bn_bwd_apply_kernel<20><<<row_grid(rows), 256, 0, st>>>((const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
+                                                              (const __nv_bfloat16*)y, stats, stats + 128, stats + 256, coef,
+                                                              coef + 128, (__nv_bfloat16*)dy, (__nv_bfloat16*)dz_out, rows,
+                                                              n_valid, board_rows, board_cols);
+  RZ_LAUNCH_CHECK("rz_learn_bn_backward_ex");
+  return 0;
+}
+
+extern "C" int rz_learn_bn_backward(const void* dout, const void* act, const void* y, const float* stats, float* dgamma,
+                                    float* dbeta, void* dy, void* dz_out, float* scratch, int n_boards, int board_rows,
+                                    int board_cols, void* stream) {
+  return rz_learn_bn_backward_ex(dout, act, y, stats, dgamma, dbeta, dy, dz_out, scratch, n_boards, board_rows, board_cols,
+                                 16, stream);
+}
+
+extern "C" int rz_learn_planes_to_tile_ex(const float* planes, int n_planes, void* tile, int n_boards, int board_rows,
+                                          int board_cols, int row_stride, void* stream) {
+  RZ_REQUIRE(planes && tile && n_boards >= 1, "rz_learn_planes_to_tile_ex: bad arguments");
+  RZ_REQUIRE(n_planes == 4 || n_planes == 17, "rz_learn_planes_to_tile_ex: n_planes %d (4 or 17)", n_planes);
+  RZ_REQUIRE_STRIDE("rz_learn_planes_to_tile_ex", row_stride);
+  RZ_REQUIRE_BOARD("rz_learn_planes_to_tile_ex", board_rows, board_cols, row_stride);
+  const long long rows = layout_rows(n_boards, row_stride);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (row_stride == 16)
+    rz_planes_to_tile_kernel<16><<<row_grid(rows), 256, 0, st>>>(planes, n_planes, (__nv_bfloat16*)tile, rows, n_boards,
+                                                                board_rows, board_cols);
+  else
+    rz_planes_to_tile_kernel<20><<<row_grid(rows), 256, 0, st>>>(planes, n_planes, (__nv_bfloat16*)tile, rows, n_boards,
+                                                                board_rows, board_cols);
+  RZ_LAUNCH_CHECK("rz_learn_planes_to_tile_ex");
   return 0;
 }
 
 extern "C" int rz_learn_planes_to_tile(const float* planes, void* tile, int n_boards, int board_rows, int board_cols,
                                        void* stream) {
-  RZ_REQUIRE(planes && tile && n_boards >= 1 && board_rows <= 15 && board_cols <= 15, "rz_learn_planes_to_tile: bad arguments");
-  rz_planes_to_tile_kernel<<<row_grid((long long)n_boards * 256), 256, 0, (cudaStream_t)stream>>>(
-      planes, (__nv_bfloat16*)tile, n_boards, board_rows, board_cols);
-  RZ_LAUNCH_CHECK("rz_learn_planes_to_tile");
-  return 0;
+  return rz_learn_planes_to_tile_ex(planes, 4, tile, n_boards, board_rows, board_cols, 16, stream);
 }
 
 extern "C" int rz_learn_nhwc_to_tile_hilo(const float* in, int channels, void* tile_a, void* tile_b, int mode, int n_boards,
@@ -677,39 +810,73 @@ extern "C" int rz_learn_tile_grad_mask_split(float* grad_a, const float* grad_b,
   return 0;
 }
 
-extern "C" int rz_learn_tile_colsum(const void* tile, float* out, float* scratch, int n_boards, void* stream) {
-  RZ_REQUIRE(tile && out && scratch && n_boards >= 1, "rz_learn_tile_colsum: bad arguments");
-  const long long rows = (long long)n_boards * 256;
+extern "C" int rz_learn_tile_colsum_ex(const void* tile, float* out, float* scratch, int n_boards, int row_stride,
+                                       void* stream) {
+  RZ_REQUIRE(tile && out && scratch && n_boards >= 1, "rz_learn_tile_colsum_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_tile_colsum_ex", row_stride);
+  const long long rows = layout_rows(n_boards, row_stride);
   const int blocks = row_grid(rows) < BN_BLOCKS ? row_grid(rows) : BN_BLOCKS;
   cudaStream_t st = (cudaStream_t)stream;
   rz_bn_reduce_kernel<0><<<blocks, 256, 0, st>>>((const __nv_bfloat16*)tile, nullptr, nullptr, nullptr, nullptr, rows, scratch);
   rz_bn_finalize_kernel<<<1, 1024, 0, st>>>(scratch, blocks, 1.0, 2, nullptr, nullptr, 0.0f, 0.0f, nullptr, nullptr, out, nullptr,
                                            nullptr, nullptr);
-  RZ_LAUNCH_CHECK("rz_learn_tile_colsum");
+  RZ_LAUNCH_CHECK("rz_learn_tile_colsum_ex");
+  return 0;
+}
+
+extern "C" int rz_learn_tile_colsum(const void* tile, float* out, float* scratch, int n_boards, void* stream) {
+  return rz_learn_tile_colsum_ex(tile, out, scratch, n_boards, 16, stream);
+}
+
+extern "C" int rz_learn_relu_bwd_bf16_ex(const void* dout, const void* act, void* grad, int n_boards, int row_stride,
+                                         void* stream) {
+  RZ_REQUIRE(dout && act && grad && n_boards >= 1, "rz_learn_relu_bwd_bf16_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_relu_bwd_bf16_ex", row_stride);
+  const long long rows = layout_rows(n_boards, row_stride);
+  rz_relu_bwd_bf16_kernel<<<row_grid(rows), 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
+                                                                            (__nv_bfloat16*)grad, rows);
+  RZ_LAUNCH_CHECK("rz_learn_relu_bwd_bf16_ex");
   return 0;
 }
 
 extern "C" int rz_learn_relu_bwd_bf16(const void* dout, const void* act, void* grad, int n_boards, void* stream) {
-  RZ_REQUIRE(dout && act && grad && n_boards >= 1, "rz_learn_relu_bwd_bf16: bad arguments");
-  const long long rows = (long long)n_boards * 256;
-  rz_relu_bwd_bf16_kernel<<<row_grid(rows), 256, 0, (cudaStream_t)stream>>>((const __nv_bfloat16*)dout, (const __nv_bfloat16*)act,
-                                                                            (__nv_bfloat16*)grad, rows);
-  RZ_LAUNCH_CHECK("rz_learn_relu_bwd_bf16");
+  return rz_learn_relu_bwd_bf16_ex(dout, act, grad, n_boards, 16, stream);
+}
+
+extern "C" int rz_learn_tile_to_nhwc_ex(const void* tile, float* out, int n_boards, int board_rows, int board_cols,
+                                        int row_stride, void* stream) {
+  RZ_REQUIRE(tile && out && n_boards >= 1, "rz_learn_tile_to_nhwc_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_tile_to_nhwc_ex", row_stride);
+  RZ_REQUIRE_BOARD("rz_learn_tile_to_nhwc_ex", board_rows, board_cols, row_stride);
+  const int grid = row_grid((long long)n_boards * board_rows * board_cols);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (row_stride == 16)
+    rz_tile_to_nhwc_kernel<16><<<grid, 256, 0, st>>>((const __nv_bfloat16*)tile, out, n_boards, board_rows, board_cols);
+  else
+    rz_tile_to_nhwc_kernel<20><<<grid, 256, 0, st>>>((const __nv_bfloat16*)tile, out, n_boards, board_rows, board_cols);
+  RZ_LAUNCH_CHECK("rz_learn_tile_to_nhwc_ex");
   return 0;
 }
 
 extern "C" int rz_learn_tile_to_nhwc(const void* tile, float* out, int n_boards, int board_rows, int board_cols, void* stream) {
-  RZ_REQUIRE(tile && out && n_boards >= 1 && board_rows <= 15 && board_cols <= 15, "rz_learn_tile_to_nhwc: bad arguments");
-  rz_tile_to_nhwc_kernel<<<row_grid((long long)n_boards * board_rows * board_cols), 256, 0, (cudaStream_t)stream>>>(
-      (const __nv_bfloat16*)tile, out, n_boards, board_rows, board_cols);
-  RZ_LAUNCH_CHECK("rz_learn_tile_to_nhwc");
+  return rz_learn_tile_to_nhwc_ex(tile, out, n_boards, board_rows, board_cols, 16, stream);
+}
+
+extern "C" int rz_learn_nhwc_to_tile_ex(const float* in, void* tile, int n_boards, int board_rows, int board_cols,
+                                        int row_stride, void* stream) {
+  RZ_REQUIRE(in && tile && n_boards >= 1, "rz_learn_nhwc_to_tile_ex: bad arguments");
+  RZ_REQUIRE_STRIDE("rz_learn_nhwc_to_tile_ex", row_stride);
+  RZ_REQUIRE_BOARD("rz_learn_nhwc_to_tile_ex", board_rows, board_cols, row_stride);
+  const long long rows = layout_rows(n_boards, row_stride);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (row_stride == 16)
+    rz_nhwc_to_tile_kernel<16><<<row_grid(rows), 256, 0, st>>>(in, (__nv_bfloat16*)tile, rows, n_boards, board_rows, board_cols);
+  else
+    rz_nhwc_to_tile_kernel<20><<<row_grid(rows), 256, 0, st>>>(in, (__nv_bfloat16*)tile, rows, n_boards, board_rows, board_cols);
+  RZ_LAUNCH_CHECK("rz_learn_nhwc_to_tile_ex");
   return 0;
 }
 
 extern "C" int rz_learn_nhwc_to_tile(const float* in, void* tile, int n_boards, int board_rows, int board_cols, void* stream) {
-  RZ_REQUIRE(in && tile && n_boards >= 1 && board_rows <= 15 && board_cols <= 15, "rz_learn_nhwc_to_tile: bad arguments");
-  rz_nhwc_to_tile_kernel<<<row_grid((long long)n_boards * 256), 256, 0, (cudaStream_t)stream>>>(
-      in, (__nv_bfloat16*)tile, n_boards, board_rows, board_cols);
-  RZ_LAUNCH_CHECK("rz_learn_nhwc_to_tile");
-  return 0;
+  return rz_learn_nhwc_to_tile_ex(in, tile, n_boards, board_rows, board_cols, 16, stream);
 }

@@ -44,8 +44,12 @@ class AlphaZeroAgent(object):
     def __init__(self, board_size, learning_rate=0.001, weight_decay=1e-4, device='cuda',
                  net=None, mode=None, trainer=None):
         """``trainer``: 'native' (hand-written kernels: the float32 step for the reference's PolicyValueNet, the
-        tensor-core step for ResNetPolicyValueNet on square boards up to 15x15; the default where one fits) or
-        'autograd' (plain PyTorch: the checker, and any other module)."""
+        tensor-core step for ResNetPolicyValueNet on square boards up to 19x19 -- 4 input planes with H*W actions, or the
+        17 planes of GoEnv.observe with H*W + 1 actions, the pass last) or 'autograd' (plain PyTorch: the checker, and
+        any other module).  The default (None) is the native step for the reference's PolicyValueNet and for 4-plane
+        ResNets up to 15x15, and autograd for everything else, Go networks and 16x16 .. 19x19 boards included: ask for
+        'native' to train those on the tensor cores (the bf16 trunk's value error on trained networks, DESIGN section
+        3.4, is measured at 15x15 only)."""
         self.board_size = board_size
         self.policy_value_net = net if net is not None else PolicyValueNet(board_size)
         self.policy_value_net.to(device)
@@ -61,6 +65,7 @@ class AlphaZeroAgent(object):
             # well (16-mantissa-bit pairs: forward still within 1e-5, gradients within 1e-3..1e-2 of the float64 oracle
             # instead of 1e-5 -- tighter than PyTorch's default TF32 convolutions -- and 3x faster at batch 512)
             self.trainer = make_trainer(self.policy_value_net, tc_trunk=(trainer == 'native_tc'),
+                                        requested=trainer in ('native', 'native_tc'),
                                         learning_rate=learning_rate, weight_decay=weight_decay, device=device)
             if self.trainer is None and trainer in ('native', 'native_tc'):
                 raise ValueError('no native trainer fits this module (use trainer="autograd")')

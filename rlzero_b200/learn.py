@@ -414,30 +414,43 @@ class NativeTrainer(object):
 
 
 class ResNetTrainer(NativeTrainer):
-    """The same step for ``ResNetPolicyValueNet`` (stem conv3x3(4 -> 128) + ReLU, N blocks of 2 x [conv3x3 +
+    """The same step for ``ResNetPolicyValueNet`` (stem conv3x3(P -> 128) + ReLU, N blocks of 2 x [conv3x3 +
     BatchNorm2d] + skip + ReLU, the reference heads) with the trunk on the tensor cores (``csrc/rz_learn_tc.cu``):
-    bf16 activations / gradients in the padded 16-stride layout, forward convolution and data gradient through
-    ``rz_net_conv3x3_tc2``, weight gradient through the tcgen05 MN-major kernel, BatchNorm in training mode with
+    bf16 activations / gradients in the padded position layout, forward convolution and data gradient through the
+    inference path's convolution, weight gradient through the tcgen05 MN-major kernel, BatchNorm in training mode with
     float32 statistics.  Heads, loss and Adam are the float32 kernels of ``NativeTrainer`` (the trunk output crosses
-    into float32 channels-last once per step).  Square boards up to 15x15, 4 input planes."""
+    into float32 channels-last once per step).
+
+    Square boards up to 19x19 in two forms: 4 input planes (GomokuEnv.current_state) with H*W actions, or 17 planes
+    (GoEnv.observe) with H*W + 1 actions, the last one the pass.  The layout follows the board: row stride S = 16 up to
+    15x15 (``rz_net_conv3x3_tc2``, [B*256][128] tensors) and S = 20 for 16x16 to 19x19 (``rz_net_conv3x3_tc3``,
+    [round_up(B*400, 256)][128]).  The stem's forward is the inference path's fused stem fed from float32 planes
+    (``rz_net_stem_tc_planes`` / ``rz_net_stem_go_tc_planes``)."""
 
     def _check_module(self, module):
         if not (hasattr(module, 'stem') and hasattr(module, 'blocks')):
             raise ValueError('ResNetTrainer trains ResNetPolicyValueNet')
-        W = int(getattr(module, 'board_width', module.board_size))
-        if W != self.H or self.H > 15 or module.stem.in_channels != 4 or int(getattr(module, 'n_actions', self.HW)) != self.HW:
-            raise ValueError('ResNetTrainer: square Gomoku-style boards up to 15x15 with 4 input planes')
+        if not resnet_trainer_fits(module):
+            raise ValueError('ResNetTrainer: square boards up to 19x19, with 4 input planes and H*W actions or 17 input '
+                             'planes (Go) and H*W + 1 actions')
+        self.in_planes = int(module.stem.in_channels)
+        self.A = int(module.n_actions)               # policy outputs (the pass included); the heads read HW squares
+        self.AS = (self.A + 31) // 32 * 32
+        self.S = 16 if self.H <= 15 else 20          # row stride of the padded layout
         self.n_blocks = len(module.blocks)
 
     def _init_trunk(self):
         dev, bf = self.device, torch.bfloat16
-        self.w_stem = torch.empty(128 * 64, dtype=bf, device=dev)
+        self.w_stem = torch.empty(128 * (64 if self.in_planes == 4 else 192), dtype=bf, device=dev)
         n_conv = 2 * self.n_blocks
         self.wf = [torch.empty(9 * 128 * 128, dtype=bf, device=dev) for _ in range(n_conv)]
         self.wb = [torch.empty(9 * 128 * 128, dtype=bf, device=dev) for _ in range(n_conv)]
         self.stats = [torch.zeros(4 * 128, dtype=torch.float32, device=dev) for _ in range(n_conv)]
         self.dw_full = torch.zeros(128 * 128 * 9, dtype=torch.float32, device=dev)
-        self.gdesc = L.GameDesc(self.H, min(5, self.H), self.HW, self.AS, self.H, L.GAME_GOMOKU, 0.0, 0, 16)
+        if self.in_planes == 17:
+            self.gdesc = L.GameDesc(self.H, 1, self.A, self.AS, self.H, L.GAME_GO, 0.0, 0, self.S)
+        else:
+            self.gdesc = L.GameDesc(self.H, min(5, self.H), self.HW, self.AS, self.H, L.GAME_GOMOKU, 0.0, 0, self.S)
         self.conv_names = []
         for i in range(self.n_blocks):
             self.conv_names += [('blocks.%d.conv1' % i, 'blocks.%d.bn1' % i), ('blocks.%d.conv2' % i, 'blocks.%d.bn2' % i)]
@@ -447,7 +460,8 @@ class ResNetTrainer(NativeTrainer):
 
     def _repack(self):
         s = L.stream_ptr()
-        L.check(self.lib.rz_learn_pack_stem_tc(L.ptr(self._p('stem.weight')), L.ptr(self.w_stem), s), 'rz_learn_pack_stem_tc')
+        L.check(self.lib.rz_learn_pack_stem_tc_ex(L.ptr(self._p('stem.weight')), self.in_planes, L.ptr(self.w_stem), s),
+                'rz_learn_pack_stem_tc_ex')
         for j, (cn, _) in enumerate(self.conv_names):
             L.check(self.lib.rz_learn_pack_conv_tc(L.ptr(self._p(cn + '.weight')), L.ptr(self.wf[j]), L.ptr(self.wb[j]), s),
                     'rz_learn_pack_conv_tc')
@@ -457,7 +471,7 @@ class ResNetTrainer(NativeTrainer):
 
     def _alloc_trunk(self, B):
         dev, bf, HW = self.device, torch.bfloat16, self.HW
-        rows = B * 256
+        rows = (B * self.S * self.S + 255) // 256 * 256
         t = lambda: torch.zeros(rows, 128, dtype=bf, device=dev)
         n_conv = 2 * self.n_blocks
         self.act0 = t()                                  # stem output
@@ -470,79 +484,95 @@ class ResNetTrainer(NativeTrainer):
         self.planes = None
 
     def _tc_conv(self, inp, w, bias, res, out):
-        L.check(self.lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(w), L.ptr(bias), L.ptr(res), L.ptr(out), self.B, self.H, self.H,
-                                            128, 0, 2, 2, 0, L.stream_ptr()), 'rz_net_conv3x3_tc2')
+        if self.S == 16:
+            L.check(self.lib.rz_net_conv3x3_tc2(L.ptr(inp), L.ptr(w), L.ptr(bias), L.ptr(res), L.ptr(out), self.B, self.H,
+                                                self.H, 128, 0, 2, 2, 0, L.stream_ptr()), 'rz_net_conv3x3_tc2')
+        else:
+            L.check(self.lib.rz_net_conv3x3_tc3(L.ptr(inp), L.ptr(w), L.ptr(bias), L.ptr(res), L.ptr(out), self.B, self.H,
+                                                self.H, self.S, 0, 0, L.stream_ptr()), 'rz_net_conv3x3_tc3')
 
     def _trunk_forward(self, st):
-        lib, s, B, H = self.lib, L.stream_ptr(), self.B, self.H
+        lib, s, B, H, S = self.lib, L.stream_ptr(), self.B, self.H, self.S
         self.planes = st
-        L.check(lib.rz_net_stem_tc_planes(C.byref(self.gdesc), L.ptr(st), L.ptr(self.w_stem), L.ptr(self._p('stem.bias')),
-                                          L.ptr(self.act0), B, 1, 0, s), 'rz_net_stem_tc_planes')
+        stem = lib.rz_net_stem_go_tc_planes if self.in_planes == 17 else lib.rz_net_stem_tc_planes
+        L.check(stem(C.byref(self.gdesc), L.ptr(st), L.ptr(self.w_stem), L.ptr(self._p('stem.bias')), L.ptr(self.act0), B, 1,
+                     0, s), 'rz_net_stem_go_tc_planes' if self.in_planes == 17 else 'rz_net_stem_tc_planes')
         cur = self.act0
         for j, (cn, bn) in enumerate(self.conv_names):
             self._tc_conv(cur if j % 2 == 0 else self.abuf[j - 1], self.wf[j], self._p(cn + '.bias'), None, self.ybuf[j])
             m = self.bns[j]
-            L.check(lib.rz_learn_bn_forward(L.ptr(self.ybuf[j]), L.ptr(cur) if j % 2 == 1 else None, L.ptr(self.abuf[j]),
-                                            L.ptr(self._p(bn + '.weight')), L.ptr(self._p(bn + '.bias')),
-                                            L.ptr(m.running_mean), L.ptr(m.running_var), float(m.eps),
-                                            float(m.momentum if m.momentum is not None else 0.1), L.ptr(self.stats[j]),
-                                            L.ptr(self.scratch), B, H, H, s), 'rz_learn_bn_forward')
+            L.check(lib.rz_learn_bn_forward_ex(L.ptr(self.ybuf[j]), L.ptr(cur) if j % 2 == 1 else None, L.ptr(self.abuf[j]),
+                                               L.ptr(self._p(bn + '.weight')), L.ptr(self._p(bn + '.bias')),
+                                               L.ptr(m.running_mean), L.ptr(m.running_var), float(m.eps),
+                                               float(m.momentum if m.momentum is not None else 0.1), L.ptr(self.stats[j]),
+                                               L.ptr(self.scratch), B, H, H, S, s), 'rz_learn_bn_forward_ex')
             if j % 2 == 1:
                 cur = self.abuf[j]
                 m.num_batches_tracked += 1
             else:
                 m.num_batches_tracked += 1
         self.trunk_out = cur
-        L.check(lib.rz_learn_tile_to_nhwc(L.ptr(cur), L.ptr(self.a_last), B, H, H, s), 'rz_learn_tile_to_nhwc')
+        L.check(lib.rz_learn_tile_to_nhwc_ex(L.ptr(cur), L.ptr(self.a_last), B, H, H, S, s), 'rz_learn_tile_to_nhwc_ex')
 
     def _trunk_backward(self):
-        lib, s, B, H = self.lib, L.stream_ptr(), self.B, self.H
+        lib, s, B, H, S = self.lib, L.stream_ptr(), self.B, self.H, self.S
         g, dy, dz, da = self.gbuf
-        L.check(lib.rz_learn_nhwc_to_tile(L.ptr(self.d_last), L.ptr(g), B, H, H, s), 'rz_learn_nhwc_to_tile')
+        L.check(lib.rz_learn_nhwc_to_tile_ex(L.ptr(self.d_last), L.ptr(g), B, H, H, S, s), 'rz_learn_nhwc_to_tile_ex')
         scr, nscr = L.ptr(self.scratch), self.scratch.numel()
         for i in reversed(range(self.n_blocks)):
             j1, j2 = 2 * i, 2 * i + 1
             block_in = self.act0 if i == 0 else self.abuf[j1 - 1]
             (c1, b1), (c2, b2) = self.conv_names[j1], self.conv_names[j2]
             # second half of the block: BatchNorm2 + skip + ReLU, conv2
-            L.check(lib.rz_learn_bn_backward(L.ptr(g), L.ptr(self.abuf[j2]), L.ptr(self.ybuf[j2]), L.ptr(self.stats[j2]),
-                                             L.ptr(self._g(b2 + '.weight')), L.ptr(self._g(b2 + '.bias')), L.ptr(dy), L.ptr(dz),
-                                             scr, B, H, H, s), 'rz_learn_bn_backward')
-            L.check(lib.rz_learn_conv_wgrad_tc(L.ptr(self.abuf[j1]), L.ptr(dy), L.ptr(self._g(c2 + '.weight')), scr, nscr, B, 0, s),
-                    'rz_learn_conv_wgrad_tc')
+            L.check(lib.rz_learn_bn_backward_ex(L.ptr(g), L.ptr(self.abuf[j2]), L.ptr(self.ybuf[j2]), L.ptr(self.stats[j2]),
+                                                L.ptr(self._g(b2 + '.weight')), L.ptr(self._g(b2 + '.bias')), L.ptr(dy),
+                                                L.ptr(dz), scr, B, H, H, S, s), 'rz_learn_bn_backward_ex')
+            L.check(lib.rz_learn_conv_wgrad_tc_ex(L.ptr(self.abuf[j1]), L.ptr(dy), L.ptr(self._g(c2 + '.weight')), scr, nscr, B,
+                                                  S, 0, s), 'rz_learn_conv_wgrad_tc_ex')
             self._tc_conv(dy, self.wb[j2], self.zero_bias, None, da)
             # first half: BatchNorm1 + ReLU, conv1; the skip gradient dz joins the data gradient
-            L.check(lib.rz_learn_bn_backward(L.ptr(da), L.ptr(self.abuf[j1]), L.ptr(self.ybuf[j1]), L.ptr(self.stats[j1]),
-                                             L.ptr(self._g(b1 + '.weight')), L.ptr(self._g(b1 + '.bias')), L.ptr(dy), None,
-                                             scr, B, H, H, s), 'rz_learn_bn_backward')
-            L.check(lib.rz_learn_conv_wgrad_tc(L.ptr(block_in), L.ptr(dy), L.ptr(self._g(c1 + '.weight')), scr, nscr, B, 0, s),
-                    'rz_learn_conv_wgrad_tc')
+            L.check(lib.rz_learn_bn_backward_ex(L.ptr(da), L.ptr(self.abuf[j1]), L.ptr(self.ybuf[j1]), L.ptr(self.stats[j1]),
+                                                L.ptr(self._g(b1 + '.weight')), L.ptr(self._g(b1 + '.bias')), L.ptr(dy), None,
+                                                scr, B, H, H, S, s), 'rz_learn_bn_backward_ex')
+            L.check(lib.rz_learn_conv_wgrad_tc_ex(L.ptr(block_in), L.ptr(dy), L.ptr(self._g(c1 + '.weight')), scr, nscr, B, S,
+                                                  0, s), 'rz_learn_conv_wgrad_tc_ex')
             self._tc_conv(dy, self.wb[j1], self.zero_bias, dz, g)
             # a convolution bias in front of a BatchNorm has no gradient (the batch mean absorbs it)
             self._g(c1 + '.bias').zero_()
             self._g(c2 + '.bias').zero_()
         # stem: ReLU mask on the tile; its weight gradient through the same tensor-core kernel with the observation
-        # planes as channels 0..3 of a tile (0/1 values: exact), its bias gradient = the column sums of dz
-        L.check(lib.rz_learn_relu_bwd_bf16(L.ptr(g), L.ptr(self.act0), L.ptr(dy), B, s), 'rz_learn_relu_bwd_bf16')
-        L.check(lib.rz_learn_planes_to_tile(L.ptr(self.planes), L.ptr(da), B, H, H, s), 'rz_learn_planes_to_tile')
-        L.check(lib.rz_learn_conv_wgrad_tc(L.ptr(da), L.ptr(dy), L.ptr(self.dw_full), scr, nscr, B, 0, s),
-                'rz_learn_conv_wgrad_tc')
-        self._g('stem.weight').view(128, 4, 9).copy_(self.dw_full.view(128, 128, 9)[:, :4, :])
-        L.check(lib.rz_learn_tile_colsum(L.ptr(dy), L.ptr(self._g('stem.bias')), scr, B, s), 'rz_learn_tile_colsum')
+        # planes as channels 0..P-1 of a tile (0/1 values: exact), its bias gradient = the column sums of dz
+        P = self.in_planes
+        L.check(lib.rz_learn_relu_bwd_bf16_ex(L.ptr(g), L.ptr(self.act0), L.ptr(dy), B, S, s), 'rz_learn_relu_bwd_bf16_ex')
+        L.check(lib.rz_learn_planes_to_tile_ex(L.ptr(self.planes), P, L.ptr(da), B, H, H, S, s), 'rz_learn_planes_to_tile_ex')
+        L.check(lib.rz_learn_conv_wgrad_tc_ex(L.ptr(da), L.ptr(dy), L.ptr(self.dw_full), scr, nscr, B, S, 0, s),
+                'rz_learn_conv_wgrad_tc_ex')
+        self._g('stem.weight').view(128, P, 9).copy_(self.dw_full.view(128, 128, 9)[:, :P, :])
+        L.check(lib.rz_learn_tile_colsum_ex(L.ptr(dy), L.ptr(self._g('stem.bias')), scr, B, S, s), 'rz_learn_tile_colsum_ex')
 
 
-def make_trainer(module, tc_trunk=False, **kw):
+def resnet_trainer_fits(module):
+    """Whether ``ResNetTrainer`` trains ``module``: square boards up to 19x19, 4 planes with H*W actions or 17 (Go) with
+    H*W + 1."""
+    H = int(module.board_size)
+    W = int(getattr(module, 'board_width', H))
+    P, A = int(module.stem.in_channels), int(module.n_actions)
+    return W == H and H <= 19 and ((P == 4 and A == H * H) or (P == 17 and A == H * H + 1))
+
+
+def make_trainer(module, tc_trunk=False, requested=False, **kw):
     """The native trainer that fits ``module``, or None (the caller then falls back to its autograd path).
-    ``tc_trunk``: the reference's own network with the whole trunk on the tensor cores (``NativeTrainer.use_tc_trunk``)."""
+    ``tc_trunk``: the reference's own network with the whole trunk on the tensor cores (``NativeTrainer.use_tc_trunk``).
+    ``requested``: the caller asked for a native trainer.  Without it only the shapes that have trained natively by
+    default all along get one (4 planes, boards up to 15x15); Go networks and 16x16 .. 19x19 boards stay on autograd
+    unless asked, because the bf16 trunk's value error on trained networks (DESIGN section 3.4) is not measured there."""
     from .games.gomoku.policy_value_net import PolicyValueNet, ResNetPolicyValueNet
     if type(module) is PolicyValueNet:
         t = NativeTrainer(module, **kw)
         t.use_tc_trunk = bool(tc_trunk)
         t._repack()
         return t
-    if isinstance(module, ResNetPolicyValueNet):
-        W = int(getattr(module, 'board_width', module.board_size))
-        if (W == module.board_size and module.board_size <= 15 and module.stem.in_channels == 4
-                and int(module.n_actions) == module.board_size ** 2):
+    if isinstance(module, ResNetPolicyValueNet) and resnet_trainer_fits(module):
+        if requested or (module.board_size <= 15 and module.stem.in_channels == 4):
             return ResNetTrainer(module, **kw)
     return None
