@@ -39,7 +39,7 @@
 extern "C" {
 #endif
 
-#define RZ_ABI_VERSION 13
+#define RZ_ABI_VERSION 14
 #define RZ_MAX_BOARD 19          /* rows live one per lane; A <= 362 (19x19 Go incl. the pass) */
 #define RZ_META_STRIDE 12
 #define RZ_GO_HIST 14            /* history planes a Go position carries besides the current board */
@@ -608,6 +608,17 @@ int rz_net_trunk_small_ex(const void* act_in, const void* weights, const float* 
                           unsigned relu_mask, unsigned res_mask, unsigned n64_mask, unsigned split_in_mask, int head_f32,
                           int n_boards, int board_size, int board_cols, const float* w1x1_host,
                           const float* b1x1_host, float* feat, void* stream);
+/* the same trunk for many boards (rz_net_trunk_tc2.cu): one launch on n_ctas / 2 CTA pairs (0 = 148 CTAs), pair p
+   carrying a contiguous range of boards in chunks of at most `chunk` (1..16) boards through every layer, the activations
+   between layers in `scratch` instead of act_in-sized tensors: bf16 [2][n_ctas / 2][chunk][256][128] (1 MB per pair at
+   chunk 8; it must start zeroed, and the kernel keeps its pad rows zero).  act_in, weights, relu_mask, res_mask and
+   feat as rz_net_trunk_small; biases_host f32 [n_layers][128] in host memory, copied into the launch parameters like
+   w1x1_host.  Per board the MMAs and the epilogue arithmetic are those of rz_net_conv3x3_tc2[_head_ex], so the results
+   are bit-identical to the per-layer launches and to rz_net_trunk_small.  Weights are STATIC as in flag 512 above. */
+int rz_net_trunk_tc2(const void* act_in, const void* weights, const float* biases_host, int n_layers,
+                     unsigned relu_mask, unsigned res_mask, void* scratch, int chunk, int n_boards, int board_size,
+                     int board_cols, const float* w1x1_host, const float* b1x1_host, float* feat, int n_ctas,
+                     void* stream);
 /* profiling aid: rz_net_trunk_small writes four %globaltimer stamps per layer of board 0 (inputs ready / MMAs issued /
    accumulator complete / layer stored) into this device buffer of 4 * n_layers uint64; NULL (the default) = off. */
 int rz_debug_set_probe(void* device_buffer);

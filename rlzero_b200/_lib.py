@@ -11,7 +11,7 @@ import torch  # noqa: F401  -- loads libcudart.so.12 into the process before our
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, 'librlzero_b200.so')
 
-ABI_VERSION = 13
+ABI_VERSION = 14
 META_STRIDE = 12
 (META_PLAYER, META_LAST_MOVE, META_STONES, META_STATUS, META_WINNER, META_PLY, META_FAULT,
  META_EPISODE, META_KO, META_PASSES) = range(10)
@@ -175,6 +175,8 @@ SIGNATURES = {
                                          C.c_int, C.c_int, _vp, _vp, _vp, _vp]),
     'rz_net_trunk_small': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_uint, C.c_uint, C.c_int, C.c_int, C.c_int, _vp, _vp, _vp,
                                       _vp]),
+    'rz_net_trunk_tc2': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_uint, C.c_uint, _vp, C.c_int, C.c_int, C.c_int, C.c_int,
+                                   _vp, _vp, _vp, C.c_int, _vp]),
     'rz_net_conv3x3_tc2_head_ex': (C.c_int, [_vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                              _vp, _vp, _vp, C.c_int, _vp]),
     'rz_net_conv3x3_tc3': (C.c_int, [_vp, _vp, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,

@@ -215,6 +215,16 @@ class NativeForward(object):
         # boards up to which the one-launch trunk of rz_net_trunk_small.cu is used (one CTA pair per board, 74 pairs at a
         # time on 148 SMs; measured crossover with the per-layer kernels near 200 boards, profiles/r2_run43_crossover.log)
         self.small_batch_max = 148
+        # boards from which the batched trunk runs in one launch (rz_net_trunk_tc2.cu: CTA pairs carry chunks of
+        # `trunk_chunk` boards through every layer, the activations in an L2-sized scratch); below it, one launch per
+        # layer.  The batched trunk is the faster one at every measured count from 300 boards up (ResNet-10 15x15: 22 %
+        # at 300, 4.6 % at 8192, profiles/r3_run1_trunk_probe.jsonl), so it starts right above the 300-board batch that
+        # keeps the per-layer kernels as the reference the small-batch path is checked against.  Chunks of 6 boards
+        # (55 MB of scratch on 74 pairs) measured fastest at 8192 boards among 4..16.  Set batched_trunk_min on an
+        # instance to a larger count to force the per-layer kernels.
+        self.batched_trunk_min = 301
+        self.trunk_chunk = 6
+        self.scratch = None
         # flags of the 128 -> 128 rz_net_conv3x3_tc2 launches, read by bench.py too: 512 = static weights
         # (include/rlzero_b200.h); bit 1 (2) is accepted and ignored
         self.conv_flags = 514
@@ -284,7 +294,8 @@ class NativeForward(object):
                 l['w'], l['b'] = wst[i], bst[i]
                 relu_mask |= int(bool(l['relu'])) << i
                 res_mask |= int(l['skip'] is not None) << i
-            self.trunk_small = dict(w=wst, b=bst, n=len(tail), relu_mask=relu_mask, res_mask=res_mask)
+            self.trunk_small = dict(w=wst, b=bst, n=len(tail), relu_mask=relu_mask, res_mask=res_mask,
+                                    b_host=np.ascontiguousarray(bst.float().cpu().numpy().reshape(-1)))
         # fused encoder + stem (rz_net_stem.cu): weight [cout][k = tap*4 + plane], k padded to 64
         conv0 = m.trunk_layers()[0][0]
         if self.mode != 'tc32':
@@ -398,6 +409,10 @@ class NativeForward(object):
                             skip=None, relu=bool(r3))]
 
     def _alloc(self, n):
+        if self._route(n) == 'batched' and self.scratch is None:
+            # [2][pairs][chunk][256][128] bf16, zeroed: the batched trunk keeps its pad rows zero
+            pairs = (self.n_ctas or 148) // 2
+            self.scratch = torch.zeros(2 * pairs * self.trunk_chunk * 256, 128, dtype=torch.bfloat16, device=self.device)
         if n <= self.max_batch:
             return
         dev = self.device
@@ -432,12 +447,19 @@ class NativeForward(object):
                              "or Go's 17 planes")
         return self.stem
 
-    def _one_launch(self, n):
-        """Whether ``n`` boards run the trunk behind the stem in one launch (rz_net_trunk_small.cu) instead of one
-        launch per layer: few boards (a sequential search evaluates ONE), a layout the one-launch kernel takes, and in
-        mode 'tc' the fused heads epilogue, which that kernel always applies."""
-        return (self.trunk_small is not None and n <= self.small_batch_max
-                and (self.mode == 'tc32' or self.fused_head))
+    def _route(self, n):
+        """How ``n`` boards run the trunk behind the stem: 'small' = one launch, one CTA pair per board
+        (rz_net_trunk_small.cu: few boards, a sequential search evaluates ONE); 'batched' = one launch, CTA pairs carrying
+        chunks of boards through every layer (rz_net_trunk_tc2.cu: a search wave's thousands of leaves); 'layers' = one
+        launch per layer.  Both one-launch kernels need a layout they take and, in mode 'tc', the fused heads epilogue,
+        which they always apply.  kernels_per_forward reads the same answer."""
+        if self.trunk_small is None or not (self.mode == 'tc32' or self.fused_head):
+            return 'layers'
+        if n <= self.small_batch_max:
+            return 'small'
+        if self.mode == 'tc' and n >= self.batched_trunk_min:
+            return 'batched'
+        return 'layers'
 
     def _conv(self, layer, inp, res, out, n):
         """One 128 -> 128 trunk layer on the tensor cores.  The layer layout picks the kernel: rz_net_tc2.cu for
@@ -489,7 +511,8 @@ class NativeForward(object):
         # the tensor-core modes: trunk behind the stem (which wrote bufs[0]) -> head features in self.feat -> FC heads
         w1p = self.w1x1_host.ctypes.data_as(C.c_void_p)
         b1p = self.b1x1_host.ctypes.data_as(C.c_void_p)
-        if self._one_launch(n):
+        route = self._route(n)
+        if route == 'small':
             # the whole trunk in one launch, one CTA pair per board (tc32: conv2 + conv3 + the 1x1 heads)
             ts = self.trunk_small
             if self.mode == 'tc32':
@@ -501,6 +524,12 @@ class NativeForward(object):
                 L.check(lib.rz_net_trunk_small(
                     L.ptr(self.bufs[0]), L.ptr(ts['w']), L.ptr(ts['b']), ts['n'], ts['relu_mask'], ts['res_mask'], n,
                     self.H, self.W, w1p, b1p, L.ptr(self.feat), s), 'rz_net_trunk_small')
+        elif route == 'batched':
+            ts = self.trunk_small
+            L.check(lib.rz_net_trunk_tc2(
+                L.ptr(self.bufs[0]), L.ptr(ts['w']), ts['b_host'].ctypes.data_as(C.c_void_p), ts['n'], ts['relu_mask'],
+                ts['res_mask'], L.ptr(self.scratch), self.trunk_chunk, n, self.H, self.W, w1p, b1p, L.ptr(self.feat),
+                self.n_ctas, s), 'rz_net_trunk_tc2')
         elif self.mode == 'tc32':
             # conv2 (one K = 128 pass, split output) and conv3 (three products per tap, fp32 features)
             l2, l3 = self.layers[1], self.layers[2]
@@ -530,7 +559,7 @@ class NativeForward(object):
 
     def kernels_per_forward(self, n=None):
         """Kernel launches of one forward_boards call of ``n`` boards (for bench.py's gpu_launches)."""
-        if n is not None and self._one_launch(n):
+        if n is not None and self._route(n) != 'layers':
             return 3                                        # stem, one-launch trunk + 1x1 heads, FC heads
         if self.mode == 'tc32':
             return 4                                        # stem, conv2, conv3 + 1x1 heads, FC heads
