@@ -366,9 +366,28 @@ int rz_eval_closed_form(const rz_tree_desc* t, int eval_id, float* prior, float*
    get_equi_data: the 8 symmetric copies of n recorded plies, in the reference's order (for i in
    1..4: rot90^i, then its fliplr).  rows [n][2][H], info [n][info_stride] int32 (mover, last_move, z,
    ...: the trajectory ring's records), pi f32 [n][AS]  ->  out_planes f32 [8n][4][H][W] (current_state
-   of the transformed position), out_pi f32 [8n][A], out_z f32 [8n]. */
+   of the transformed position), out_pi f32 [8n][A], out_z f32 [8n].  Square Gomoku boards only: any other
+   game_type or width is rejected on the host (Go records go through rz_go_records_pack / _expand). */
 int rz_augment_equi(const rz_game_desc* g, const uint32_t* rows, const int32_t* info, int info_stride,
                     const float* pi, float* out_planes, float* out_pi, float* out_z, int n, void* stream);
+/* Go training records (g: an RZ_GAME_GO descriptor, A = H*H + 1, AS = action_stride).  n trajectory-ring records in
+   drain order -- rows [n][2][H], info [n][info_stride >= 6] int32 (mover, last_move, z, slot, episode, ply), pi f32
+   [n][AS] -- are packed into a caller-owned ring of `capacity` compact records: planes uint32 [capacity][16][H] (the
+   first 16 GoEnv.observe planes as row bitmasks: entry e = 0..7 is the position e plies back as (stones of its previous
+   mover, stones of its mover), rebuilt from the preceding records of the same slot and episode, zero where there is
+   none -- BatchedSelfPlay._go_states), mover int32 [capacity], pi f32 [capacity][A], z f32 [capacity].  Record i goes
+   to slot (dst_start + i) % capacity; every input record serves as history, but with n > capacity only the newest
+   capacity are written.  2672 bytes per position at 19x19. */
+int rz_go_records_pack(const rz_game_desc* g, const uint32_t* rows, const int32_t* info, int info_stride,
+                       const float* pi, int n, uint32_t* planes, int32_t* mover, float* out_pi, float* z, int capacity,
+                       int dst_start, void* stream);
+/* n (slot, symmetry) pairs of such a ring -> out_states f32 [n][17][H][H] (plane 16 = mover == 1, GoEnv.observe),
+   out_pi f32 [n][A], out_z f32 [n]: what AlphaZeroAgent.learn takes.  Symmetry s: rot90 (s / 2 + 1) times, then fliplr
+   when s is odd (rz_augment_equi's plane maps; s = 6 is the identity), applied to the planes AND to the H*H square
+   probabilities; the pass is unchanged.  slots / syms are device int64; only slot % capacity and sym & 7 are read. */
+int rz_go_records_expand(const rz_game_desc* g, const uint32_t* planes, const int32_t* mover, const float* pi,
+                         const float* z, int capacity, const long long* slots, const long long* syms, int n,
+                         float* out_states, float* out_pi, float* out_z, void* stream);
 /* dst[i][:] = src[index[i]][:] for a [.][width] float table: mini-batch gather from the replay buffer
    (random.sample(self.data_buffer, batch_size), tools/train_alphazero.py:94). */
 int rz_gather_rows(const float* src, const long long* index, float* dst, int n, int width, void* stream);

@@ -119,6 +119,8 @@ SIGNATURES = {
     'rz_eval_closed_form': (C.c_int, [_TD, C.c_int, _vp, _vp, _vp]),
     'rz_augment_equi': (C.c_int, [_GD, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int, _vp]),
     'rz_gather_rows': (C.c_int, [_vp, _vp, _vp, C.c_int, C.c_int, _vp]),
+    'rz_go_records_pack': (C.c_int, [_GD, _vp, _vp, C.c_int, _vp, C.c_int, _vp, _vp, _vp, _vp, C.c_int, C.c_int, _vp]),
+    'rz_go_records_expand': (C.c_int, [_GD, _vp, _vp, _vp, _vp, C.c_int, _vp, _vp, C.c_int, _vp, _vp, _vp, _vp]),
     'rz_learn_sgemm': (C.c_int, [C.c_int, C.c_int, C.c_int, _vp, C.c_longlong, C.c_longlong, _vp, C.c_longlong,
                                  C.c_longlong, _vp, C.c_longlong, C.c_float, C.c_int, _vp]),
     'rz_learn_colsum': (C.c_int, [_vp, C.c_longlong, C.c_int, C.c_longlong, _vp, C.c_float, _vp, C.c_int, _vp]),

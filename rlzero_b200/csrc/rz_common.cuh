@@ -75,6 +75,13 @@ static inline int rz_check_game(const rz_game_desc* g) {
   return 0;
 }
 
+// rz_check_game, and the descriptor must be Go (entry points that only know Go's layout)
+static inline int rz_check_go(const rz_game_desc* g, const char* who) {
+  if (rz_check_game(g)) return -1;
+  RZ_REQUIRE(g->game_type == RZ_GAME_GO, "%s: game_type %d is not RZ_GAME_GO", who, g->game_type);
+  return 0;
+}
+
 // Row stride S of the padded position layout of the tensor-core network path (a board owns S*S rows of
 // [128 channels] bf16, square (y, x) at row y*S + x, squares with x >= W or y >= H hold zero): the smallest of
 // 8 / 16 / 20 that leaves one zero column and one zero row, or the caller's explicit choice.  Returns 0 when

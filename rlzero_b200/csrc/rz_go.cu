@@ -136,11 +136,6 @@ rz_go_encode_f32_kernel(rz_game_desc gd, const uint32_t* rows, const uint32_t* h
 // ---------------------------------------------------------------------------
 // C ABI
 // ---------------------------------------------------------------------------
-static int rz_check_go(const rz_game_desc* g, const char* who) {
-  if (rz_check_game(g)) return -1;
-  RZ_REQUIRE(g->game_type == RZ_GAME_GO, "%s: game_type %d is not RZ_GAME_GO", who, g->game_type);
-  return 0;
-}
 static inline dim3 rz_go_grid(int n) { return dim3((unsigned)((n + RZ_GO_WARPS - 1) / RZ_GO_WARPS)); }
 
 extern "C" int rz_go_reset(const rz_game_desc* g, uint32_t* rows, uint32_t* hist, int32_t* meta, int n_games,

@@ -10,7 +10,8 @@ The only exchanges are off the hot path, once per generation / training step:
 * ``gather_records_device`` -- the finished plies of every rank as COMPACT device records (the
   trajectory ring's own format: two row-bitboards, 6 info words, pi -- 1.2 KB per ply at 15x15
   against 4.5 KB for float32 planes + pi), one NCCL all-gather on device tensors, no host hop for
-  the payload; the 8-fold augmentation (``rz_augment_equi``) then expands them on the receiving GPU;
+  the payload; the 8-fold augmentation (``rz_augment_equi``; Go: ``GoReplayBuffer``) then expands them on the
+  receiving GPU;
 * ``broadcast_weights``     -- after ``AlphaZeroAgent.learn`` on the learner rank the parameters and
   buffers of the policy-value module go to every rank in one flat buffer per dtype, which then
   re-packs them for the kernels (``refresh_weights``; the captured wave graph is re-captured);
@@ -146,8 +147,14 @@ def generation_step(selfplay, agent, n_moves=1, batch_size=512, epochs=1, learne
     """One generation of the multi-GPU loop: every rank plays ``n_moves`` moves of its games, the finished plies
     are all-gathered as compact device records, the learner rank augments them (8 symmetries, rz_augment_equi) and
     runs ``epochs`` ``AlphaZeroAgent.learn`` steps on mini-batches of them, the new weights are broadcast and every
-    rank re-packs them (its captured wave graph is re-captured on the next wave).  Returns a dict of counters."""
-    from .train_pipeline import augment_equi_device
+    rank re-packs them (its captured wave graph is re-captured on the next wave).  Returns a dict of counters.
+
+    Go: the learner packs the records into a ``GoReplayBuffer`` of this generation (17 planes, the history rebuilt
+    from the preceding plies of each episode) and every epoch expands ``batch_size`` distinct (record, symmetry)
+    pairs of the 8n.  The gathered records keep each rank's drain order, and column 3 of ``info`` holds global game
+    ids, so an episode's plies stay contiguous and distinct from other ranks' episodes: the history is rebuilt across
+    ranks as on one."""
+    from .train_pipeline import GoReplayBuffer, augment_equi_device
     f = selfplay.forest
     selfplay.play(n_moves)
     rec = f.drain_trajectories_device()
@@ -155,7 +162,15 @@ def generation_step(selfplay, agent, n_moves=1, batch_size=512, epochs=1, learne
                                                    global_offset=int(f.desc.global_offset), group=group)
     loss = None
     n = int(info.shape[0])
-    if dist.get_rank(group) == learner and n > 0:
+    if dist.get_rank(group) == learner and n > 0 and f.is_go:
+        buf = GoReplayBuffer(n, f.H, device=rows.device)
+        buf.extend(rows, info, pi)
+        g = torch.Generator(device='cpu')
+        g.manual_seed(n)
+        for _ in range(epochs):
+            k = torch.randperm(8 * n, generator=g)[:batch_size].to(rows.device)
+            loss, _ = agent.learn(*buf.expand(k // 8, k % 8))
+    elif dist.get_rank(group) == learner and n > 0:
         if augment:
             states, pis, zs = augment_equi_device(f.gdesc, rows, info, pi)
         else:

@@ -85,6 +85,86 @@ class DeviceReplayBuffer(object):
         return out_s.reshape(n, 4, self.H, self.H), out_p, out_z.reshape(n)
 
 
+class GoReplayBuffer(object):
+    """Replay buffer of Go self-play positions on the device, kept compact: per position the first 16 GoEnv.observe
+    planes as row bitmasks (the history is rebuilt from the trajectory ring's records when they are packed, as
+    ``BatchedSelfPlay._go_states`` does on the host), the mover, pi [A] and z -- 2672 bytes at 19x19 against 208 000
+    for the 8 augmented float32 copies ``DeviceReplayBuffer`` would hold.  The 8 board symmetries are applied when a
+    mini-batch is expanded (``rz_go_records_expand``).  Logical index 0 is the oldest record."""
+
+    def __init__(self, capacity, board_size, device='cuda'):
+        if not torch.cuda.is_available():
+            raise L.NativeLibraryError('GoReplayBuffer needs a CUDA device (no CPU fallback)')
+        self.lib = L.load()
+        self.capacity = int(capacity)
+        if self.capacity < 1:
+            raise ValueError('capacity must be at least 1')
+        self.H = int(board_size)
+        self.A = self.H * self.H + 1
+        self.gdesc = L.GameDesc(self.H, 1, self.A, (self.A + 31) // 32 * 32, self.H, L.GAME_GO, 0.0, 0)
+        self.device = torch.device(device)
+        self.planes = torch.zeros(self.capacity, 16, self.H, dtype=torch.int32, device=self.device)
+        self.mover = torch.zeros(self.capacity, dtype=torch.int32, device=self.device)
+        self.pis = torch.zeros(self.capacity, self.A, dtype=torch.float32, device=self.device)
+        self.zs = torch.zeros(self.capacity, dtype=torch.float32, device=self.device)
+        self.start = 0      # physical slot of logical index 0
+        self.size = 0
+
+    def __len__(self):
+        return self.size
+
+    def bytes_per_position(self):
+        return 16 * self.H * 4 + 4 + self.A * 4 + 4
+
+    def extend(self, rows, info, pi):
+        """Append n trajectory-ring records in drain order (``SearchForest.drain_trajectories_device`` or
+        ``parallel.gather_records_device``: rows int32 [n,2,H], info int32 [n,6], pi float32 [n,AS]); the oldest
+        records fall out.  The history of a record comes from the records of this call only, so pass whole drains."""
+        n = int(info.shape[0])
+        if n == 0:
+            return
+        if tuple(rows.shape[1:]) != (2, self.H) or int(pi.shape[1]) != self.gdesc.action_stride:
+            raise ValueError('ring records of a %dx%d Go board expected (rows [n,2,%d], pi [n,%d])' % (
+                self.H, self.H, self.H, self.gdesc.action_stride))
+        rows, info, pi = rows.contiguous(), info.contiguous(), pi.contiguous()
+        end = (self.start + self.size) % self.capacity
+        L.check(self.lib.rz_go_records_pack(C.byref(self.gdesc), L.ptr(rows), L.ptr(info), int(info.shape[1]),
+                                            L.ptr(pi), n, L.ptr(self.planes), L.ptr(self.mover), L.ptr(self.pis),
+                                            L.ptr(self.zs), self.capacity, end, L.stream_ptr()), 'rz_go_records_pack')
+        size = min(self.capacity, self.size + n)
+        self.start = (self.start + self.size + n - size) % self.capacity
+        self.size = size
+
+    def expand(self, logical_idx, sym):
+        """Records ``logical_idx`` (in [0, len)) under symmetries ``sym`` (in [0, 8); device or host integer sequences
+        of one length) -> (states [B,17,H,H], pis [B,A], zs [B]) float32 device tensors.  Symmetry s: ``np.rot90`` (s // 2 + 1) times,
+        then ``np.fliplr`` when s is odd (6 is the identity), on the planes and on the H*H square probabilities."""
+        idx = torch.as_tensor(logical_idx, dtype=torch.int64, device=self.device).reshape(-1)
+        sym = torch.as_tensor(sym, dtype=torch.int64, device=self.device).reshape(-1)
+        if idx.shape != sym.shape:
+            raise ValueError('logical_idx and sym differ in length')
+        B = int(idx.shape[0])
+        slots = (idx + self.start) % self.capacity
+        out_s = torch.empty(B, 17, self.H, self.H, dtype=torch.float32, device=self.device)
+        out_p = torch.empty(B, self.A, dtype=torch.float32, device=self.device)
+        out_z = torch.empty(B, dtype=torch.float32, device=self.device)
+        L.check(self.lib.rz_go_records_expand(C.byref(self.gdesc), L.ptr(self.planes), L.ptr(self.mover),
+                                              L.ptr(self.pis), L.ptr(self.zs), self.capacity, L.ptr(slots), L.ptr(sym),
+                                              B, L.ptr(out_s), L.ptr(out_p), L.ptr(out_z), L.stream_ptr()),
+                'rz_go_records_expand')
+        return out_s, out_p, out_z
+
+    def sample(self, batch_size, generator=None):
+        """``batch_size`` distinct (record, symmetry) pairs out of the 8 * len: ``random.sample`` over the 8-fold
+        augmented buffer, drawn with ``torch.randperm`` on the device (``generator``: a CUDA generator, or None)."""
+        batch_size = int(batch_size)
+        total = 8 * self.size
+        if batch_size < 0 or batch_size > total:
+            raise ValueError('sample larger than population or is negative')
+        k = torch.randperm(total, generator=generator, device=self.device)[:batch_size]
+        return self.expand(k // 8, k % 8)
+
+
 def augment_equi_device(forest_or_desc, rows, info, pi):
     """Device ``get_equi_data`` (tools/train_alphazero.py:59-79) for n trajectory records:
     rows int32 [n,2,H], info int32 [n,6] (mover, last_move, z, ...), pi float32 [n,AS] ->
