@@ -42,30 +42,54 @@ def _conv3x3_backward(x, w, dy):
     return dxp[:, :, 1:-1, 1:-1], dw, dy.sum(axis=(0, 2, 3))
 
 
-def forward(p, x):
-    """The stock network (policy_value_net.py:34-52).  Returns (log_p [B,HW], v [B,1], cache of activations)."""
+_MASKED = ('a1', 'a2', 'a3', 'pa', 'va', 'h')
+
+
+def _relu(z, masks, name):
+    """max(z, 0), or z times the fixed 0/1 mask ``masks[name]`` (a ReLU pinned to given masks)."""
+    if masks is None:
+        return np.maximum(z, 0.0)
+    m = np.asarray(masks[name], dtype=bool)
+    if m.shape != z.shape:
+        raise ValueError('mask %s has shape %s, the activation %s' % (name, m.shape, z.shape))
+    return z * m
+
+
+def forward(p, x, masks=None):
+    """The stock network (policy_value_net.py:34-52).  Returns (log_p [B,HW], v [B,1], cache of activations).
+
+    ``masks``: None, or {'a1', 'a2', 'a3', 'pa', 'va', 'h': boolean arrays in the shapes of those activations}; each
+    ReLU then multiplies by its mask instead of testing the sign (and ``loss_and_grads`` back-propagates through the same
+    masks).  With the masks a device produced, the float64 result differs from the device's only by rounding: a
+    pre-activation within rounding of zero cannot land on the other side of the ReLU than on the device."""
     B = x.shape[0]
-    a1 = np.maximum(_conv3x3(x, p['conv1.weight'], p['conv1.bias']), 0.0)
-    a2 = np.maximum(_conv3x3(a1, p['conv2.weight'], p['conv2.bias']), 0.0)
-    a3 = np.maximum(_conv3x3(a2, p['conv3.weight'], p['conv3.bias']), 0.0)
-    pa = np.maximum(np.einsum('bchw,oc->bohw', a3, p['act_conv1.weight'][:, :, 0, 0])
-                    + p['act_conv1.bias'][None, :, None, None], 0.0)
+    a1 = _relu(_conv3x3(x, p['conv1.weight'], p['conv1.bias']), masks, 'a1')
+    a2 = _relu(_conv3x3(a1, p['conv2.weight'], p['conv2.bias']), masks, 'a2')
+    a3 = _relu(_conv3x3(a2, p['conv3.weight'], p['conv3.bias']), masks, 'a3')
+    pa = _relu(np.einsum('bchw,oc->bohw', a3, p['act_conv1.weight'][:, :, 0, 0])
+               + p['act_conv1.bias'][None, :, None, None], masks, 'pa')
     pf = pa.reshape(B, -1)                                   # x.view(-1, 4*H*W): channel-major flatten
     logits = pf @ p['act_fc1.weight'].T + p['act_fc1.bias']
     m = logits.max(axis=1, keepdims=True)
     log_p = logits - m - np.log(np.exp(logits - m).sum(axis=1, keepdims=True))
-    va = np.maximum(np.einsum('bchw,oc->bohw', a3, p['val_conv1.weight'][:, :, 0, 0])
-                    + p['val_conv1.bias'][None, :, None, None], 0.0)
+    va = _relu(np.einsum('bchw,oc->bohw', a3, p['val_conv1.weight'][:, :, 0, 0])
+               + p['val_conv1.bias'][None, :, None, None], masks, 'va')
     vf = va.reshape(B, -1)
-    h = np.maximum(vf @ p['val_fc1.weight'].T + p['val_fc1.bias'], 0.0)
+    h = _relu(vf @ p['val_fc1.weight'].T + p['val_fc1.bias'], masks, 'h')
     v = np.tanh(h @ p['val_fc2.weight'].T + p['val_fc2.bias'])
-    return log_p, v, dict(x=x, a1=a1, a2=a2, a3=a3, pa=pa, pf=pf, va=va, vf=vf, h=h, v=v, log_p=log_p)
+    if masks is None:
+        relu_masks = dict(a1=a1 > 0, a2=a2 > 0, a3=a3 > 0, pa=pa > 0, va=va > 0, h=h > 0)
+    else:
+        relu_masks = {k: np.asarray(masks[k], dtype=bool) for k in _MASKED}
+    return log_p, v, dict(x=x, a1=a1, a2=a2, a3=a3, pa=pa, pf=pf, va=va, vf=vf, h=h, v=v, log_p=log_p, masks=relu_masks)
 
 
-def loss_and_grads(p, x, pi, z):
-    """(loss, entropy, grads) of alphazero_agent.py:66-85; grads keyed like the state_dict."""
+def loss_and_grads(p, x, pi, z, masks=None):
+    """(loss, entropy, grads) of alphazero_agent.py:66-85; grads keyed like the state_dict.  ``masks``: as in
+    ``forward`` (the backward pass uses the same masks as the forward)."""
     B = x.shape[0]
-    log_p, v, c = forward(p, x)
+    log_p, v, c = forward(p, x, masks)
+    m = c['masks']
     value_loss = np.mean((v.reshape(-1) - z) ** 2)
     policy_loss = -np.mean(np.sum(pi * log_p, axis=1))
     loss = value_loss + policy_loss
@@ -77,10 +101,10 @@ def loss_and_grads(p, x, pi, z):
     dpre2 = dv * (1.0 - v ** 2)                              # tanh'
     g['val_fc2.weight'] = dpre2.T @ c['h']
     g['val_fc2.bias'] = dpre2.sum(axis=0)
-    dh = (dpre2 @ p['val_fc2.weight']) * (c['h'] > 0)
+    dh = (dpre2 @ p['val_fc2.weight']) * m['h']
     g['val_fc1.weight'] = dh.T @ c['vf']
     g['val_fc1.bias'] = dh.sum(axis=0)
-    dva = (dh @ p['val_fc1.weight']).reshape(c['va'].shape) * (c['va'] > 0)
+    dva = (dh @ p['val_fc1.weight']).reshape(c['va'].shape) * m['va']
     g['val_conv1.weight'] = np.einsum('bohw,bchw->oc', dva, c['a3'])[:, :, None, None]
     g['val_conv1.bias'] = dva.sum(axis=(0, 2, 3))
     da3 = np.einsum('bohw,oc->bchw', dva, p['val_conv1.weight'][:, :, 0, 0])
@@ -88,16 +112,16 @@ def loss_and_grads(p, x, pi, z):
     dlogits = (prob * pi.sum(axis=1, keepdims=True) - pi) / B
     g['act_fc1.weight'] = dlogits.T @ c['pf']
     g['act_fc1.bias'] = dlogits.sum(axis=0)
-    dpa = (dlogits @ p['act_fc1.weight']).reshape(c['pa'].shape) * (c['pa'] > 0)
+    dpa = (dlogits @ p['act_fc1.weight']).reshape(c['pa'].shape) * m['pa']
     g['act_conv1.weight'] = np.einsum('bohw,bchw->oc', dpa, c['a3'])[:, :, None, None]
     g['act_conv1.bias'] = dpa.sum(axis=(0, 2, 3))
     da3 = da3 + np.einsum('bohw,oc->bchw', dpa, p['act_conv1.weight'][:, :, 0, 0])
     # trunk
-    dz3 = da3 * (c['a3'] > 0)
+    dz3 = da3 * m['a3']
     da2, g['conv3.weight'], g['conv3.bias'] = _conv3x3_backward(c['a2'], p['conv3.weight'], dz3)
-    dz2 = da2 * (c['a2'] > 0)
+    dz2 = da2 * m['a2']
     da1, g['conv2.weight'], g['conv2.bias'] = _conv3x3_backward(c['a1'], p['conv2.weight'], dz2)
-    dz1 = da1 * (c['a1'] > 0)
+    dz1 = da1 * m['a1']
     _, g['conv1.weight'], g['conv1.bias'] = _conv3x3_backward(c['x'], p['conv1.weight'], dz1)
     return float(loss), float(entropy), g
 

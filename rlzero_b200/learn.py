@@ -80,7 +80,10 @@ class NativeTrainer(object):
     use_tc_trunk = False       # True ('native_tc'): forward AND data-gradient convolutions on the tensor cores too, on
                                # 16-mantissa-bit pairs: 3x faster at batch 512.  Forward within 1e-5 as before; the
                                # gradients within ~1e-3..1e-2 of the float64 oracle instead of 1e-5 (ReLU masks of
-                               # pre-activations within 2e-6 of zero flip) -- tighter than PyTorch's default TF32
+                               # pre-activations within 2e-6 of zero flip) -- tighter than PyTorch's default TF32.
+                               # With the oracle's ReLU masks pinned to the device's, the gradients are within 1.9e-5
+                               # of their largest entry on a B200 (act_fc1.weight: up to 2.6e-4 when almost no policy
+                               # feature is positive, the cost of 16-bit weights; tests/test_gpu_learn_split.py)
 
     def _init_trunk(self):
         f32 = torch.float32
